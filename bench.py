@@ -14,6 +14,7 @@ against the local rows, exchanges the packed top-k candidates in ONE NCCL all-ga
 (SURVEY.md 8(e), `dist.ShardedKNN.predict_sharded`).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]           # our CUDA path
+  python bench.py ... --dump-outputs DIR                        # + what the last timed step computed, DIR/<name>.npy
   python bench.py --impl reference ...                          # the reference's own code on the host cores
   torchrun --nproc-per-node N ... bench.py --gpus N ...         # N>1
 
@@ -57,7 +58,12 @@ def parse():
     ap.add_argument("--train-utts", type=int, default=100000, help="utterances of the KNN train set (whole job)")
     ap.add_argument("--knn-path", default="sharded", choices=["sharded", "replicated"],
                     help="N>1: row-sharded train set with the candidate all-gather (north star), or train rows replicated")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) to DIR/<name>.npy, for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
@@ -366,6 +372,40 @@ def traffic_of_record(kernel_src):
         return None
 
 
+DUMP_MAX_UTTS = 200000      # per-utterance arrays: 236 B an utterance in float64 / float32 -> at most 47 MB
+DUMP_FRAME_UTTS = 512       # per-frame arrays for a fixed sample of utterances (<= 343 frames each at 256 / 128)
+
+
+def dump_outputs(out_dir, fe, qn, labels):
+    """What one step of the timed path hands its caller -- KNN labels, z-scored features, the front end's statistics,
+    endpoints, frame counts and status per utterance, per-frame energy / magnitude / ZCR -- as out_dir/<name>.npy.
+    Integer outputs are stored as float64 (exact).  Batches above DUMP_MAX_UTTS utterances keep a fixed, seeded sample
+    of utterances (`utterances` lists which); the per-frame arrays cover a fixed, seeded sample of DUMP_FRAME_UTTS
+    utterances (`frame_utterances`), packed back to back at `frame_offsets`."""
+    import torch
+    n = fe.n_utts
+    rows = np.arange(n) if n <= DUMP_MAX_UTTS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_UTTS, replace=False))
+    f64 = lambda t: t.cpu().numpy().astype(np.float64)
+    out = {"utterances": rows.astype(np.float64), "labels": f64(labels)[rows], "zscores": f64(qn)[rows],
+           "stats": fe.stats.cpu().numpy()[rows]}
+    for name in ("start", "end", "n_epd_frames", "n_frames", "status"):
+        out[name] = f64(getattr(fe, name))[rows]
+    picked = np.sort(np.random.default_rng(1).choice(n, min(n, DUMP_FRAME_UTTS), replace=False))
+    nf = fe.n_frames.cpu().numpy()[picked].astype(np.int64)
+    idx = np.concatenate([np.arange(fe.h_feat_offsets[b], fe.h_feat_offsets[b] + k) for b, k in zip(picked, nf)] + [[]])
+    idx = torch.from_numpy(idx.astype(np.int64)).to(fe.device)
+    out["frame_utterances"] = picked.astype(np.float64)
+    out["frame_offsets"] = np.concatenate([[0], np.cumsum(nf)]).astype(np.float64)
+    for name in ("energy", "magnitude", "zcr"):
+        out[f"frame_{name}"] = getattr(fe, name)[idx].cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    assert total <= 64 << 20 and all(a.dtype in (np.float32, np.float64) for a in out.values()), total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return total
+
+
 # --------------------------------------------------------------------------------------------
 def run_ours(args):
     import faulthandler
@@ -464,6 +504,11 @@ def run_ours(args):
             ev[i + 1].record(stream)
     stream.synchronize()
     torch.cuda.cudart().cudaProfilerStop()
+    if args.dump_outputs and rank == 0:
+        # before anything below reruns the front end or the classifier on these buffers
+        nbytes = dump_outputs(args.dump_outputs, frontends[WINDOWS[(args.steps - 1) % 3]], qn, labels[0])
+        print(f"bench: outputs of timed step {args.steps} ({WINDOWS[(args.steps - 1) % 3]} window, {nbytes / 1e6:.1f} MB) "
+              f"-> {args.dump_outputs}", file=sys.stderr, flush=True)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.launch_count - launches0

@@ -7,7 +7,9 @@ subprocess: once as the reference itself (CPU, stub plotting modules) and once t
 `python -m dsp_audioreclabs_b200.run <script>` (drop-in `config` / `src.*`, CUDA).  Outputs must be identical:
 the drop-in serves the float64 replay kernel's values, which are the reference's own bit for bit.  The run
 report proves the CUDA path ran (kernel launches > 0, modules resolved to the drop-in) and that a whole data
-tree costs ONE front-end launch per configuration (SURVEY.md 8 f2).
+tree costs ONE front-end launch per configuration (SURVEY.md 8 f2).  Without that copy those tests skip;
+test_config1_feature_matrix_matches_the_stored_reference_matrix still holds the CUDA path to the matrix the reference
+built (tests/golden/scripts_golden.npz).
 """
 import json
 import os
@@ -110,6 +112,48 @@ def test_load_dataset_matrix_matches_the_reference(work):
                DSP_RESULTS_DIR=str(work["base"] / "res_h"))
     subprocess.run([sys.executable, "-m", "dsp_audioreclabs_b200.run", str(harness)], cwd=str(work["base"]), env=env, check=True,
                    stdout=subprocess.DEVNULL)
+    z, g = np.load(out), np.load(GOLD)
+    X, y = z["X"], z["y"]
+    order = np.lexsort(tuple(X[:, j] for j in range(X.shape[1] - 1, -1, -1)) + (y,))
+    assert X.shape == (200, 15) and X.dtype == np.float64
+    assert np.array_equal(y[order], g["y_sorted"])
+    assert np.array_equal(X[order], g["X_sorted"])
+    assert list(z["names"]) == list(g["names"])
+
+
+def test_config1_feature_matrix_matches_the_stored_reference_matrix(tmp_path):
+    """The same comparison without a copy of the reference: the per-file loop of load_dataset('hamming') (sorted class
+    folders, glob('*.wav') per class, process_audio_file + extract_features_from_frames with config's constants) over
+    the drop-in modules reproduces the stored (200, 15) matrix bit for bit, and the whole tree costs ONE launch."""
+    from oracle import synth
+    data = tmp_path / "data"
+    assert synth.write_config1_dataset(data) == 200
+    harness = tmp_path / "harness.py"
+    out = tmp_path / "x.npz"
+    harness.write_text(
+        "import glob, os, numpy as np\n"
+        "import config\n"
+        "from src.audio_processing import process_audio_file\n"
+        "from src.feature_extraction import extract_features_from_frames\n"
+        "X, y, names = [], [], None\n"
+        "classes = sorted(c for c in os.listdir(config.DATA_DIR) if os.path.isdir(os.path.join(config.DATA_DIR, c)) and not c.startswith('.'))\n"
+        "for label, c in enumerate(classes):\n"
+        "    for p in glob.glob(os.path.join(config.DATA_DIR, c, '*.wav')):\n"
+        "        frames, _, _ = process_audio_file(p, config.FRAME_LENGTH, config.FRAME_SHIFT, 'hamming', True,\n"
+        "                                          config.ENERGY_HIGH_RATIO, config.ENERGY_LOW_RATIO, config.ZCR_THRESHOLD_RATIO)\n"
+        "        vec, names = extract_features_from_frames(frames, method='statistical')\n"
+        "        X.append(vec)\n"
+        "        y.append(label)\n"
+        f"np.savez({str(out)!r}, X=np.array(X), y=np.array(y), names=np.array(names))\n")
+    report = str(tmp_path / "report.jsonl")
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([ROOT, STUBS]), SPEECH_DATA_DIR=str(data),
+               DSP_RESULTS_DIR=str(tmp_path / "results"), DSP_RUN_REPORT=report)
+    subprocess.run([sys.executable, "-m", "dsp_audioreclabs_b200.run", str(harness)], cwd=str(tmp_path), env=env, check=True,
+                   stdout=subprocess.DEVNULL)
+    rep = json.loads(open(report).read().strip().splitlines()[-1])
+    assert "error" not in rep, rep
+    assert rep["src.audio_processing"].startswith(DROPIN) and rep["config"].startswith(DROPIN)
+    assert rep["gpu_launches"] > 0 and rep["frontend_launches"] == [["tree", 200]]
     z, g = np.load(out), np.load(GOLD)
     X, y = z["X"], z["y"]
     order = np.lexsort(tuple(X[:, j] for j in range(X.shape[1] - 1, -1, -1)) + (y,))
