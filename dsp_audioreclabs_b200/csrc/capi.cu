@@ -118,6 +118,7 @@ struct dsp_context {
   int pcm_variant = -1;         // -1 automatic; else a build of frontend_pcm.cu's kVariants (dsp_set_tuning / DSP_PCM_VARIANT)
   int stagger_ns = 0;           // DSP_STAGGER_NS (tuning knob)
   int tma_chunk = 4096;         // bytes per bulk copy; DSP_TMA_CHUNK overrides (tuning knob)
+  int knn_prune = 1;            // tile pruning of the D <= 15 filter: 0 off, 1 unless the lists keep > 85 % of the tiles, 2 always
   int occ = 0;
   Slot slot[2];
   DevBuf tmp[16];
@@ -130,10 +131,12 @@ struct dsp_knn {
   float tnorm_max = 0.f;
   bool dense = false;          // tensor-core candidate scan (knn_dense.cu): feature dimension beyond the tiled scan
   bool tc16 = false;           // d <= 15: tensor-core candidate filter (knn_tc16.cu); the fp32 tiled scan stands in when a value leaves its range
-  DevBuf tc_train, tc_q, tc_flags;
+  DevBuf tc_train, tc_train_rows, tc_q, tc_flags;      // train packed in tile order / in row order (knn_prune 0)
   DevBuf train64, train32, labels, tnorm, cand_idx, cand_worst, qnorm, redo_list, redo_count, nbr_label, q, o_idx, o_dist, o_lab;
   DevBuf refine_list, refine_thr, surv_count, surv_rows;     // second pass of the D <= 15 path (knn_refine)
-  DevBuf thr0;                                               // bounded calls: per-query start thresholds of the filter
+  DevBuf thr0;                                               // bounded / pruned calls: per-query start thresholds of the filter
+  DevBuf prune_perm, prune_geom, prune_box, prune_ws, prune_bound;   // tile pruning (knn_prune_plan / knn_prune_prepare)
+  int64_t prune_tiles = 0;
   DevBuf tpacked, tnorm_dense, qpacked, qnorm_chunk, dense_flags, part_d, part_i;
 };
 
@@ -465,6 +468,9 @@ int dsp_set_tuning(dsp_context* c, const char* key, int value) {
     c->tma_chunk = value;
   } else if (!std::strcmp(key, "stagger_ns")) {
     c->stagger_ns = value;
+  } else if (!std::strcmp(key, "knn_prune")) {
+    if (value < 0 || value > 2) return fail(DSP_ERR_INVALID, "knn_prune must be 0 (off), 1 (automatic) or 2 (always)");
+    c->knn_prune = value;
   } else {
     return fail(DSP_ERR_INVALID, "unknown tuning key '%s'", key);
   }
@@ -835,7 +841,8 @@ static void knn_release(dsp_knn* k) {
   DevBuf* all[] = {&k->train64, &k->train32, &k->labels, &k->tnorm, &k->cand_idx, &k->cand_worst, &k->qnorm,
                    &k->redo_list, &k->redo_count, &k->nbr_label, &k->q, &k->o_idx, &k->o_dist, &k->o_lab,
                    &k->tpacked, &k->tnorm_dense, &k->qpacked, &k->qnorm_chunk, &k->dense_flags, &k->part_d, &k->part_i,
-                   &k->tc_train, &k->tc_q, &k->tc_flags, &k->refine_list, &k->refine_thr, &k->surv_count, &k->surv_rows, &k->thr0};
+                   &k->tc_train, &k->tc_train_rows, &k->tc_q, &k->tc_flags, &k->refine_list, &k->refine_thr, &k->surv_count, &k->surv_rows, &k->thr0,
+                   &k->prune_perm, &k->prune_geom, &k->prune_box, &k->prune_ws, &k->prune_bound};
   for (DevBuf* b : all) b->release();
 }
 
@@ -862,13 +869,39 @@ int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* label
   }
   int tc_flags[2] = {0, 1};
   if (h->dp == 16 && n >= 64 && k < kKnnCand && std::getenv("DSP_KNN_NO_TC16") == nullptr) {
-    // the 15-dim statistical features: split-fp16 operands in tensor-core tile order, |t|^2 as the 16th feature
-    if (h->tc_train.ensure(knn_tc16_packed_bytes(n, false)) != cudaSuccess || h->tc_flags.ensure(64) != cudaSuccess)
+    // the 15-dim statistical features: split-fp16 operands in tensor-core tile order, |t|^2 as the 16th feature; tc_train
+    // holds the rows in the tile order of the pruning plan (principal-axis median splits), train64 / train32 keep the
+    // original order
+    std::vector<double> host((size_t)n * d);
+    if (cudaMemcpyAsync(host.data(), h->train64.p, sizeof(double) * host.size(), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
+        cudaStreamSynchronize(c->stream) != cudaSuccess)
+      return bail(fail(DSP_ERR_CUDA, "knn fit: %s", cudaGetErrorString(cudaGetLastError())));
+    KnnPrunePlan plan;
+    knn_prune_plan(host.data(), n, d, plan);
+    h->prune_tiles = (int64_t)plan.slack.size();
+    const size_t box = sizeof(double) * plan.lo.size();
+    if (h->tc_train.ensure(knn_tc16_packed_bytes(n, false)) != cudaSuccess || h->tc_flags.ensure(64) != cudaSuccess ||
+        h->prune_perm.ensure(sizeof(int) * (size_t)n) != cudaSuccess || h->prune_geom.ensure(sizeof(KnnPruneGeom)) != cudaSuccess ||
+        h->prune_box.ensure(2 * box + sizeof(double) * plan.slack.size()) != cudaSuccess)
       return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
-    cudaError_t e = knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train.p, nullptr, h->tc_flags.as<int>(), c->stream);
+    unsigned char* pb = h->prune_box.as<unsigned char>();
+    cudaMemcpyAsync(h->prune_perm.p, plan.perm.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(h->prune_geom.p, &plan.geom, sizeof(KnnPruneGeom), cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(pb, plan.lo.data(), box, cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(pb + box, plan.hi.data(), box, cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(pb + 2 * box, plan.slack.data(), sizeof(double) * plan.slack.size(), cudaMemcpyHostToDevice, c->stream);
+    if (h->tc_train_rows.ensure(knn_tc16_packed_bytes(n, false)) != cudaSuccess) return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
+    // row order for unpruned calls: a walk over spatially ordered tiles finds its neighbours late, and the filter pays
+    // for the insertions (2x on the bench's features)
+    cudaError_t e = knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train_rows.p, nullptr, h->tc_flags.as<int>(), c->stream);
+    if (e == cudaSuccess)
+      e = knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train.p, nullptr, h->tc_flags.as<int>(), c->stream,
+                        h->prune_perm.as<int>());
     c->launches++;
     if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "knn_tc16_pack: %s", cudaGetErrorString(e)));
     cudaMemcpyAsync(tc_flags, h->tc_flags.p, sizeof tc_flags, cudaMemcpyDeviceToHost, c->stream);
+    if (cudaStreamSynchronize(c->stream) != cudaSuccess)        // (the plan's host vectors are sources of the copies above)
+      return bail(fail(DSP_ERR_CUDA, "knn fit: %s", cudaGetErrorString(cudaGetLastError())));
   }
   int dense_flags[2] = {0, 0};
   if (!h->dp && d <= kKnnDenseMaxDim && std::getenv("DSP_KNN_NO_DENSE") == nullptr) {
@@ -928,6 +961,8 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
   dsp_context* c = h->ctx;
   CU(cudaSetDevice(c->device));
   CU(h->redo_list.ensure(sizeof(int32_t) * (size_t)m));
+  const unsigned long long* prune_kept = nullptr;     // (DSP_KNN_DEBUG report)
+  int64_t prune_visits = 0;
   if (h->dp) {
     CU(h->cand_idx.ensure(sizeof(int) * (size_t)m * kKnnCand));
     CU(h->cand_worst.ensure(sizeof(float) * (size_t)m));
@@ -935,24 +970,52 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
     double err_rel = (double)(h->d + 4) * 1.1920929e-7, err_floor = 0.0;
     float qnorm_limit = 0.f;
     const float* thr0 = nullptr;       // only the tensor-core filter takes start thresholds; the other scans ignore `bound`
+    const double* rerank_bound = nullptr;
     if (h->tc16) {
       // tensor-core filter; a query outside its range (|q|^2 above knn_tc16_max_norm(), NaN / inf) is scored as the zero
       // vector there and handed to the exhaustive float64 scan by the rerank kernel -- per query, on the device
       CU(h->tc_q.ensure(knn_tc16_packed_bytes(m, true)));
       int* qflags = h->tc_flags.as<int>() + 4;
-      CU(knn_tc16_pack(q, m, h->d, true, h->tc_q.p, h->qnorm.as<float>(), qflags, c->stream));
       err_rel = knn_dense_err_rel(16);
       err_floor = 1.0;
       qnorm_limit = knn_tc16_max_norm();
-      if (bound) {
+      Tc16Work work;
+      const void* tpacked = h->tc_train_rows.p;
+      // (the tile lists take units x tiles ints, indexed in int)
+      const bool prune = c->knn_prune && knn_tc16_padded_rows(m, true) / kTc16UnitQueries * h->prune_tiles <= INT32_MAX;
+      if (prune) {
+        // tile pruning: queries in curve order, a seed pass bounds every query's k-th distance U (capped by the caller's
+        // bound), and the main pass visits per unit only the tiles that can hold a row within U; its candidates are
+        // certified against U like a bounded call's
+        CU(h->prune_ws.ensure(knn_prune_scratch_bytes(m, h->n)));
+        CU(h->prune_bound.ensure(sizeof(double) * (size_t)m));
+        CU(h->thr0.ensure(sizeof(float) * (size_t)m));
+        const unsigned char* pb = h->prune_box.as<unsigned char>();
+        const size_t box = sizeof(double) * (size_t)h->prune_tiles * h->d;
+        CU(knn_prune_prepare(q, m, h->n, h->d, h->k, h->train64.as<double>(), h->prune_geom.as<KnnPruneGeom>(), h->prune_perm.as<int>(),
+                             (const double*)pb, (const double*)(pb + box), (const double*)(pb + 2 * box), h->tc_train.p, h->tc_q.p,
+                             h->qnorm.as<float>(), qflags, bound, h->prune_bound.as<double>(), h->cand_idx.as<int>(),
+                             h->cand_worst.as<float>(), h->prune_ws.p, c->knn_prune == 1, c->sm_count, c->stream, work));
+        tpacked = h->tc_train.p;
+        rerank_bound = h->prune_bound.as<double>();
+        prune_kept = work.kept;
+        prune_visits = knn_tc16_padded_rows(m, true) / kTc16UnitQueries * h->prune_tiles;
+        CU(knn_bound_thresholds(rerank_bound, h->qnorm.as<float>(), m, err_rel, err_floor, h->thr0.as<float>(), c->stream));
+        thr0 = h->thr0.as<float>();
+        c->launches += 12;
+      } else {
+        CU(knn_tc16_pack(q, m, h->d, true, h->tc_q.p, h->qnorm.as<float>(), qflags, c->stream));
+      }
+      if (bound && !prune) {
         // bounded call (row-sharded KNN): every query's filter starts at the score threshold of its radius
         CU(h->thr0.ensure(sizeof(float) * (size_t)m));
         CU(knn_bound_thresholds(bound, h->qnorm.as<float>(), m, err_rel, err_floor, h->thr0.as<float>(), c->stream));
         thr0 = h->thr0.as<float>();
+        rerank_bound = bound;
         c->launches += 1;
       }
-      CU(knn_tc16_filter(h->tc_q.p, h->tc_train.p, m, h->n, h->k, qflags, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
-                         c->sm_count, c->stream, thr0));
+      CU(knn_tc16_filter(h->tc_q.p, tpacked, m, h->n, h->k, qflags, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
+                         c->sm_count, c->stream, thr0, work));
       c->launches += 2;
     } else {
       CU(knn_scan(h->dp, h->train32.as<float>(), h->n, q, m, h->d, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
@@ -972,13 +1035,13 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
                   h->labels.as<int32_t>(), h->cand_idx.as<int>(), h->cand_worst.as<float>(), h->qnorm.as<float>(),
                   h->tnorm_max, err_rel, err_floor, nbr_idx, nbr_sqdist, nbr_label, h->redo_list.as<int32_t>(),
                   h->redo_count.as<int32_t>(), c->stream, refine_cap ? h->refine_list.as<int32_t>() : nullptr,
-                  h->refine_thr.as<float>(), refine_cap, qnorm_limit, thr0 ? bound : nullptr, thr0));
+                  h->refine_thr.as<float>(), refine_cap, qnorm_limit, rerank_bound, thr0, bound && thr0));
     c->launches += 1;
     if (refine_cap) {
       CU(knn_refine(h->train64.as<double>(), h->train32.as<float>(), h->dp, h->n, q, h->d, h->k, h->index_base,
                     h->labels.as<int32_t>(), h->refine_list.as<int32_t>(), h->refine_thr.as<float>(), refine_cap,
                     h->surv_count.as<int32_t>(), h->surv_rows.as<int32_t>(), h->redo_count.as<int32_t>(),
-                    h->redo_list.as<int32_t>(), nbr_idx, nbr_sqdist, nbr_label, c->sm_count, c->stream, thr0 != nullptr));
+                    h->redo_list.as<int32_t>(), nbr_idx, nbr_sqdist, nbr_label, c->sm_count, c->stream, bound && thr0));
       c->launches += 2;
     }
   } else if (h->dense) {
@@ -1031,6 +1094,13 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
     cudaMemcpyAsync(cnt, h->redo_count.p, sizeof cnt, cudaMemcpyDeviceToHost, c->stream);
     cudaStreamSynchronize(c->stream);
     fprintf(stderr, "[knn] m=%lld n=%lld exhaustive=%d refined=%d refined->exhaustive=%d\n", (long long)m, (long long)h->n, cnt[0], cnt[1], cnt[2]);
+    if (prune_kept) {
+      unsigned long long kept = 0;
+      cudaMemcpyAsync(&kept, prune_kept, sizeof kept, cudaMemcpyDeviceToHost, c->stream);
+      cudaStreamSynchronize(c->stream);
+      fprintf(stderr, "[knn] prune: tile visits kept=%llu of %lld (%s)\n", kept, (long long)prune_visits,
+              c->knn_prune == 1 && kept > (unsigned long long)(0.85 * (double)prune_visits) ? "every tile walked" : "lists walked");
+    }
   }
   return DSP_OK;
 }

@@ -211,7 +211,7 @@ __global__ void knn_rerank_kernel(const double* __restrict__ train, const float*
                                   int32_t* __restrict__ nbr_label, int32_t* __restrict__ redo_list,
                                   int32_t* __restrict__ redo_count, int32_t* __restrict__ refine_list,
                                   float* __restrict__ refine_thr, int refine_cap, float qnorm_limit,
-                                  const double* __restrict__ bound, const float* __restrict__ thr0) {
+                                  const double* __restrict__ bound, const float* __restrict__ thr0, bool allow_short) {
   const int64_t qi = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (qi >= m) return;
   const double* q = queries + qi * d;
@@ -238,7 +238,8 @@ __global__ void knn_rerank_kernel(const double* __restrict__ train, const float*
   const double U = bound ? bound[qi] : INFINITY;
   const double Dk = nc >= kk ? cd[kk - 1] : INFINITY;
   const double T = fmin(Dk, U);
-  bool ok = in_range && T < INFINITY;
+  // allow_short = false: the bound is the call's own (tile pruning), and k rows inside it are known to exist
+  bool ok = in_range && T < INFINITY && (allow_short || nc >= kk);
   if (ok && (n > kKnnCand || bound)) {
     // The scan's score of row t is within err_rel * (|q| + |t|)^2 of |t|^2 - 2 q.t (the roundings act on terms bounded by
     // (|q| + |t|)^2).  A row that could still matter has exact distance <= T, hence |t| <= |q| + sqrt(T) by the triangle
@@ -818,7 +819,7 @@ cudaError_t knn_rerank(const double* train, const float* train32, int dp, int64_
                        const int* cand_idx, const float* cand_worst, const float* qnorm,
                        float tnorm_max_host, double err_rel, double err_floor, int64_t* nbr_idx, double* nbr_sqdist, int32_t* nbr_label,
                        int32_t* redo_list, int32_t* redo_count, cudaStream_t st, int32_t* refine_list, float* refine_thr,
-                       int refine_cap, float qnorm_limit, const double* bound, const float* thr0) {
+                       int refine_cap, float qnorm_limit, const double* bound, const float* thr0, bool allow_short) {
   if (m == 0) return cudaSuccess;
   cudaMemsetAsync(redo_count, 0, 4 * sizeof(int32_t), st);
   if (d > 64) {
@@ -830,7 +831,8 @@ cudaError_t knn_rerank(const double* train, const float* train32, int dp, int64_
   }
   knn_rerank_kernel<<<(unsigned)((m + 127) / 128), 128, 0, st>>>(
       train, train32, dp, n, q, m, d, k, index_base, labels, cand_idx, cand_worst, qnorm, tnorm_max_host, err_rel, err_floor,
-      nbr_idx, nbr_sqdist, nbr_label, redo_list, redo_count, refine_list, refine_thr, refine_cap, qnorm_limit, bound, thr0);
+      nbr_idx, nbr_sqdist, nbr_label, redo_list, redo_count, refine_list, refine_thr, refine_cap, qnorm_limit, bound, thr0,
+      allow_short);
   return cudaGetLastError();
 }
 

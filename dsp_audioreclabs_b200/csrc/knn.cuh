@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <vector>
+
 namespace dsp {
 
 constexpr int kKnnCand = 8;    // fp32 candidates kept per query by the scan
@@ -21,7 +23,7 @@ cudaError_t knn_rerank(const double* train, const float* train32, int dp, int64_
                        float tnorm_max_host, double err_rel, double err_floor, int64_t* nbr_idx, double* nbr_sqdist, int32_t* nbr_label,
                        int32_t* redo_list, int32_t* redo_count, cudaStream_t st, int32_t* refine_list = nullptr,
                        float* refine_thr = nullptr, int refine_cap = 0, float qnorm_limit = 0.f,
-                       const double* bound = nullptr, const float* thr0 = nullptr);
+                       const double* bound = nullptr, const float* thr0 = nullptr, bool allow_short = true);
 // D <= 15: second pass for the queries the certificate rejected (fp32 threshold scan + float64 ranking of the survivors);
 // counts = redo_count: [0] exhaustive rescans, [1] refined queries, [2] refined queries passed on to the exhaustive scan
 int knn_refine_survivor_cap();
@@ -47,12 +49,57 @@ cudaError_t knn_merge_vote(const double* cd, const int64_t* ci, const int32_t* c
 float knn_tc16_max_norm();                                   // largest |x|^2 the filter accepts (else: fp32 scan)
 int64_t knn_tc16_padded_rows(int64_t rows, bool query);
 size_t knn_tc16_packed_bytes(int64_t rows, bool query);
-// flags[0] = max |x|^2 (float bits), flags[1] = 1 when a row is outside the range; norms (optional): |x|^2 per row
-cudaError_t knn_tc16_pack(const double* x, int64_t rows, int d, bool query, void* packed, float* norms, int* flags, cudaStream_t st);
+constexpr int kTc16TileRows = 128;                           // train rows per filter tile
+constexpr int kTc16UnitQueries = 256;                        // queries per filter work unit
+// flags[0] = max |x|^2 (float bits), flags[1] = 1 when a row is outside the range; norms (optional): |x|^2 per row,
+// at the source row; gather (optional): packed row r holds source row gather[r]
+cudaError_t knn_tc16_pack(const double* x, int64_t rows, int d, bool query, void* packed, float* norms, int* flags, cudaStream_t st,
+                          const int* gather = nullptr);
+// What the filter walks and how its positions map back.  Default: every work unit in turn, every train tile in order,
+// packed positions = row / query indices.
+struct Tc16Work {
+  const int* tiles = nullptr;        // [units][stride]: the train tiles each unit visits (nullptr: all of them)
+  const int* tile_count = nullptr;   // [units]
+  int stride = 0;
+  const int* unit_order = nullptr;   // units in the order they are claimed (nullptr: 0, 1, ...)
+  int* counter = nullptr;            // claim counter, zero at launch (nullptr: static stride over the grid)
+  const unsigned long long* kept = nullptr;   // (optional, device) tile visits of all lists: above kept_limit, walk every tile
+  unsigned long long kept_limit = 0;
+  const int* qperm = nullptr;        // packed query position -> query index
+  const int* tperm = nullptr;        // packed train position -> train row
+};
 // k: neighbours the caller will certify (the filter keeps k + 2 candidates for k <= 3, else 8); needs n >= 64
-// thr0 (optional, [m]): start every query's filter at this score threshold (knn_bound_thresholds)
+// thr0 (optional, [m], by query index): start every query's filter at this score threshold (knn_bound_thresholds)
 cudaError_t knn_tc16_filter(const void* qpacked, const void* tpacked, int64_t m, int64_t n, int k, const int* qflags, int* cand_idx,
-                            float* cand_worst, int sm_count, cudaStream_t st, const float* thr0 = nullptr);
+                            float* cand_worst, int sm_count, cudaStream_t st, const float* thr0 = nullptr, const Tc16Work& work = Tc16Work());
+
+// Tile pruning for the filter (knn_tc16.cu).  At fit the train rows are ordered into 128-row tiles by recursive median
+// splits along their principal axes, and every tile keeps its bounding box in those axes.  Per call the queries are
+// sorted along a space-filling curve into 256-query units; a seed pass over each unit's nearest tiles bounds every
+// query's k-th distance U, and a unit visits only the tiles whose box lies within max U of its own box.
+constexpr int kPruneMaxDim = 15;
+constexpr int kPruneSeedTiles = 4;                           // tiles per unit in the seed pass
+struct KnnPruneGeom {
+  int d;
+  double mean[kPruneMaxDim];
+  double axis[kPruneMaxDim][kPruneMaxDim];                   // principal axes, largest variance first: axis[a][j]
+  double key_lo[3], key_scale[3];                            // curve quantisation of the first three projections
+};
+struct KnnPrunePlan {
+  KnnPruneGeom geom;
+  std::vector<int> perm;                                     // tile-ordered position -> train row
+  std::vector<double> lo, hi, slack;                         // per tile: [tiles][d] box in the axes, rounding slack
+};
+void knn_prune_plan(const double* train, int64_t n, int d, KnnPrunePlan& plan);      // host, float64
+// device scratch of one call: knn_prune_scratch_bytes() bytes, 256-byte aligned
+size_t knn_prune_scratch_bytes(int64_t m, int64_t n);
+// Builds the query order, packs the queries, runs the seed pass and leaves the main pass's tile lists: bound[m] = U per
+// query (min with caller_bound when given), work = the schedule of the main filter call.  auto_fallback: the main pass
+// walks every tile when the lists keep more than 85 % of all tile visits.
+cudaError_t knn_prune_prepare(const double* q, int64_t m, int64_t n, int d, int k, const double* train, const KnnPruneGeom* geom,
+                              const int* tperm, const double* tile_lo, const double* tile_hi, const double* tile_slack, const void* tpacked,
+                              void* qpacked, float* qnorm, int* qflags, const double* caller_bound, double* bound, int* cand_idx,
+                              float* cand_worst, void* scratch, bool auto_fallback, int sm_count, cudaStream_t st, Tc16Work& work);
 // bound[i] = an upper bound on query i's k-th squared distance (exact arithmetic) -> thr0[i] = the score threshold below
 // which every row that can still matter is guaranteed to fall (bound - |q|^2 + twice the scan's error at that radius)
 cudaError_t knn_bound_thresholds(const double* bound, const float* qnorm, int64_t m, double err_rel, double err_floor, float* thr0,
