@@ -102,6 +102,7 @@ struct Slot {
 struct dsp_context {
   int device = 0;
   int sm_count = 0;
+  size_t smem_optin = 0;        // opt-in shared memory per block (227 KB on sm_100), static + dynamic
   cudaStream_t own = nullptr, stream = nullptr, s_in = nullptr, s_out = nullptr;
   int64_t launches = 0;
   // window tables stay resident per (type, length): a context that alternates windows (three front ends sharing one
@@ -316,8 +317,13 @@ int frontend_device(dsp_context* c, const void* samples, int dtype, const int64_
   if (fast) {
     cap_samples = (int)((std::max<int64_t>(max_len, 1) + 63) / 64 * 64);
     smem = pcm_kernel_smem_bytes(cap_samples, (int)cap_frames64, fl, !pcm_variant_streams(variant));
-    if (smem > kMaxSmemPerCta && !pcm_variant_streams(variant)) fast = false;
-    if (smem > kMaxSmemPerCta) fast = false;
+    if (c->occ_smem != smem || c->occ_variant != variant) {
+      c->occ = pcm_kernel_max_ctas_per_sm(variant, smem, c->smem_optin);
+      c->occ_smem = smem;
+      c->occ_variant = variant;
+    }
+    // static + dynamic shared memory beyond the per-block maximum: the float64 replay takes the batch
+    if (c->occ < 1) fast = false;
   }
   if (!fast) {
     const int grid = (int)std::min<int64_t>(B, (int64_t)c->sm_count * 4);
@@ -326,12 +332,6 @@ int frontend_device(dsp_context* c, const void* samples, int dtype, const int64_
     ex.stats_f64 = out->stats_f64; ex.epd_zcr_f64 = out->epd_zcr_f64; ex.frames_out = out->frames_f64;
     return launch_exact(c, samples, dtype, offsets, lengths, feat_offsets, epd_offsets, nullptr, nullptr, B, max_len,
                         p, out, ex, grid);
-  }
-  if (c->occ_smem != smem || c->occ_variant != variant) {
-    c->occ = pcm_kernel_max_ctas_per_sm(variant, smem);
-    c->occ_smem = smem;
-    c->occ_variant = variant;
-    if (c->occ < 1) return fail(DSP_ERR_CUDA, "fast kernel does not fit: %zu bytes of shared memory", smem);
   }
   CU(c->counters.ensure(64));
   CU(c->flag_list.ensure(sizeof(int32_t) * (size_t)B));
@@ -407,6 +407,7 @@ int dsp_create(int device, dsp_context** out) {
   dsp_context* c = new dsp_context();
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
+  c->smem_optin = prop.sharedMemPerBlockOptin;
   CU(cudaStreamCreateWithFlags(&c->own, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));

@@ -524,17 +524,18 @@ frontend_pcm_kernel(const PcmArgs a) {
       for (; v < nvec; v += kMainThreads) { const int4 q = ld16(xv + v); acc1(q); }
       int mn = min(sext16(mn2), (int)mn2 >> 16), mx = max(sext16(mx2), (int)mx2 >> 16);
       if (tid < (n & 7)) { const int k = x[(nvec << 3) + tid]; sum += k; mn = min(mn, k); mx = max(mx, k); }
-      // per-warp partials (a warp sees < 2^31 / 2^15 samples: the utterance fits shared memory)
-      sum = warp_reduce(sum, OpAddI());
+      // a thread's sum covers at most 2^20 / 96 samples (< 2^31 / 2^15), a warp's does not: a streaming build's warp
+      // sees n / kMainWarps samples (up to 2^20 / 3), so the per-warp partials are 64-bit
+      const long long wsum = warp_reduce((long long)sum, OpAddLL());
       mn = warp_reduce(mn, OpMinI());
       mx = warp_reduce(mx, OpMaxI());
-      int* part = reinterpret_cast<int*>(s_sh);
-      if (lane == 0) { part[wid] = sum; part[kWarps + wid] = mn; part[2 * kWarps + wid] = mx; }
+      long long* part = reinterpret_cast<long long*>(s_sh);      // 3 * kWarps <= 27 values of the 64 in s_sh
+      if (lane == 0) { part[wid] = wsum; part[kWarps + wid] = mn; part[2 * kWarps + wid] = mx; }
       main_sync();
       if (tid == kLeadTid) {
         long long S = 0; int gmn = 32767, gmx = -32768;
         #pragma unroll 1
-        for (int w = 0; w < kMainWarps; ++w) { S += part[w]; gmn = min(gmn, part[kWarps + w]); gmx = max(gmx, part[2 * kWarps + w]); }
+        for (int w = 0; w < kMainWarps; ++w) { S += part[w]; gmn = min(gmn, (int)part[kWarps + w]); gmx = max(gmx, (int)part[2 * kWarps + w]); }
         const long long N = n > 0 ? n : 1;
         long long q = S / N; if ((S % N) != 0 && (S < 0)) --q;      // floor(S/N)
         const long long thr = q + 1;
@@ -1048,10 +1049,16 @@ cudaError_t launch_frontend_pcm(int variant, const PcmArgs& a, int grid, size_t 
   return cudaGetLastError();
 }
 
-int pcm_kernel_max_ctas_per_sm(int variant, size_t smem) {
+int pcm_kernel_max_ctas_per_sm(int variant, size_t smem, size_t smem_optin) {
   const Variant& v = kVariants[variant];
+  cudaFuncAttributes fa{};
   int n = 0;
-  cudaFuncSetAttribute(v.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  // the kernel's static shared memory (s_prof) counts against the opt-in per-block maximum too
+  if (cudaFuncGetAttributes(&fa, v.fn) != cudaSuccess || fa.sharedSizeBytes + smem > smem_optin) return 0;
+  if (cudaFuncSetAttribute(v.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    cudaGetLastError();      // a refused size means "does not fit", not an error for the next launch to report
+    return 0;
+  }
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, v.fn, v.threads, smem) != cudaSuccess) return 0;
   return n;
 }

@@ -74,7 +74,7 @@ __global__ void sequence_stats_kernel(const double* s0, const double* s1, const 
 // frontend_pcm.cu
 size_t pcm_kernel_smem_bytes(int cap_samples, int cap_frames, int fl, bool resident);
 cudaError_t launch_frontend_pcm(int variant, const PcmArgs& a, int grid, size_t smem, cudaStream_t st);
-int pcm_kernel_max_ctas_per_sm(int variant, size_t smem);
+int pcm_kernel_max_ctas_per_sm(int variant, size_t smem, size_t smem_optin);   // 0: the build does not fit
 int pcm_num_variants();
 // frontend_pipe.cu
 struct PipePlan { int ring_slots, n_rec, cap_groups; size_t smem; };
