@@ -279,20 +279,39 @@ def sequence_stats(seq, ctx=None):
     return out
 
 
+def _axis0_is_inner(x):
+    """True when NumPy's reduction over axis 0 of `x` (np.mean / np.std, axis=0) runs along its inner loop, i.e. sums
+    every column with its pairwise algorithm; False when it adds the rows one after another.  The iterator puts axis 0
+    innermost when, after dropping length-1 axes, it is the only axis left, or its |stride| is strictly below every
+    other axis's and no stride involved is zero (zero or equal strides leave the axes in C order).  `x` is a NumPy
+    array or a torch tensor; decide on the caller's array, before any contiguous copy."""
+    strides = x.strides if isinstance(x, np.ndarray) else tuple(x.stride())
+    if x.ndim == 0 or x.shape[0] <= 1:
+        return True                      # a single row: both orders give the same sums
+    s0 = abs(strides[0])
+    rest = [abs(s) for n, s in zip(x.shape[1:], strides[1:]) if n != 1]
+    return not rest or (s0 != 0 and all(s != 0 and s0 < s for s in rest))
+
+
 def zscore(features, mean=None, std=None, ctx=None):
-    """normalize_features (src/feature_extraction.py:157-181)."""
+    """normalize_features (src/feature_extraction.py:157-181).  The fit sums each column in the order NumPy would
+    for this array's layout (_axis0_is_inner), so mean and std are bit-identical to np.mean / np.std(axis=0)."""
     ctx = _host_ctx(ctx)
+    features = np.asarray(features)
+    pairwise = _axis0_is_inner(features)
     x = _f64(features)
     one_d = x.ndim == 1
     x2 = x.reshape(-1, 1) if one_d else x.reshape(x.shape[0], -1)
     n, d = x2.shape
     fit_mean, fit_std = mean is None, std is None
-    m = np.empty(d, np.float64) if fit_mean else _f64(np.broadcast_to(mean, (d,))).copy()
-    s = np.empty(d, np.float64) if fit_std else _f64(np.broadcast_to(std, (d,))).copy()
+    # mean / std have the shape of one row (np.mean(axis=0)); given ones broadcast to it
+    row = (1,) if one_d else x.shape[1:]
+    m = np.empty(d, np.float64) if fit_mean else _f64(np.broadcast_to(mean, row)).reshape(d).copy()
+    s = np.empty(d, np.float64) if fit_std else _f64(np.broadcast_to(std, row)).reshape(d).copy()
     out = np.empty_like(x2)
     if fit_mean or fit_std:
         fm, fsd = np.empty(d, np.float64), np.empty(d, np.float64)
-        check(ctx.lib.dsp_zscore_host(ctx.handle, _ptr(x2), n, d, 2 if one_d else 1, _ptr(fm), _ptr(fsd), None))
+        check(ctx.lib.dsp_zscore_host(ctx.handle, _ptr(x2), n, d, 2 if pairwise else 1, _ptr(fm), _ptr(fsd), None))
         if fit_mean:
             m = fm
         if fit_std:
@@ -300,7 +319,7 @@ def zscore(features, mean=None, std=None, ctx=None):
     check(ctx.lib.dsp_zscore_host(ctx.handle, _ptr(x2), n, d, 0, _ptr(m), _ptr(s), _ptr(out)))
     if one_d:
         return out.reshape(x.shape), m[0], s[0]
-    return out.reshape(x.shape), m, s
+    return out.reshape(x.shape), m.reshape(x.shape[1:]), s.reshape(x.shape[1:])
 
 
 class KNN:

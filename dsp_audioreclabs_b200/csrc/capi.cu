@@ -138,6 +138,7 @@ struct dsp_knn {
   DevBuf thr0;                                               // bounded / pruned calls: per-query start thresholds of the filter
   DevBuf prune_perm, prune_geom, prune_box, prune_ws, prune_bound;   // tile pruning (knn_prune_plan / knn_prune_prepare)
   int64_t prune_tiles = 0;
+  int refine_cap = 0;          // refine list capacity of the last call (rejected queries past it count in redo_count[1] too)
   DevBuf tpacked, tnorm_dense, qpacked, qnorm_chunk, dense_flags, part_d, part_i;
 };
 
@@ -930,7 +931,8 @@ int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* label
 
 int dsp_knn_fit_host(dsp_context* c, const double* train, const int32_t* labels, int64_t n, int32_t d, int32_t k,
                      int64_t index_base, dsp_knn** out) {
-  if (!c || !out || n < 1 || d < 1 || !train || !labels) return fail(DSP_ERR_INVALID, "bad argument");
+  if (!c || !out || n < 1 || d < 1 || k < 1 || !train || !labels) return fail(DSP_ERR_INVALID, "bad argument");
+  if (k > kKnnMaxK) return fail(DSP_ERR_UNSUPPORTED, "n_neighbors > %d is not supported", kKnnMaxK);   // before any copy
   CU(cudaSetDevice(c->device));
   OneShot os(c);
   double* dt = os.dev<double>((size_t)n * d);
@@ -1026,6 +1028,7 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
     // rejected queries: fp32 threshold scan + float64 ranking of the survivors (knn_refine) for up to refine_cap of them,
     // the exhaustive float64 scan for the rest
     const int refine_cap = (h->dp == 16 && h->k < kKnnCand) ? (int)std::min<int64_t>(m, 65536) : 0;
+    h->refine_cap = refine_cap;
     if (refine_cap) {
       CU(h->refine_list.ensure(sizeof(int32_t) * (size_t)refine_cap));
       CU(h->refine_thr.ensure(sizeof(float) * (size_t)refine_cap));
@@ -1046,6 +1049,7 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
       c->launches += 2;
     }
   } else if (h->dense) {
+    h->refine_cap = 0;
     // tensor-core candidate scan in chunks of queries (bounded staging), float64 rerank + certificate per chunk;
     // the rejected queries of every chunk accumulate in one redo list
     CU(h->cand_idx.ensure(sizeof(int) * (size_t)m * kKnnCand));
@@ -1080,6 +1084,7 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
     }
     c->launches++;
   } else {
+    h->refine_cap = 0;
     // feature dimension beyond both scans (or values outside the fp16 range): exhaustive float64 scan of every query
     CU(knn_redo_all(h->redo_list.as<int32_t>(), h->redo_count.as<int32_t>(), m, c->stream));
     c->launches++;
@@ -1094,7 +1099,8 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
     int32_t cnt[4];
     cudaMemcpyAsync(cnt, h->redo_count.p, sizeof cnt, cudaMemcpyDeviceToHost, c->stream);
     cudaStreamSynchronize(c->stream);
-    fprintf(stderr, "[knn] m=%lld n=%lld exhaustive=%d refined=%d refined->exhaustive=%d\n", (long long)m, (long long)h->n, cnt[0], cnt[1], cnt[2]);
+    fprintf(stderr, "[knn] m=%lld n=%lld exhaustive=%d refined=%d refined->exhaustive=%d\n", (long long)m, (long long)h->n, cnt[0],
+            std::min(cnt[1], h->refine_cap), cnt[2]);
     if (prune_kept) {
       unsigned long long kept = 0;
       cudaMemcpyAsync(&kept, prune_kept, sizeof kept, cudaMemcpyDeviceToHost, c->stream);
@@ -1226,14 +1232,15 @@ int dsp_dtw_topk_host(dsp_context* c, const float* q_feats, const int64_t* q_off
 int dsp_knn_last_stats(dsp_knn* h, int64_t* rescanned, int32_t* scan_kind) {
   if (!h) return fail(DSP_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(h->ctx->device));
-  // queries the first certificate rejected: refined ([1]) + sent straight to the exhaustive scan ([0] minus those the
-  // refinement passed on, [2])
+  // queries the first certificate rejected: refined ([1], up to the list's capacity: a query past it took a slot number
+  // there, then went to the exhaustive scan) + sent straight to the exhaustive scan ([0] minus those the refinement
+  // passed on, [2])
   int32_t cnt[4] = {0, 0, 0, 0};
   if (h->redo_count.p) {
     CU(cudaMemcpyAsync(cnt, h->redo_count.p, sizeof cnt, cudaMemcpyDeviceToHost, h->ctx->stream));
     CU(cudaStreamSynchronize(h->ctx->stream));
   }
-  if (rescanned) *rescanned = (int64_t)cnt[0] + cnt[1] - cnt[2];
+  if (rescanned) *rescanned = (int64_t)cnt[0] + std::min(cnt[1], h->refine_cap) - cnt[2];
   if (scan_kind) *scan_kind = h->dp ? (h->tc16 ? 3 : 1) : (h->dense ? 2 : 0);
   return DSP_OK;
 }

@@ -1,10 +1,13 @@
 // normalize_features (src/feature_extraction.py:157-181): z-score over axis 0.
 //
-// np.mean / np.std over axis 0 of a C-contiguous [n, d] float64 array add the rows one
-// after another (no pairwise blocking on that axis; checked against NumPy 2.3.5), so the fit is
-// one thread per column walking the rows in order: the result is bit-identical to the
-// reference, which matters because these statistics feed the KNN distances.  A 1-D input
-// (d == 1 with `pairwise` set) uses NumPy's pairwise association instead.
+// np.mean / np.std over axis 0 sum in one of two orders, chosen by the array's layout (checked
+// against NumPy 2.3.5).  When another axis is the iterator's inner loop (C order, row- or
+// column-strided C views) they add the rows one after another.  When axis 0 is the inner loop
+// (1-D, (n, 1), Fortran order, transposed views) every column is a 1-D pairwise sum.  The fit is
+// one thread per column doing the same: rows in order, or with `pairwise` set NumPy's pairwise
+// tree.  The caller picks the mode from its array's strides before copying it to C order
+// (batch._axis0_is_inner), so the result is bit-identical to the reference, which matters
+// because these statistics feed the KNN distances.
 #include "kernels.cuh"
 #include "misc.cuh"
 

@@ -10,7 +10,7 @@ import torch
 
 from . import _capi
 from ._capi import FrontendOutputs, check
-from .batch import default_context, make_params, plan
+from .batch import _axis0_is_inner, default_context, make_params, plan
 
 _TORCH_DTYPES = {torch.int16: _capi.DSP_S16, torch.uint8: _capi.DSP_U8,
                  torch.float32: _capi.DSP_F32, torch.float64: _capi.DSP_F64}
@@ -180,16 +180,19 @@ class DeviceKNN:
 
 
 def zscore_device(x, mean=None, std=None, ctx=None):
-    """normalize_features on a CUDA float64 [n, d] tensor."""
-    assert x.is_cuda and x.dtype == torch.float64 and x.is_contiguous() and x.dim() == 2
+    """normalize_features on a CUDA float64 [n, d] tensor: the result of normalize_features(x.cpu().numpy()), whose
+    column sums follow the tensor's layout (batch._axis0_is_inner), e.g. pairwise for a transposed tensor."""
+    assert x.is_cuda and x.dtype == torch.float64 and x.dim() == 2
     ctx = ctx or default_context(x.device.index or 0)
     ctx.set_stream(torch.cuda.current_stream(x.device).cuda_stream)
+    pairwise = _axis0_is_inner(x)
+    x = x.contiguous()
     n, d = x.shape
     fit = mean is None or std is None
     fm = torch.empty(d, dtype=torch.float64, device=x.device)
     fs = torch.empty(d, dtype=torch.float64, device=x.device)
     if fit:
-        check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 1, _dp(fm), _dp(fs), None))
+        check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 2 if pairwise else 1, _dp(fm), _dp(fs), None))
     m = fm if mean is None else mean.clone()
     s = fs if std is None else std.clone()
     out = torch.empty_like(x)

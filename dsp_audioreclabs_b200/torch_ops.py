@@ -22,7 +22,7 @@ import torch
 
 from . import _capi
 from ._capi import FrontendOutputs, check
-from .batch import default_context, make_params, plan as _host_plan
+from .batch import _axis0_is_inner, default_context, make_params, plan as _host_plan
 
 NS = "dsp_audioreclabs"
 _WINDOWS = ("rectangular", "hamming", "hanning")
@@ -91,14 +91,16 @@ def _(samples, offsets, feat_offsets, n_utts, max_len, total_frames, frame_lengt
 
 @torch.library.custom_op(f"{NS}::zscore_fit", mutates_args=(), device_types="cuda")
 def zscore_fit(x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-    """normalize_features' statistics (feature_extraction.py:171-177): (mean[d], std[d] with 0 -> 1), float64."""
+    """normalize_features' statistics (feature_extraction.py:171-177): (mean[d], std[d] with 0 -> 1), float64; the
+    column sums follow x's layout like NumPy's on x.cpu().numpy() (batch._axis0_is_inner)."""
     assert x.dtype == torch.float64 and x.dim() == 2
     ctx = _ctx_for(x)
+    pairwise = _axis0_is_inner(x)
     x = x.contiguous()
     n, d = x.shape
     mean = torch.empty(d, dtype=torch.float64, device=x.device)
     std = torch.empty(d, dtype=torch.float64, device=x.device)
-    check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 1, _dp(mean), _dp(std), None))
+    check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 2 if pairwise else 1, _dp(mean), _dp(std), None))
     return mean, torch.where(std == 0, torch.ones_like(std), std)
 
 

@@ -185,7 +185,10 @@ int dsp_frame_features_host(dsp_context* ctx, const double* frames, int64_t n_fr
 int dsp_sequence_stats_host(dsp_context* ctx, const double* seq, int64_t n, double* out5);
 
 /* normalize_features (src/feature_extraction.py:157-181).  fit != 0 computes mean/std
- * (population) over axis 0 into mean/std first; std == 0 is replaced by 1 when applying
+ * (population) over axis 0 of the C-ordered [n, d] x into mean/std first, in NumPy's summation
+ * order for the caller's original layout: fit = 1 adds the rows one after another (np.mean over
+ * axis 0 of a C-ordered array), fit = 2 sums every column pairwise (np.mean of each column as a
+ * 1-D array: 1-D, (n, 1) and Fortran-ordered inputs).  std == 0 is replaced by 1 when applying
  * (the returned std keeps the replacement, as the reference does). */
 int dsp_zscore_host(dsp_context* ctx, const double* x, int64_t n, int32_t d, int fit, double* mean,
                     double* std, double* out);
