@@ -81,6 +81,19 @@ __device__ double np_pairwise_sum(Term term, int64_t n) {
   return ret;
 }
 
+// np.mean of the <= 10 noise frames of endpoint detection in NumPy's association (audio_processing.py:188-195;
+// pairwise: < 8 terms sequential, else eight accumulators combined as a tree, then the tail) -- out of line, it is
+// cold code.
+static __device__ __noinline__ double noise_mean(const double* v, int n) {
+  double r;
+  if (n < 8) { r = 0.0; for (int i = 0; i < n; ++i) r += v[i]; }
+  else { r = ((v[0] + v[1]) + (v[2] + v[3])) + ((v[4] + v[5]) + (v[6] + v[7])); for (int i = 8; i < n; ++i) r += v[i]; }
+  return r / (double)n;
+}
+
+// the low 16-bit half of a word of two int16 PCM samples, sign-extended (the high half is (int)w >> 16)
+__device__ __forceinline__ int sext16(uint32_t w) { return (int)(short)(w & 0xffffu); }
+
 // np.percentile(..., method='linear') interpolation between the two order statistics
 // (numpy/lib/_function_base_impl.py:4671-4675): a + (b-a)*g, or b - (b-a)*(1-g) when g >= 0.5.
 __device__ __forceinline__ double np_lerp(double a, double b, double g) {

@@ -25,6 +25,7 @@
 //
 // Reference: src/audio_processing.py:49-90,135-275,299-333; src/feature_extraction.py:12-88.
 #include "kernels.cuh"
+#include "ptx.cuh"
 
 namespace dsp {
 
@@ -59,38 +60,6 @@ __host__ __device__ inline SmemLayout make_layout(int cap_samples, int cap_frame
   L.misc = o;    o += 384;
   L.total = o;
   return L;
-}
-
-// ---- mbarrier / bulk-copy PTX ---------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-          smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 
 // ---- sign-bit string helpers ----------------------------------------------------------
@@ -142,8 +111,6 @@ __device__ __noinline__ int frame_zcr(const uint32_t* bits, int p, int valid, in
   return zc;
 }
 
-__device__ __forceinline__ int sext16(uint32_t w) { return (int)(short)(w & 0xffffu); }
-
 struct UttConst {
   int thr;         // floor(S/N) + 1: sample is above the mean iff k >= thr
   float phi;       // S/N - thr, in [-1, 0)
@@ -157,9 +124,6 @@ constexpr int kBarMain = 1;       // main warps only
 constexpr int kBarFeatFull = 2;   // main arrive, stats wait: feature sequences are in shared memory
 constexpr int kBarFeatEmpty = 3;  // stats arrive, main wait: feature sequences have been consumed
 constexpr int kStatsRegs = 11;    // feature frames per lane held in registers by the stats warps
-
-__device__ __forceinline__ void bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
-__device__ __forceinline__ void bar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
 // Radix-select bookkeeping shared by the block- and warp-level selects: after the 256-bin
 // histogram of (key - lo) >> s is in `hist`, one warp finds the bin holding `rank`.
@@ -278,15 +242,6 @@ __device__ __noinline__ void warp_sequence_stats(const float* vals, int stride, 
   }
 }
 
-// np.mean of the <= 10 noise frames in NumPy's association (pairwise: < 8 terms sequential, else
-// eight accumulators combined as a tree, then the tail) -- compact, it is cold code.
-__device__ __noinline__ double noise_mean(const double* v, int n) {
-  double r;
-  if (n < 8) { r = 0.0; for (int i = 0; i < n; ++i) r += v[i]; }
-  else { r = ((v[0] + v[1]) + (v[2] + v[3])) + ((v[4] + v[5]) + (v[6] + v[7])); for (int i = 8; i < n; ++i) r += v[i]; }
-  return r / (double)n;
-}
-
 }  // namespace
 
 size_t pcm_kernel_smem_bytes(int cap_samples, int cap_frames, int fl, bool resident) {
@@ -338,7 +293,7 @@ frontend_pcm_kernel(const PcmArgs a) {
   for (int j = tid; j < fl; j += kThreads) s_win[j] = a.win_f32[j];
   if (tid == 0) {
     mbar_init(s_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
     s_int[0] = (int)atomicAdd(a.work_counter, 1u);
   }
   __syncthreads();
@@ -442,7 +397,7 @@ frontend_pcm_kernel(const PcmArgs a) {
           const uint32_t chunk = (uint32_t)a.tma_chunk;
           for (uint32_t o = (uint32_t)tid * chunk; o < bytes; o += 32u * chunk) {
             const uint32_t sz = min(chunk, bytes - o);
-            bulk_g2s(reinterpret_cast<unsigned char*>(s_x) + o, reinterpret_cast<const unsigned char*>(src) + o, sz, s_bar);
+            bulk_g2s(smem_u32(s_x) + o, reinterpret_cast<const unsigned char*>(src) + o, sz, s_bar);
           }
         }
       }
@@ -464,7 +419,7 @@ frontend_pcm_kernel(const PcmArgs a) {
     const int64_t off = a.offsets[uu];
     const int n = a.lengths ? a.lengths[uu] : (int)(a.offsets[uu + 1] - off);
     const bool tma = ((reinterpret_cast<uintptr_t>(a.samples + off) & 15) == 0);
-    if (tma && (((uint32_t)n * 2u) & ~15u) > 0) { mbar_wait(s_bar, parity); parity ^= 1; }
+    if (tma && (((uint32_t)n * 2u) & ~15u) > 0) { mbar_wait_spin(s_bar, parity); parity ^= 1; }
     main_sync();
   };
 

@@ -17,7 +17,6 @@
 //           bound on the fp32 error -- otherwise the query is rescanned exhaustively in
 //           float64 (rescan kernel), so labels never depend on fp32 rounding.
 #include <algorithm>
-#include <cstdlib>
 #include "kernels.cuh"
 #include "knn.cuh"
 
@@ -801,9 +800,7 @@ cudaError_t knn_scan(int dp, const float* train32, int64_t n, const double* q, i
   if (dp == 16) {
     constexpr int QPT = 2;
     const unsigned grid = (unsigned)((m + (int64_t)kScanThreads * QPT - 1) / ((int64_t)kScanThreads * QPT));
-    static const bool scalar = std::getenv("DSP_KNN_SCALAR_SCAN") != nullptr;      // tuning: the scalar FFMA build
-    if (scalar) knn_scan_kernel<16, QPT><<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);
-    else knn_scan_pair_kernel<<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);
+    knn_scan_pair_kernel<<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);
   } else if (dp == 32) {
     const unsigned grid = (unsigned)((m + kScanThreads - 1) / kScanThreads);
     knn_scan_kernel<32, 1><<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);

@@ -26,6 +26,7 @@
 
 #include "kernels.cuh"
 #include "knn.cuh"
+#include "ptx.cuh"
 
 namespace dsp {
 
@@ -45,50 +46,6 @@ constexpr size_t kDenseSmem = (size_t)kStages * kStageBytes + 256;
 constexpr uint32_t kLBO = 128, kSBO = 1024;
 // instruction descriptor (kind::f16): D = F32 (bits 4-5 = 1), A = B = F16 (0), both K-major, N >> 3 at bit 17, M >> 4 at bit 24
 constexpr uint32_t kIdesc = (1u << 4) | ((uint32_t)(kBN >> 3) << 17) | ((uint32_t)(kBM >> 4) << 24);
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-               "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// shared-memory matrix descriptor: start address, LBO, SBO (16-byte units), version 1 (sm_100), no swizzle
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr) {
-  return (uint64_t)((saddr >> 4) & 0x3fffu) | ((uint64_t)(kLBO >> 4) << 16) | ((uint64_t)(kSBO >> 4) << 32) | (1ull << 46);
-}
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(kIdesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 
 __device__ __forceinline__ void cand_insert8(float (&cd)[kKnnCand], int (&ci)[kKnnCand], float d, int idx) {
   if (d < cd[kKnnCand - 1]) {
@@ -164,12 +121,9 @@ knn_dense_scan_kernel(const unsigned char* __restrict__ qpacked, const unsigned 
   if (tid == 0) {
     for (int i = 0; i < kStages; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
     for (int i = 0; i < kAccStages; ++i) { mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"((uint32_t)kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, kTmemCols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -208,9 +162,9 @@ knn_dense_scan_kernel(const unsigned char* __restrict__ qpacked, const unsigned 
 #pragma unroll
             for (int k4 = 0; k4 < kBK / 16; ++k4) {
               const uint32_t off = (uint32_t)k4 * 2u * kLBO;   // 16 features = two core matrices along K
-              umma_f16(d_tmem, umma_desc(q_hi + off), umma_desc(t_hi + off), (uint32_t)((kb | k4) != 0));
-              umma_f16(d_tmem, umma_desc(q_hi + off), umma_desc(t_lo + off), 1u);
-              umma_f16(d_tmem, umma_desc(q_lo + off), umma_desc(t_hi + off), 1u);
+              umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_hi + off), umma_desc<kLBO, kSBO>(t_hi + off), kIdesc, (uint32_t)((kb | k4) != 0));
+              umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_hi + off), umma_desc<kLBO, kSBO>(t_lo + off), kIdesc, 1u);
+              umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_lo + off), umma_desc<kLBO, kSBO>(t_hi + off), kIdesc, 1u);
             }
             umma_commit(&bar_empty[s]);                   // the ring slot is free once these MMAs have read it
             if (++s == kStages) { s = 0; ph ^= 1u; }
@@ -236,17 +190,8 @@ knn_dense_scan_kernel(const unsigned char* __restrict__ qpacked, const unsigned 
 #pragma unroll 1
         for (int c0 = 0; c0 < kBN; c0 += 32) {
           uint32_t v[32];
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-              "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-              "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-              : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-                "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-                "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-                "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-              : "r"(taddr + (uint32_t)c0)
-              : "memory");
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+          tmem_ld32(taddr + (uint32_t)c0, v);
+          tmem_ld_wait();
           const float4* tn4 = reinterpret_cast<const float4*>(tnorm + (size_t)tb * kBN + c0);
           const int base = tb * kBN + c0;
 #pragma unroll
@@ -275,7 +220,7 @@ knn_dense_scan_kernel(const unsigned char* __restrict__ qpacked, const unsigned 
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)kTmemCols) : "memory");
+    tmem_dealloc(tmem_base, kTmemCols);
   }
 }
 

@@ -12,16 +12,17 @@
 // certifies the top k against a bound on this kernel's evaluation error and sends a query to the exhaustive float64
 // rescan otherwise.  Neighbours and labels never depend on the reduced-precision arithmetic.
 //
-// One persistent CTA per SM, 320 threads:
+// One persistent CTA per SM, 576 threads:
 //   warp 0      TMA producer (cp.async.bulk, no tensor map: the pack kernels write tiles in the tensor core's canonical
 //               K-major no-swizzle layout, so a tile is ONE contiguous 8 KB copy): the CTA's 256 queries
 //               ({hi, lo} x 2 blocks of 128, double-buffered across work units) and a ring of 128-row train tiles
 //   warp 1      one thread issues tcgen05.mma.cta_group::1.kind::f16, M 128 x N 128 x K 16, six per train tile
 //               (2 query blocks x 3 split passes) into a double-buffered accumulator that fills TMEM
 //               (2 stages x 2 query blocks x 128 columns = 512); tcgen05.commit frees the ring slot and publishes the stage
-//   warps 2-9   epilogue, one query per thread (TMEM lane = query row): tcgen05.ld 32 columns at a time, software
-//               pipelined; a 3-input min tree gives the minimum of each 8 scores and of the 32; only when that beats
-//               some lane's 8th-best score does the warp reload the offending 8 columns and look at them one by one.
+//   warps 2-17  epilogue, one query per thread (TMEM lane = query row), two warps per (lane group, query block) on 64
+//               columns of every tile each: tcgen05.ld 32 columns at a time; a 3-input min tree gives the minimum of
+//               each 8 scores and of the 32; only when that beats some lane's 8th-best score does the warp reload the
+//               offending 8 columns and look at them one by one.
 //               After the first few thousand train rows that happens for a few columns in a thousand: the epilogue
 //               costs ~0.6 instructions per pair and the kernel is bound by the TMEM -> register path (4 B per pair).
 // A train tile (8 KB) serves 256 queries, which halves the L2 -> SM operand traffic per pair against one M = 128 block
@@ -31,7 +32,6 @@
 #include <algorithm>
 #include <climits>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <numeric>
 
@@ -40,6 +40,7 @@
 
 #include "kernels.cuh"
 #include "knn.cuh"
+#include "ptx.cuh"
 
 namespace dsp {
 
@@ -51,18 +52,9 @@ constexpr int kPlaneBytes = kRows * kK * 2;      // one fp16 plane of a tile: 4 
 constexpr int kTileBytes = 2 * kPlaneBytes;      // {hi, lo}: 8 KB
 constexpr int kUnitQ = 2 * kRows;                // queries per work unit
 constexpr int kQBufBytes = 2 * kTileBytes;       // two query blocks
-#ifndef DSP_TC16_SPLIT
-#define DSP_TC16_SPLIT 2            // epilogue warps per (TMEM lane group, query block): 1 = one warp on all 128 columns of a tile, 2 = two on 64 each
-#endif
-constexpr int kSplit = DSP_TC16_SPLIT;
-constexpr int kTStages = kSplit == 1 ? 18 : 16;                     // 144 KB of train tiles in flight; with the query buffers and the candidate lists the CTA owns its SM (all of TMEM is allocated)
-// kSplit 4 (experiment, kept compilable): the 16 epilogue warps of kSplit 2 on HALF tiles -- MMAs of N = 64, four
-// accumulator stages of 2 x 64 columns, a warp compares 32 columns per stage and loads the next stage's 32 while it does
-// (register double buffer).  Parity-green and slower: 1 M x 100 k in 25.0 ms against 20.1 ms -- twice the MMA issues,
-// commits and barrier round trips per pair cost more than the hidden TMEM-load latency returns.
-constexpr int kAccStages = kSplit == 4 ? 4 : 2;
-constexpr int kMmaN = kSplit == 4 ? 64 : kRows;           // train rows per MMA
-constexpr int kEpiWarps = kSplit == 1 ? 8 : 16;
+constexpr int kTStages = 16;                     // 128 KB of train tiles in flight; with the query buffers and the candidate lists the CTA owns its SM (all of TMEM is allocated)
+constexpr int kAccStages = 2;
+constexpr int kEpiWarps = 16;
 constexpr int kTcThreads = 32 * (2 + kEpiWarps);
 constexpr int kTmemCols = 512;
 constexpr int kEpiThreads = 32 * kEpiWarps;
@@ -72,81 +64,9 @@ constexpr size_t kTcSmem = 2 * kQBufBytes + (size_t)kTStages * kTileBytes + kLis
 // K of one 8-row group are adjacent (LBO = 128 B); row groups follow every 256 B (SBO)
 constexpr uint32_t kLBO = 128, kSBO = 256;
 // instruction descriptor (kind::f16): D = F32 (bit 4), A = B = F16, both K-major, N >> 3 at bit 17, M >> 4 at bit 24
-constexpr uint32_t kIdesc = (1u << 4) | ((uint32_t)(kMmaN >> 3) << 17) | ((uint32_t)(kRows >> 4) << 24);
+constexpr uint32_t kIdesc = (1u << 4) | ((uint32_t)(kRows >> 3) << 17) | ((uint32_t)(kRows >> 4) << 24);
 static_assert(8 * (4 + 2 * kTStages + 2 * kAccStages) + 8 <= 512, "barrier block of the shared-memory plan (unit slots at 512)");
 constexpr float kPadNorm = 30000.f;              // |t|^2 of padding rows: above every real score (knn_tc16_max_norm)
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)
-      : "memory");
-}
-// plain try_wait loop (no suspend-time hint): the waits of this kernel are a few hundred cycles long
-__device__ __forceinline__ void mbar_wait_spin(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-               "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr) {
-  return (uint64_t)((saddr >> 4) & 0x3fffu) | ((uint64_t)(kLBO >> 4) << 16) | ((uint64_t)(kSBO >> 4) << 32) | (1ull << 46);
-}
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(kIdesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "r"(taddr)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 __device__ __forceinline__ float min3f(float a, float b, float c) { return fminf(fminf(a, b), c); }
 __device__ __forceinline__ float min8(const uint32_t* v) {
@@ -220,25 +140,6 @@ __global__ void knn_tc16_pack_kernel(const double* __restrict__ x, int64_t rows,
 // ---------------------------------------------------------------------------------------
 // filter
 // ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void tmem_ld64(uint32_t taddr, uint32_t (&v)[64]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x64.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, "
-      "%32, %33, %34, %35, %36, %37, %38, %39, %40, %41, %42, %43, %44, %45, %46, %47, "
-      "%48, %49, %50, %51, %52, %53, %54, %55, %56, %57, %58, %59, %60, %61, %62, %63}, [%64];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31]), "=r"(v[32]),
-        "=r"(v[33]), "=r"(v[34]), "=r"(v[35]), "=r"(v[36]), "=r"(v[37]), "=r"(v[38]), "=r"(v[39]), "=r"(v[40]),
-        "=r"(v[41]), "=r"(v[42]), "=r"(v[43]), "=r"(v[44]), "=r"(v[45]), "=r"(v[46]), "=r"(v[47]), "=r"(v[48]),
-        "=r"(v[49]), "=r"(v[50]), "=r"(v[51]), "=r"(v[52]), "=r"(v[53]), "=r"(v[54]), "=r"(v[55]), "=r"(v[56]),
-        "=r"(v[57]), "=r"(v[58]), "=r"(v[59]), "=r"(v[60]), "=r"(v[61]), "=r"(v[62]), "=r"(v[63])
-      : "r"(taddr)
-      : "memory");
-}
-
 // The slow path: ONE out-of-line copy per list length.  A thread's candidate list lives in shared memory
 // ([entry][thread]: conflict-free), so the function takes nothing but scalars -- 8 scores, their first train row, the
 // current threshold -- and the 16 call sites of the epilogue (4 groups of 8 in each of 4 chunks of a tile) are a few
@@ -268,12 +169,10 @@ __device__ __noinline__ float tc16_slow8(float v0, float v1, float v2, float v3,
   return thr;
 }
 
-// kDebug (tuning experiments only, DSP_TC16_DEBUG): bit 0 = waits with a suspend-time hint, bit 1 = the epilogue reads
-// TMEM but compares nothing (wrong results: isolates the MMA / TMA pipeline)
 // kC: candidates kept per query (k + 2 for k <= 3, else 8): a shorter list is inserted into less often (C ln(n / C)
 // insertions per query, each executed by the whole warp for the one or two lanes that need it) and costs less per
 // insertion; the float64 certificate decides, per query, whether it was enough.
-template <int kDebug, int kC>
+template <int kC>
 __global__ void __launch_bounds__(kTcThreads, 1)
 knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned char* __restrict__ tpacked, int64_t m, int n,
                        int units, int t_tiles, const int* __restrict__ qflags, int* __restrict__ cand_idx,
@@ -296,21 +195,16 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
   // AND every epilogue warp's arrival on q_empty, so the epilogue reads the unit it is about to process
   int4* s_info = reinterpret_cast<int4*>(reinterpret_cast<unsigned char*>(bars) + 512);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  // the producer and the MMA thread wait for hundreds of cycles at a time: suspended waits (a spinning try_wait loop took 28 % of all
-  // issued instructions away from the epilogue warps that share their schedulers); kDebug bit 0 makes the epilogue spin instead
-  auto wait = [](uint64_t* bar, uint32_t parity) { mbar_wait(bar, parity); };
-  auto wait_epi = [](uint64_t* bar, uint32_t parity) { if constexpr (kDebug & 1) mbar_wait_spin(bar, parity); else mbar_wait(bar, parity); };
+  // every wait is the suspended form: the producer and the MMA thread wait for hundreds of cycles at a time, and a
+  // spinning try_wait loop took 28 % of all issued instructions away from the epilogue warps that share their schedulers
 
   if (tid == 0) {
     for (int i = 0; i < 2; ++i) { mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + kEpiWarps); }
     for (int i = 0; i < kTStages; ++i) { mbar_init(&t_full[i], 1); mbar_init(&t_empty[i], 1); }
     for (int i = 0; i < kAccStages; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], kEpiWarps); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"((uint32_t)kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, kTmemCols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -323,7 +217,7 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
       int qb = 0; uint32_t qph = 0;
       const bool lists = w.tiles && !(w.kept && *w.kept > w.kept_limit);
       for (int i = 0;; ++i) {
-        wait(&q_empty[qb], qph ^ 1u);
+        mbar_wait(&q_empty[qb], qph ^ 1u);
         const int slot = w.counter ? atomicAdd(w.counter, 1) : (int)blockIdx.x + i * (int)gridDim.x;
         const int u = slot < units ? (w.unit_order ? w.unit_order[slot] : slot) : -1;
         const int cnt = (u >= 0 && lists) ? w.tile_count[u] : t_tiles, list = (u >= 0 && lists) ? u * w.stride : -1;
@@ -335,7 +229,7 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
         int tb = cnt > 0 ? (list < 0 ? 0 : w.tiles[list]) : 0;
         for (int j = 0; j < cnt; ++j) {
           const int tb_next = j + 1 < cnt ? (list < 0 ? j + 1 : w.tiles[list + j + 1]) : 0;
-          wait(&t_empty[s], ph ^ 1u);
+          mbar_wait(&t_empty[s], ph ^ 1u);
           mbar_expect_tx(&t_full[s], (uint32_t)kTileBytes);
           bulk_g2s(smem_u32(s_t + (size_t)s * kTileBytes), tpacked + (size_t)tb * kTileBytes, kTileBytes, &t_full[s]);
           if (++s == kTStages) { s = 0; ph ^= 1u; }
@@ -349,47 +243,23 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
     if (lane == 0) {
       int s = 0, as = 0, qb = 0; uint32_t ph = 0, aph = 0, qph = 0;
       for (;;) {
-        wait(&q_full[qb], qph);
+        mbar_wait(&q_full[qb], qph);
         tc_fence_after();
         const int4 info = s_info[qb];
         if (info.x < 0) break;
         const uint32_t q0 = smem_u32(s_q + (size_t)qb * kQBufBytes);
         for (int tb = 0; tb < info.y; ++tb) {
-          if constexpr (kSplit == 4) {
-            // two half-tile steps of 64 train rows: row groups of 8 lie kSBO bytes apart in the K-major tile
-            wait(&t_full[s], ph);
-            const uint32_t t_base = smem_u32(s_t + (size_t)s * kTileBytes);
-#pragma unroll
-            for (int sub = 0; sub < 2; ++sub) {
-              wait(&acc_empty[as], aph ^ 1u);           // the epilogue has loaded this accumulator stage
-              tc_fence_after();
-              const uint32_t t_hi = t_base + (uint32_t)sub * (kMmaN / 8) * kSBO, t_lo = t_hi + kPlaneBytes;
-#pragma unroll
-              for (int h = 0; h < 2; ++h) {
-                const uint32_t q_hi = q0 + (uint32_t)h * kTileBytes, q_lo = q_hi + kPlaneBytes;
-                const uint32_t d_tmem = tmem_base + (uint32_t)(as * 2 * kMmaN + h * kMmaN);
-                umma_f16(d_tmem, umma_desc(q_hi), umma_desc(t_hi), 0u);
-                umma_f16(d_tmem, umma_desc(q_hi), umma_desc(t_lo), 1u);
-                umma_f16(d_tmem, umma_desc(q_lo), umma_desc(t_hi), 1u);
-              }
-              if (sub == 1) umma_commit(&t_empty[s]);               // ring slot free once these MMAs have read it
-              umma_commit(&acc_full[as]);
-              if (++as == kAccStages) { as = 0; aph ^= 1u; }
-            }
-            if (++s == kTStages) { s = 0; ph ^= 1u; }
-            continue;
-          }
-          wait(&acc_empty[as], aph ^ 1u);             // the epilogue has drained this accumulator stage
-          wait(&t_full[s], ph);
+          mbar_wait(&acc_empty[as], aph ^ 1u);             // the epilogue has drained this accumulator stage
+          mbar_wait(&t_full[s], ph);
           tc_fence_after();
           const uint32_t t_hi = smem_u32(s_t + (size_t)s * kTileBytes), t_lo = t_hi + kPlaneBytes;
 #pragma unroll
           for (int h = 0; h < 2; ++h) {
             const uint32_t q_hi = q0 + (uint32_t)h * kTileBytes, q_lo = q_hi + kPlaneBytes;
             const uint32_t d_tmem = tmem_base + (uint32_t)((as * 2 + h) * kRows);
-            umma_f16(d_tmem, umma_desc(q_hi), umma_desc(t_hi), 0u);
-            umma_f16(d_tmem, umma_desc(q_hi), umma_desc(t_lo), 1u);
-            umma_f16(d_tmem, umma_desc(q_lo), umma_desc(t_hi), 1u);
+            umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_hi), umma_desc<kLBO, kSBO>(t_hi), kIdesc, 0u);
+            umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_hi), umma_desc<kLBO, kSBO>(t_lo), kIdesc, 1u);
+            umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_lo), umma_desc<kLBO, kSBO>(t_hi), kIdesc, 1u);
           }
           umma_commit(&t_empty[s]);                         // ring slot free once these MMAs have read it
           umma_commit(&acc_full[as]);                       // both query blocks of this stage are complete
@@ -405,14 +275,14 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
     // ===== epilogue: TMEM lane group = warp % 4 (hardware rule); (warp - 2) / 4 picks the query block and, with two
     // warps per (lane group, query block), the 64-column half of every tile the warp compares =====
     const int lg = warp & 3, grp = (warp - 2) >> 2;
-    const int h = kSplit == 1 ? grp : grp >> 1, half = kSplit == 1 ? 0 : grp & 1;
+    const int h = grp >> 1, half = grp & 1;
     const int et = tid - 64;                                   // epilogue thread
     float* l_cd = reinterpret_cast<float*>(smem + 2 * kQBufBytes + (size_t)kTStages * kTileBytes + 1024) + et;     // behind the barrier block
     int* l_ci = reinterpret_cast<int*>(l_cd - et + kKnnCand * kEpiThreads) + et;
     const uint32_t lane_addr = tmem_base + ((uint32_t)(lg * 32) << 16);
     int as = 0, qb = 0; uint32_t aph = 0, qph = 0;
     for (;;) {
-      wait_epi(&q_full[qb], qph);
+      mbar_wait(&q_full[qb], qph);
       const int4 info = s_info[qb];
       __syncwarp();
       if (lane == 0) mbar_arrive(&q_empty[qb]);
@@ -435,7 +305,6 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
       // cache misses on every excursion) 170 ms; reloading the offending 8 columns from TMEM 33 ms; selects + rolled loop,
       // bubble sort 31 ms; 5-entry list + min/max network 22 ms; out-of-line slow path + 64-column loads: DESIGN.md.
       auto process = [&](const uint32_t* v, int idx0) {
-        if constexpr (kDebug & 2) { if (__uint_as_float(v[0]) == 12345.678f) thr = 0.f; return; }
         const float s0 = min8(v), s1 = min8(v + 8), s2 = min8(v + 16), s3 = min8(v + 24);
         if (fminf(fminf(s0, s1), fminf(s2, s3)) < thr) {
 #define DSP_TC16_GROUP(g, sg)                                                                                                     \
@@ -448,108 +317,45 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
         }
         __syncwarp();
       };
-      if constexpr (kSplit == 1) {
-        // two 64-column halves per tile, double-buffered ACROSS tiles: while one half is compared the other is in flight
-        uint32_t va[64], vb[64];
-        if (cnt > 0) {
-          wait_epi(&acc_full[as], aph);
-          tc_fence_after();
-          tmem_ld64(lane_addr + (uint32_t)((as * 2 + h) * kRows), va);
-        }
-        for (int tb = 0; tb < cnt; ++tb) {
-          const int base = tile_row(tb);
-          tmem_ld_wait();                                          // first half of tile tb is in registers
-          tmem_ld64(lane_addr + (uint32_t)((as * 2 + h) * kRows + 64), vb);
-          process(va, base);
-          process(va + 32, base + 32);
-          tmem_ld_wait();                                          // second half too: the accumulator stage can be reused
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&acc_empty[as]);
-          if (++as == kAccStages) { as = 0; aph ^= 1u; }
-          if (tb + 1 < cnt) {
-            wait_epi(&acc_full[as], aph);
-            tc_fence_after();
-            tmem_ld64(lane_addr + (uint32_t)((as * 2 + h) * kRows), va);     // first half of the next tile
-          }
-          process(vb, base + 64);
-          process(vb + 32, base + 96);
-        }
-      } else if constexpr (kSplit == 4) {
-        // half-tile stages: 32 columns per warp and stage, the next stage's 32 in flight while these are compared
-        uint32_t va[32], vb[32];
-        auto stage_col = [&](int st) { return (uint32_t)(st * 2 * kMmaN + h * kMmaN + half * 32); };
-        if (cnt > 0) {
-          wait_epi(&acc_full[as], aph);
-          tc_fence_after();
-          tmem_ld32(lane_addr + stage_col(as), va);
-        }
-        for (int tb = 0; tb < cnt; ++tb) {
-          const int base = tile_row(tb) + half * 32;
-          tmem_ld_wait();                                          // (tb, rows 0..63) is in registers
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&acc_empty[as]);
-          if (++as == kAccStages) { as = 0; aph ^= 1u; }
-          wait_epi(&acc_full[as], aph);
-          tc_fence_after();
-          tmem_ld32(lane_addr + stage_col(as), vb);                 // (tb, rows 64..127)
-          process(va, base);
-          tmem_ld_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&acc_empty[as]);
-          if (++as == kAccStages) { as = 0; aph ^= 1u; }
-          if (tb + 1 < cnt) {
-            wait_epi(&acc_full[as], aph);
-            tc_fence_after();
-            tmem_ld32(lane_addr + stage_col(as), va);               // (tb + 1, rows 0..63)
-          }
-          process(vb, base + 64);
-        }
-      } else {
-        // Two warps per (lane group, query block), each on its own 64 columns of every tile with its own candidate list:
-        // four epilogue warps per scheduler hide one another's TMEM-load and min-tree latencies (with two, issue slots
-        // were 28 % busy and the tensor pipe 20 %), the accumulator stage goes back to the MMA thread as soon as the 64
-        // scores are in registers, and the two lists are merged once per work unit.
-        uint32_t va[32], vb[32];
-        int row_next = cnt > 0 ? tile_row(0) : 0;
-        for (int tb = 0; tb < cnt; ++tb) {
-          const int base = row_next + half * 64;
-          if (tb + 1 < cnt) row_next = tile_row(tb + 1);
-          wait_epi(&acc_full[as], aph);
-          tc_fence_after();
-          const uint32_t col = (uint32_t)((as * 2 + h) * kRows + half * 64);
-          tmem_ld32(lane_addr + col, va);
-          tmem_ld32(lane_addr + col + 32, vb);
-          tmem_ld_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&acc_empty[as]);
-          if (++as == kAccStages) { as = 0; aph ^= 1u; }
-          process(va, base);
-          process(vb, base + 32);
-        }
+      // Two warps per (lane group, query block), each on its own 64 columns of every tile with its own candidate list:
+      // four epilogue warps per scheduler hide one another's TMEM-load and min-tree latencies (with two, issue slots
+      // were 28 % busy and the tensor pipe 20 %), the accumulator stage goes back to the MMA thread as soon as the 64
+      // scores are in registers, and the two lists are merged once per work unit.
+      uint32_t va[32], vb[32];
+      int row_next = cnt > 0 ? tile_row(0) : 0;
+      for (int tb = 0; tb < cnt; ++tb) {
+        const int base = row_next + half * 64;
+        if (tb + 1 < cnt) row_next = tile_row(tb + 1);
+        mbar_wait(&acc_full[as], aph);
+        tc_fence_after();
+        const uint32_t col = (uint32_t)((as * 2 + h) * kRows + half * 64);
+        tmem_ld32(lane_addr + col, va);
+        tmem_ld32(lane_addr + col + 32, vb);
+        tmem_ld_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&acc_empty[as]);
+        if (++as == kAccStages) { as = 0; aph ^= 1u; }
+        process(va, base);
+        process(vb, base + 32);
       }
-      if constexpr (kSplit >= 2) {
-        // merge: the warp of half 0 folds its partner's list (same lane group, same query block: 128 threads up) into its own
-        const int pair_bar = 1 + lg + 4 * h;
-        asm volatile("bar.sync %0, 64;" ::"r"(pair_bar) : "memory");
-        if (half == 0) {
-          float cd[kC]; int ci[kC];
+      // merge: the warp of half 0 folds its partner's list (same lane group, same query block: 128 threads up) into its own
+      const int pair_bar = 1 + lg + 4 * h;
+      bar_sync(pair_bar, 64);
+      if (half == 0) {
+        float cd[kC]; int ci[kC];
 #pragma unroll
-          for (int c = 0; c < kC; ++c) { cd[c] = l_cd[c * kEpiThreads]; ci[c] = l_ci[c * kEpiThreads]; }
+        for (int c = 0; c < kC; ++c) { cd[c] = l_cd[c * kEpiThreads]; ci[c] = l_ci[c * kEpiThreads]; }
 #pragma unroll
-          for (int b = 0; b < kC; ++b) {
-            float d = l_cd[b * kEpiThreads + 128]; int i = l_ci[b * kEpiThreads + 128];
+        for (int b = 0; b < kC; ++b) {
+          float d = l_cd[b * kEpiThreads + 128]; int i = l_ci[b * kEpiThreads + 128];
 #pragma unroll
-            for (int c = 0; c < kC; ++c) {          // sorted insertion: carry the displaced entry down the list
-              if (d < cd[c]) { const float td = cd[c]; const int ti = ci[c]; cd[c] = d; ci[c] = i; d = td; i = ti; }
-            }
+          for (int c = 0; c < kC; ++c) {          // sorted insertion: carry the displaced entry down the list
+            if (d < cd[c]) { const float td = cd[c]; const int ti = ci[c]; cd[c] = d; ci[c] = i; d = td; i = ti; }
           }
-#pragma unroll
-          for (int c = 0; c < kC; ++c) { l_cd[c * kEpiThreads] = cd[c]; l_ci[c * kEpiThreads] = ci[c]; }
         }
+#pragma unroll
+        for (int c = 0; c < kC; ++c) { l_cd[c * kEpiThreads] = cd[c]; l_ci[c * kEpiThreads] = ci[c]; }
       }
       if (half == 0 && q_idx >= 0) {
 #pragma unroll
@@ -559,17 +365,15 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
         }
         cand_worst[q_idx] = l_cd[(kC - 1) * kEpiThreads];
       }
-      if constexpr (kSplit >= 2) {
-        // the partner must not re-initialise its list for the next unit before it has been read
-        asm volatile("bar.sync %0, 64;" ::"r"(1 + lg + 4 * h) : "memory");
-      }
+      // the partner must not re-initialise its list for the next unit before it has been read
+      bar_sync(pair_bar, 64);
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)kTmemCols) : "memory");
+    tmem_dealloc(tmem_base, kTmemCols);
   }
 }
 
@@ -803,11 +607,7 @@ cudaError_t knn_tc16_filter(const void* qpacked, const void* tpacked, int64_t m,
                             float* cand_worst, int sm_count, cudaStream_t st, const float* thr0, const Tc16Work& work) {
   if (m == 0) return cudaSuccess;
   const int units = (int)(knn_tc16_padded_rows(m, true) / kUnitQ), t_tiles = (int)(knn_tc16_padded_rows(n, false) / kRows);
-  static const int debug = [] { const char* e = std::getenv("DSP_TC16_DEBUG"); return e ? std::atoi(e) & 3 : 0; }();
-  static const int force_c = [] { const char* e = std::getenv("DSP_TC16_CAND"); return e ? std::atoi(e) : 0; }();
-  const bool small = force_c ? force_c < kKnnCand : k <= 3;
-  auto fn = debug == 1 ? knn_tc16_filter_kernel<1, 5> : debug == 2 ? knn_tc16_filter_kernel<2, 5> : debug == 3 ? knn_tc16_filter_kernel<3, 5>
-            : (small ? knn_tc16_filter_kernel<0, 5> : knn_tc16_filter_kernel<0, kKnnCand>);
+  auto fn = k <= 3 ? knn_tc16_filter_kernel<5> : knn_tc16_filter_kernel<kKnnCand>;
   cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem);
   if (e != cudaSuccess) return e;
   const int grid = units < sm_count ? units : sm_count;

@@ -5,7 +5,7 @@ VIADDMNMX / VIMNMX3, packed fp32 = FFMA2 / FADD2 / FMUL2, warp reductions = REDU
 occurrence of each as a sample line.  Usage: sass_excerpt.py [lib.so] > profiles/r02_sass_excerpt.txt"""
 import collections, os, re, subprocess, sys
 lib = sys.argv[1] if len(sys.argv) > 1 else os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "dsp_audioreclabs_b200", "libdspfront.so")
-HOT = ["frontend_pipe_kernelILb1", "frontend_pipe_kernelILb0", "knn_tc16_filter_kernelILi0ELi5", "knn_dense_scan_kernel", "knn_scan_pair_kernel",
+HOT = ["frontend_pipe_kernelILb1", "frontend_pipe_kernelILb0", "knn_tc16_filter_kernelILi5E", "knn_dense_scan_kernel", "knn_scan_pair_kernel",
        "knn_refine_collect_kernel", "frontend_pcm_kernel", "frontend_exact_kernel", "dtw_kernel", "mfcc_kernel"]
 KEYS = ["UTCHMMA", "LDTM", "UTCBAR", "UTCATOMSWS", "UBLKCP", "SYNCS", "IDP.4A", "VIADDMNMX", "VIMNMX3", "FFMA2", "FADD2", "FMUL2", "FFMA", "DFMA", "DADD",
         "REDUX", "SHFL", "POPC", "LDS", "STS", "LDG", "STG", "BAR", "USETMAXREG", "PRMT", "HMMA"]
