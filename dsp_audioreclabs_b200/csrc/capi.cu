@@ -74,6 +74,8 @@ constexpr size_t kMaxSmemPerCta = 227 * 1024;
 constexpr int64_t kFastMaxLen = 1 << 20;          // exact-integer bounds of the fast kernel
 constexpr int kKnnDenseMaxDim = 16384;            // feature dimensions served by the tensor-core scan
 constexpr int64_t kKnnDenseQueryChunk = 32768;    // queries packed per scan launch
+// candidate scan of a KNN handle, numbered as dsp_knn_last_stats reports it
+enum KnnScan { kScanF64 = 0, kScanFp32 = 1, kScanDense = 2, kScanTc16 = 3 };
 constexpr size_t kHostChunkBytesDefault = 512u << 20;    // samples per staged chunk of the host pipeline (DSP_HOST_CHUNK_MB overrides): 96 MB 550 k audio-s/s end to end, 512 MB 586 k, 2 GB 592 k (pinned H2D alone: 55.6 GB/s = 630 k)
 static size_t host_chunk_bytes() {
   static const size_t v = [] { const char* e = std::getenv("DSP_HOST_CHUNK_MB"); const long mb = e ? std::atol(e) : 0; return mb >= 1 && mb <= 4096 ? (size_t)mb << 20 : kHostChunkBytesDefault; }();
@@ -114,6 +116,7 @@ struct dsp_context {
   const float* win32 = nullptr;
   DevBuf counters;   // [0] work counter (u32)  [1] flag count (i32)
   DevBuf flag_list, zbuf, seqbuf;
+  DevBuf prof;       // DSP_PROF phase counters of the fast kernels
   size_t occ_smem = 0;
   int occ_variant = -1;
   int pcm_variant = -1;         // -1 automatic; else a build of frontend_pcm.cu's kVariants (dsp_set_tuning / DSP_PCM_VARIANT)
@@ -130,8 +133,9 @@ struct dsp_knn {
   int64_t n = 0, index_base = 0;
   int d = 0, dp = 0, k = 0;
   float tnorm_max = 0.f;
-  bool dense = false;          // tensor-core candidate scan (knn_dense.cu): feature dimension beyond the tiled scan
-  bool tc16 = false;           // d <= 15: tensor-core candidate filter (knn_tc16.cu); the fp32 tiled scan stands in when a value leaves its range
+  // candidate scan, decided at fit: a train value outside the range of the tensor-core filter (knn_tc16.cu) / the dense
+  // scan (knn_dense.cu) sends every call to the fp32 tiled / the float64 scan instead
+  KnnScan scan = kScanF64;
   DevBuf tc_train, tc_train_rows, tc_q, tc_flags;      // train packed in tile order / in row order (knn_prune 0)
   DevBuf train64, train32, labels, tnorm, cand_idx, cand_worst, qnorm, redo_list, redo_count, nbr_label, q, o_idx, o_dist, o_lab;
   DevBuf refine_list, refine_thr, surv_count, surv_rows;     // second pass of the D <= 15 path (knn_refine)
@@ -229,6 +233,77 @@ int launch_exact(dsp_context* c, const void* samples, int dtype, const int64_t* 
   return DSP_OK;
 }
 
+// Kernel route of one front-end batch (DESIGN §3.1b), first match wins:
+//   not int16 mono, force_exact, a float64 output, max_len > 2^20 or no feat_offsets  -> float64 replay
+//   pcm_variant -1 or 10 and pipe_kernel_plan fits                                    -> frontend_pipe_kernel
+//   pcm_variant 0..9                                                                  -> that frontend_pcm_kernel build
+//   otherwise                                         -> build 2 (streaming) for aligned16 batches, else build 0 (resident)
+//   the build fits no CTA on an SM (static + dynamic shared memory)                   -> float64 replay
+// Alone, the replay runs on a grid of 4 x SMs and writes the float64 outputs; behind a fast kernel it runs on one CTA per
+// SM and replays only the utterances that kernel flagged.
+struct FrontRoute {
+  enum Kind { kReplay, kPipe, kPcm } kind = kReplay;
+  int build = 0;             // kPcm: index into frontend_pcm.cu's kVariants
+  PipePlan plan{};           // kPipe
+  int cap_samples = 0;       // kPcm
+  size_t smem = 0;
+  int grid = 0, replay_grid = 0;
+};
+
+FrontRoute route_frontend(dsp_context* c, int dtype, const int64_t* feat_offsets, int64_t B, int64_t max_len,
+                          int cap_frames, const dsp_frontend_params* p, bool want64) {
+  FrontRoute r;
+  const int64_t sms = c->sm_count;
+  r.replay_grid = (int)std::min<int64_t>(B, sms * 4);
+  if (dtype != DSP_S16 || p->channels != 1 || p->force_exact || want64 || max_len > kFastMaxLen || !feat_offsets) return r;
+  const int knob = c->pcm_variant, pipe_knob = pcm_num_variants();
+  // the pipelined kernel first: 2.2-5x faster than build 0 on every geometry whose per-utterance records fit (DESIGN §3.1c)
+  if ((knob < 0 || knob == pipe_knob) && pipe_kernel_plan(max_len, cap_frames, p->frame_length, kMaxSmemPerCta, &r.plan)) {
+    r.kind = FrontRoute::kPipe;
+    r.smem = r.plan.smem;
+    r.grid = r.replay_grid = (int)std::min<int64_t>(B, sms);
+    return r;
+  }
+  constexpr int kAutoStream = 2, kAutoResident = 0;
+  r.build = knob >= 0 && knob < pipe_knob ? knob : (knob < 0 && p->aligned16 ? kAutoStream : kAutoResident);
+  r.cap_samples = (int)((std::max<int64_t>(max_len, 1) + 63) / 64 * 64);
+  r.smem = pcm_kernel_smem_bytes(r.cap_samples, cap_frames, p->frame_length, !pcm_variant_streams(r.build));
+  if (c->occ_smem != r.smem || c->occ_variant != r.build) {
+    c->occ = pcm_kernel_max_ctas_per_sm(r.build, r.smem, c->smem_optin);
+    c->occ_smem = r.smem;
+    c->occ_variant = r.build;
+  }
+  if (c->occ < 1) return r;
+  r.kind = FrontRoute::kPcm;
+  r.grid = (int)std::min<int64_t>(B, sms * c->occ);
+  r.replay_grid = (int)std::min<int64_t>(B, sms);
+  return r;
+}
+
+// DSP_PROF: per-phase cycle counters of the fast kernels, printed to stderr after every launch (tools/cmp_variants.sh
+// reads these lines).  Returns the zeroed counters, or nullptr when DSP_PROF is unset.
+long long* prof_begin(dsp_context* c) {
+  if (!std::getenv("DSP_PROF") || c->prof.ensure(16 * sizeof(long long)) != cudaSuccess) return nullptr;
+  cudaMemsetAsync(c->prof.p, 0, 16 * sizeof(long long), c->stream);
+  return c->prof.as<long long>();
+}
+
+void prof_report(dsp_context* c, const FrontRoute& r) {
+  long long h[16];
+  cudaMemcpyAsync(h, c->prof.p, sizeof h, cudaMemcpyDeviceToHost, c->stream);
+  cudaStreamSynchronize(c->stream);
+  if (r.kind == FrontRoute::kPipe) {
+    const char* nm[12] = {"S.wait_full", "S.passA", "S.bar1", "S.passB", "S.bar2", "S.wait_rec", "S.passF", "-", "T.wait", "T.decide", "T.window", "T.stats+out"};
+    fprintf(stderr, "[prof pipe R=%d nrec=%d] utterances=%lld (cycles/utt, stream warp 0 / tail warp 0 x nrec)", r.plan.ring_slots, r.plan.n_rec, h[15]);
+    for (int i = 0; i < 12; ++i) fprintf(stderr, "  %s=%.0f", nm[i], (double)h[i] / (double)std::max<long long>(h[15], 1) * (i >= 8 ? r.plan.n_rec : 1));
+    fprintf(stderr, "\n");
+  } else {
+    const char* nm[12] = {"load_wait", "P1", "feat_empty_wait", "P2", "P2b", "P3tail(searches)", "P4", "fixup+handoff", "P3a(select passes)", "P3b(gather)", "P3c(rank+thresholds)", "P3d(N3N4)"};
+    double tot = 0; for (int i = 0; i < 12; ++i) tot += (double)h[i];
+    fprintf(stderr, "[prof] utterances=%lld", h[15]); for (int i = 0; i < 12; ++i) fprintf(stderr, "  %s=%.0f", nm[i], (double)h[i] / (double)h[15]); fprintf(stderr, "  total=%.0f cycles/utt\n", tot / (double)h[15]);
+  }
+}
+
 int frontend_device(dsp_context* c, const void* samples, int dtype, const int64_t* offsets, const int32_t* lengths,
                     const int64_t* feat_offsets, const int64_t* epd_offsets, int64_t B, int64_t max_len,
                     const dsp_frontend_params* p, const dsp_frontend_outputs* out) {
@@ -245,8 +320,7 @@ int frontend_device(dsp_context* c, const void* samples, int dtype, const int64_
   if ((out->epd_energy || out->epd_zcr) && !epd_offsets) return fail(DSP_ERR_INVALID, "epd_offsets is NULL");
   rc = ensure_window(c, p->window, p->frame_length);
   if (rc) return rc;
-  const int fl = p->frame_length, fs = p->frame_shift;
-  const int64_t cap_frames64 = std::max<int64_t>(frame_count_host_device(max_len, fl, fs), 1);
+  const int cap_frames = (int)std::max<int64_t>(frame_count_host_device(max_len, p->frame_length, p->frame_shift), 1);
 
   const bool want64 = out->energy_f64 || out->magnitude_f64 || out->zcr_f64 || out->stats_f64 || out->epd_zcr_f64 || out->frames_f64;
   if (out->frames_f64 && !feat_offsets) return fail(DSP_ERR_INVALID, "feat_offsets is NULL");
@@ -254,122 +328,39 @@ int frontend_device(dsp_context* c, const void* samples, int dtype, const int64_
     return fail(DSP_ERR_INVALID, "energy_f64, magnitude_f64 and zcr_f64 are written together: pass all three or none");
   if (out->energy_f64 && !feat_offsets) return fail(DSP_ERR_INVALID, "feat_offsets is NULL");
   if (out->epd_zcr_f64 && !epd_offsets) return fail(DSP_ERR_INVALID, "epd_offsets is NULL");
-  bool fast = dtype == DSP_S16 && p->channels == 1 && !p->force_exact && !want64 && max_len <= kFastMaxLen &&
-              feat_offsets;
-  size_t smem = 0;
-  int cap_samples = 0;
-  // automatic choice: the streaming build when the caller vouches for 16-byte aligned utterances,
-  // the shared-memory-resident build (any alignment) otherwise
-  constexpr int kAutoStream = 2, kAutoResident = 0;
-  int variant = (c->pcm_variant >= 0 && c->pcm_variant < pcm_num_variants()) ? c->pcm_variant : (p->aligned16 ? kAutoStream : kAutoResident);
-  if (pcm_variant_streams(variant) && !p->aligned16 && c->pcm_variant < 0) variant = kAutoResident;
-  // the pipelined kernel (frontend_pipe.cu): automatic for its geometries, or forced by the
-  // tuning knob (pcm_variant == pcm_num_variants())
-  const int kPipeVariant = pcm_num_variants();
-  PipePlan plan{};
-  // automatic choice: the pipelined kernel (frontend_pipe.cu) for every geometry its shared-memory plan fits -- any
-  // frame length / shift (frames that are not whole 64-sample groups take its ragged-edge forms), any utterance
-  // alignment.  tools/config_sweep.py, ms per 20k packed 1 s utterances, resident vs pipelined: 256/128 2.85 vs 0.71,
-  // 1102/441 (the reference's default) 3.73 vs 1.41, 512/256 2.79 vs 0.99, 2048/1024 5.71 vs 1.03, 2205/441 8.55 vs 1.83,
-  // 1102/1323 3.32 vs 1.18.  Geometries with very many frames per utterance (hops under ~100 samples at 1 s) do not fit
-  // its per-utterance records and stay on frontend_pcm_kernel.
-  bool pipe = fast && (c->pcm_variant == kPipeVariant || c->pcm_variant < 0) &&
-              pipe_kernel_plan(max_len, (int)cap_frames64, fl, kMaxSmemPerCta, &plan);
-  if (fast && !pipe && c->pcm_variant == kPipeVariant) variant = kAutoResident;
-  if (pipe) {
+  const FrontRoute r = route_frontend(c, dtype, feat_offsets, B, max_len, cap_frames, p, want64);
+  ExactExtras ex;
+  PcmArgs a{};                // flag_list stays NULL on the replay route: the replay takes the whole batch
+  if (r.kind == FrontRoute::kReplay) {
+    ex.feat_f64[0] = out->energy_f64; ex.feat_f64[1] = out->magnitude_f64; ex.feat_f64[2] = out->zcr_f64;
+    ex.stats_f64 = out->stats_f64; ex.epd_zcr_f64 = out->epd_zcr_f64; ex.frames_out = out->frames_f64;
+  } else {
     CU(c->counters.ensure(64));
     CU(c->flag_list.ensure(sizeof(int32_t) * (size_t)B));
     CU(cudaMemsetAsync(c->counters.p, 0, 64, c->stream));
-    PcmArgs a{};
     a.samples = reinterpret_cast<const int16_t*>(samples);
     a.offsets = offsets; a.lengths = lengths; a.feat_offsets = feat_offsets; a.epd_offsets = epd_offsets;
-    a.n_utts = B; a.fl = fl; a.fs = fs; a.window = p->window; a.do_epd = p->do_endpoint_detection;
+    a.n_utts = B; a.fl = p->frame_length; a.fs = p->frame_shift; a.window = p->window; a.do_epd = p->do_endpoint_detection;
     a.hr = p->energy_high_ratio; a.lr = p->energy_low_ratio; a.zr = p->zcr_threshold_ratio;
     a.win_f32 = c->win32;
-    a.cap_frames = (int)cap_frames64;
-    a.tma_chunk = std::getenv("DSP_PIPE_DEBUG") ? std::atoi(std::getenv("DSP_PIPE_DEBUG")) : 0;   // debug switches, 0 in production
-    a.ring_slots = plan.ring_slots; a.n_rec = plan.n_rec; a.cap_groups = plan.cap_groups;
+    a.cap_samples = r.cap_samples; a.cap_frames = cap_frames;
+    a.tma_chunk = c->tma_chunk;
+    a.stagger_ns = c->stagger_ns;
     a.sm_count = c->sm_count;
+    a.ring_slots = r.plan.ring_slots; a.n_rec = r.plan.n_rec; a.cap_groups = r.plan.cap_groups;
+    a.prof = prof_begin(c);
     a.work_counter = c->counters.as<unsigned int>();
     a.flag_count = c->counters.as<int32_t>() + 1;
     a.flag_list = c->flag_list.as<int32_t>();
     a.out = *out;
-    const int grid = (int)std::min<int64_t>(B, (int64_t)c->sm_count);
-    static long long* d_prof = nullptr;
-    if (std::getenv("DSP_PROF")) {
-      if (!d_prof) cudaMalloc(&d_prof, 16 * sizeof(long long));
-      cudaMemsetAsync(d_prof, 0, 16 * sizeof(long long), c->stream);
-      a.prof = d_prof;
-    }
-    CU(launch_frontend_pipe(a, grid, plan.smem, c->stream));
-    if (a.prof) {
-      long long h[16]; cudaMemcpyAsync(h, d_prof, sizeof h, cudaMemcpyDeviceToHost, c->stream); cudaStreamSynchronize(c->stream);
-      const char* nm[12] = {"S.wait_full", "S.passA", "S.bar1", "S.passB", "S.bar2", "S.wait_rec", "S.passF", "-", "T.wait", "T.decide", "T.window", "T.stats+out"};
-      fprintf(stderr, "[prof pipe R=%d nrec=%d] utterances=%lld (cycles/utt, stream warp 0 / tail warp 0 x nrec)", plan.ring_slots, plan.n_rec, h[15]);
-      for (int i = 0; i < 12; ++i) fprintf(stderr, "  %s=%.0f", nm[i], (double)h[i] / (double)std::max<long long>(h[15], 1) * (i >= 8 ? plan.n_rec : 1));
-      fprintf(stderr, "\n");
-    }
+    if (r.kind == FrontRoute::kPipe) CU(launch_frontend_pipe(a, r.grid, r.smem, c->stream));
+    else CU(launch_frontend_pcm(r.build, a, r.grid, r.smem, c->stream));
+    if (a.prof) prof_report(c, r);
     c->launches++;
-    ExactExtras ex;
-    const int xgrid = (int)std::min<int64_t>(B, (int64_t)c->sm_count);
-    return launch_exact(c, samples, dtype, offsets, lengths, feat_offsets, epd_offsets, a.flag_list, a.flag_count, 0,
-                        max_len, p, out, ex, xgrid);
   }
-  if (fast) {
-    cap_samples = (int)((std::max<int64_t>(max_len, 1) + 63) / 64 * 64);
-    smem = pcm_kernel_smem_bytes(cap_samples, (int)cap_frames64, fl, !pcm_variant_streams(variant));
-    if (c->occ_smem != smem || c->occ_variant != variant) {
-      c->occ = pcm_kernel_max_ctas_per_sm(variant, smem, c->smem_optin);
-      c->occ_smem = smem;
-      c->occ_variant = variant;
-    }
-    // static + dynamic shared memory beyond the per-block maximum: the float64 replay takes the batch
-    if (c->occ < 1) fast = false;
-  }
-  if (!fast) {
-    const int grid = (int)std::min<int64_t>(B, (int64_t)c->sm_count * 4);
-    ExactExtras ex;
-    ex.feat_f64[0] = out->energy_f64; ex.feat_f64[1] = out->magnitude_f64; ex.feat_f64[2] = out->zcr_f64;
-    ex.stats_f64 = out->stats_f64; ex.epd_zcr_f64 = out->epd_zcr_f64; ex.frames_out = out->frames_f64;
-    return launch_exact(c, samples, dtype, offsets, lengths, feat_offsets, epd_offsets, nullptr, nullptr, B, max_len,
-                        p, out, ex, grid);
-  }
-  CU(c->counters.ensure(64));
-  CU(c->flag_list.ensure(sizeof(int32_t) * (size_t)B));
-  CU(cudaMemsetAsync(c->counters.p, 0, 64, c->stream));
-  PcmArgs a{};
-  a.samples = reinterpret_cast<const int16_t*>(samples);
-  a.offsets = offsets; a.lengths = lengths; a.feat_offsets = feat_offsets; a.epd_offsets = epd_offsets;
-  a.n_utts = B; a.fl = fl; a.fs = fs; a.window = p->window; a.do_epd = p->do_endpoint_detection;
-  a.hr = p->energy_high_ratio; a.lr = p->energy_low_ratio; a.zr = p->zcr_threshold_ratio;
-  a.win_f32 = c->win32;
-  a.cap_samples = cap_samples; a.cap_frames = (int)cap_frames64;
-  a.tma_chunk = c->tma_chunk;
-  a.stagger_ns = c->stagger_ns;
-  a.sm_count = c->sm_count;
-  a.prof = nullptr;
-  static long long* d_prof = nullptr;
-  if (std::getenv("DSP_PROF")) {
-    if (!d_prof) cudaMalloc(&d_prof, 16 * sizeof(long long));
-    cudaMemsetAsync(d_prof, 0, 16 * sizeof(long long), c->stream);
-    a.prof = d_prof;
-  }
-  a.work_counter = c->counters.as<unsigned int>();
-  a.flag_count = c->counters.as<int32_t>() + 1;
-  a.flag_list = c->flag_list.as<int32_t>();
-  a.out = *out;
-  const int grid = (int)std::min<int64_t>(B, (int64_t)c->sm_count * c->occ);
-  CU(launch_frontend_pcm(variant, a, grid, smem, c->stream));
-  if (a.prof) { long long h[16]; cudaMemcpyAsync(h, d_prof, sizeof h, cudaMemcpyDeviceToHost, c->stream); cudaStreamSynchronize(c->stream);
-    const char* nm[12] = {"load_wait", "P1", "feat_empty_wait", "P2", "P2b", "P3tail(searches)", "P4", "fixup+handoff", "P3a(select passes)", "P3b(gather)", "P3c(rank+thresholds)", "P3d(N3N4)"};
-    double tot = 0; for (int i = 0; i < 12; ++i) tot += (double)h[i];
-    fprintf(stderr, "[prof] utterances=%lld", h[15]); for (int i = 0; i < 12; ++i) fprintf(stderr, "  %s=%.0f", nm[i], (double)h[i] / (double)h[15]); fprintf(stderr, "  total=%.0f cycles/utt\n", tot / (double)h[15]); }
-  c->launches++;
-  // float64 replay of the utterances whose threshold margins could not be certified
-  ExactExtras ex;
-  const int xgrid = (int)std::min<int64_t>(B, (int64_t)c->sm_count);
-  return launch_exact(c, samples, dtype, offsets, lengths, feat_offsets, epd_offsets, a.flag_list, a.flag_count, 0,
-                      max_len, p, out, ex, xgrid);
+  // behind a fast kernel: float64 replay of the utterances whose threshold margins could not be certified
+  return launch_exact(c, samples, dtype, offsets, lengths, feat_offsets, epd_offsets, a.flag_list, a.flag_count,
+                      a.flag_list ? 0 : B, max_len, p, out, ex, r.replay_grid);
 }
 
 // small helper for the single-signal host entry points
@@ -439,7 +430,7 @@ int dsp_destroy(dsp_context* c) {
   for (auto& b : c->tmp) b.release();
   for (auto* e : c->windows) { e->w64.release(); e->w32.release(); delete e; }
   c->windows.clear();
-  c->counters.release(); c->flag_list.release();
+  c->counters.release(); c->flag_list.release(); c->prof.release();
   c->zbuf.release(); c->seqbuf.release();
   if (c->own) cudaStreamDestroy(c->own);
   if (c->s_in) cudaStreamDestroy(c->s_in);
@@ -920,11 +911,9 @@ int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* label
   }
   cudaError_t e = cudaStreamSynchronize(c->stream);
   if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "knn fit: %s", cudaGetErrorString(e)));
-  h->tc16 = h->tc_train.p && tc_flags[1] == 0;      // a train row outside the filter's range: fp32 scan for every call
-  if (h->tpacked.p) {
-    std::memcpy(&h->tnorm_max, &dense_flags[0], sizeof(float));
-    h->dense = dense_flags[1] == 0;          // a value outside the fp16 range: every query takes the float64 scan instead
-  }
+  if (h->tpacked.p) std::memcpy(&h->tnorm_max, &dense_flags[0], sizeof(float));
+  if (h->dp) h->scan = h->tc_train.p && tc_flags[1] == 0 ? kScanTc16 : kScanFp32;
+  else h->scan = h->tpacked.p && dense_flags[1] == 0 ? kScanDense : kScanF64;
   *out = h;
   return DSP_OK;
 }
@@ -956,6 +945,71 @@ int dsp_knn_topk_device(dsp_knn* h, const double* q, int64_t m, int64_t* nbr_idx
   return dsp_knn_topk_bounded_device(h, q, m, nullptr, nbr_idx, nbr_sqdist, nbr_label);
 }
 
+// What a candidate stage leaves for the certificate tail of dsp_knn_topk_bounded_device (knn_rerank / knn_refine)
+struct KnnStage {
+  double err_rel = 0.0, err_floor = 0.0;     // error bound of the candidate scores
+  float qnorm_limit = 0.f;                   // > 0: queries with a larger |q|^2 were scored as the zero vector
+  const float* thr0 = nullptr;               // per-query start thresholds of the filter
+  const double* rerank_bound = nullptr;      // per-query radius the candidates are certified against
+  bool allow_short = false;                  // fewer than k rows inside the radius is an answer
+  bool redo_all = false;                     // no candidates: every query takes the exhaustive float64 scan
+  int refine_cap = 0;                        // rejected queries the second pass (knn_refine) takes
+  int launches = 0;
+  const unsigned long long* prune_kept = nullptr;    // (DSP_KNN_DEBUG report)
+  int64_t prune_visits = 0;
+};
+
+// Tensor-core filter.  A query outside its range (|q|^2 above knn_tc16_max_norm(), NaN / inf) is scored as the zero
+// vector there and handed to the exhaustive float64 scan by the rerank kernel -- per query, on the device.
+static int knn_stage_tc16(dsp_knn* h, const double* q, int64_t m, const double* bound, KnnStage& s) {
+  dsp_context* c = h->ctx;
+  CU(h->tc_q.ensure(knn_tc16_packed_bytes(m, true)));
+  int* qflags = h->tc_flags.as<int>() + 4;
+  s.err_rel = knn_dense_err_rel(16);
+  s.err_floor = 1.0;
+  s.qnorm_limit = knn_tc16_max_norm();
+  Tc16Work work;
+  const void* tpacked = h->tc_train_rows.p;
+  const int64_t visits = knn_tc16_padded_rows(m, true) / kTc16UnitQueries * h->prune_tiles;
+  if (c->knn_prune && visits <= INT32_MAX) {          // (the tile lists take units x tiles ints, indexed in int)
+    // tile pruning: queries in curve order, a seed pass bounds every query's k-th distance U (capped by the caller's
+    // bound), and the main pass visits per unit only the tiles that can hold a row within U; its candidates are
+    // certified against U like a bounded call's
+    CU(h->prune_ws.ensure(knn_prune_scratch_bytes(m, h->n)));
+    CU(h->prune_bound.ensure(sizeof(double) * (size_t)m));
+    CU(h->thr0.ensure(sizeof(float) * (size_t)m));
+    const unsigned char* pb = h->prune_box.as<unsigned char>();
+    const size_t box = sizeof(double) * (size_t)h->prune_tiles * h->d;
+    CU(knn_prune_prepare(q, m, h->n, h->d, h->k, h->train64.as<double>(), h->prune_geom.as<KnnPruneGeom>(), h->prune_perm.as<int>(),
+                         (const double*)pb, (const double*)(pb + box), (const double*)(pb + 2 * box), h->tc_train.p, h->tc_q.p,
+                         h->qnorm.as<float>(), qflags, bound, h->prune_bound.as<double>(), h->cand_idx.as<int>(),
+                         h->cand_worst.as<float>(), h->prune_ws.p, c->knn_prune == 1, c->sm_count, c->stream, work));
+    tpacked = h->tc_train.p;
+    s.rerank_bound = h->prune_bound.as<double>();
+    s.prune_kept = work.kept;
+    s.prune_visits = visits;
+    CU(knn_bound_thresholds(s.rerank_bound, h->qnorm.as<float>(), m, s.err_rel, s.err_floor, h->thr0.as<float>(), c->stream));
+    s.thr0 = h->thr0.as<float>();
+    s.launches += 12;
+  } else {
+    CU(knn_tc16_pack(q, m, h->d, true, h->tc_q.p, h->qnorm.as<float>(), qflags, c->stream));
+    if (bound) {
+      // bounded call (row-sharded KNN): every query's filter starts at the score threshold of its radius
+      CU(h->thr0.ensure(sizeof(float) * (size_t)m));
+      CU(knn_bound_thresholds(bound, h->qnorm.as<float>(), m, s.err_rel, s.err_floor, h->thr0.as<float>(), c->stream));
+      s.thr0 = h->thr0.as<float>();
+      s.rerank_bound = bound;
+      s.launches += 1;
+    }
+  }
+  CU(knn_tc16_filter(h->tc_q.p, tpacked, m, h->n, h->k, qflags, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
+                     c->sm_count, c->stream, s.thr0, work));
+  s.launches += 2;
+  s.allow_short = bound && s.thr0;
+  s.refine_cap = (int)std::min<int64_t>(m, 65536);
+  return DSP_OK;
+}
+
 int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const double* bound, int64_t* nbr_idx, double* nbr_sqdist,
                                 int32_t* nbr_label) {
   if (!h || m < 0 || (!q && m)) return fail(DSP_ERR_INVALID, "bad argument");
@@ -964,97 +1018,24 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
   dsp_context* c = h->ctx;
   CU(cudaSetDevice(c->device));
   CU(h->redo_list.ensure(sizeof(int32_t) * (size_t)m));
-  const unsigned long long* prune_kept = nullptr;     // (DSP_KNN_DEBUG report)
-  int64_t prune_visits = 0;
-  if (h->dp) {
+  if (h->scan != kScanF64) {
     CU(h->cand_idx.ensure(sizeof(int) * (size_t)m * kKnnCand));
     CU(h->cand_worst.ensure(sizeof(float) * (size_t)m));
     CU(h->qnorm.ensure(sizeof(float) * (size_t)m));
-    double err_rel = (double)(h->d + 4) * 1.1920929e-7, err_floor = 0.0;
-    float qnorm_limit = 0.f;
-    const float* thr0 = nullptr;       // only the tensor-core filter takes start thresholds; the other scans ignore `bound`
-    const double* rerank_bound = nullptr;
-    if (h->tc16) {
-      // tensor-core filter; a query outside its range (|q|^2 above knn_tc16_max_norm(), NaN / inf) is scored as the zero
-      // vector there and handed to the exhaustive float64 scan by the rerank kernel -- per query, on the device
-      CU(h->tc_q.ensure(knn_tc16_packed_bytes(m, true)));
-      int* qflags = h->tc_flags.as<int>() + 4;
-      err_rel = knn_dense_err_rel(16);
-      err_floor = 1.0;
-      qnorm_limit = knn_tc16_max_norm();
-      Tc16Work work;
-      const void* tpacked = h->tc_train_rows.p;
-      // (the tile lists take units x tiles ints, indexed in int)
-      const bool prune = c->knn_prune && knn_tc16_padded_rows(m, true) / kTc16UnitQueries * h->prune_tiles <= INT32_MAX;
-      if (prune) {
-        // tile pruning: queries in curve order, a seed pass bounds every query's k-th distance U (capped by the caller's
-        // bound), and the main pass visits per unit only the tiles that can hold a row within U; its candidates are
-        // certified against U like a bounded call's
-        CU(h->prune_ws.ensure(knn_prune_scratch_bytes(m, h->n)));
-        CU(h->prune_bound.ensure(sizeof(double) * (size_t)m));
-        CU(h->thr0.ensure(sizeof(float) * (size_t)m));
-        const unsigned char* pb = h->prune_box.as<unsigned char>();
-        const size_t box = sizeof(double) * (size_t)h->prune_tiles * h->d;
-        CU(knn_prune_prepare(q, m, h->n, h->d, h->k, h->train64.as<double>(), h->prune_geom.as<KnnPruneGeom>(), h->prune_perm.as<int>(),
-                             (const double*)pb, (const double*)(pb + box), (const double*)(pb + 2 * box), h->tc_train.p, h->tc_q.p,
-                             h->qnorm.as<float>(), qflags, bound, h->prune_bound.as<double>(), h->cand_idx.as<int>(),
-                             h->cand_worst.as<float>(), h->prune_ws.p, c->knn_prune == 1, c->sm_count, c->stream, work));
-        tpacked = h->tc_train.p;
-        rerank_bound = h->prune_bound.as<double>();
-        prune_kept = work.kept;
-        prune_visits = knn_tc16_padded_rows(m, true) / kTc16UnitQueries * h->prune_tiles;
-        CU(knn_bound_thresholds(rerank_bound, h->qnorm.as<float>(), m, err_rel, err_floor, h->thr0.as<float>(), c->stream));
-        thr0 = h->thr0.as<float>();
-        c->launches += 12;
-      } else {
-        CU(knn_tc16_pack(q, m, h->d, true, h->tc_q.p, h->qnorm.as<float>(), qflags, c->stream));
-      }
-      if (bound && !prune) {
-        // bounded call (row-sharded KNN): every query's filter starts at the score threshold of its radius
-        CU(h->thr0.ensure(sizeof(float) * (size_t)m));
-        CU(knn_bound_thresholds(bound, h->qnorm.as<float>(), m, err_rel, err_floor, h->thr0.as<float>(), c->stream));
-        thr0 = h->thr0.as<float>();
-        rerank_bound = bound;
-        c->launches += 1;
-      }
-      CU(knn_tc16_filter(h->tc_q.p, tpacked, m, h->n, h->k, qflags, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
-                         c->sm_count, c->stream, thr0, work));
-      c->launches += 2;
-    } else {
-      CU(knn_scan(h->dp, h->train32.as<float>(), h->n, q, m, h->d, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
-                  h->qnorm.as<float>(), nullptr, c->stream));
-      c->launches += 1;
-    }
-    // rejected queries: fp32 threshold scan + float64 ranking of the survivors (knn_refine) for up to refine_cap of them,
-    // the exhaustive float64 scan for the rest
-    const int refine_cap = (h->dp == 16 && h->k < kKnnCand) ? (int)std::min<int64_t>(m, 65536) : 0;
-    h->refine_cap = refine_cap;
-    if (refine_cap) {
-      CU(h->refine_list.ensure(sizeof(int32_t) * (size_t)refine_cap));
-      CU(h->refine_thr.ensure(sizeof(float) * (size_t)refine_cap));
-      CU(h->surv_count.ensure(sizeof(int32_t) * (size_t)refine_cap));
-      CU(h->surv_rows.ensure(sizeof(int32_t) * (size_t)refine_cap * knn_refine_survivor_cap()));
-    }
-    CU(knn_rerank(h->train64.as<double>(), h->train32.as<float>(), h->dp, h->n, q, m, h->d, h->k, h->index_base,
-                  h->labels.as<int32_t>(), h->cand_idx.as<int>(), h->cand_worst.as<float>(), h->qnorm.as<float>(),
-                  h->tnorm_max, err_rel, err_floor, nbr_idx, nbr_sqdist, nbr_label, h->redo_list.as<int32_t>(),
-                  h->redo_count.as<int32_t>(), c->stream, refine_cap ? h->refine_list.as<int32_t>() : nullptr,
-                  h->refine_thr.as<float>(), refine_cap, qnorm_limit, rerank_bound, thr0, bound && thr0));
-    c->launches += 1;
-    if (refine_cap) {
-      CU(knn_refine(h->train64.as<double>(), h->train32.as<float>(), h->dp, h->n, q, h->d, h->k, h->index_base,
-                    h->labels.as<int32_t>(), h->refine_list.as<int32_t>(), h->refine_thr.as<float>(), refine_cap,
-                    h->surv_count.as<int32_t>(), h->surv_rows.as<int32_t>(), h->redo_count.as<int32_t>(),
-                    h->redo_list.as<int32_t>(), nbr_idx, nbr_sqdist, nbr_label, c->sm_count, c->stream, bound && thr0));
-      c->launches += 2;
-    }
-  } else if (h->dense) {
-    h->refine_cap = 0;
-    // tensor-core candidate scan in chunks of queries (bounded staging), float64 rerank + certificate per chunk;
-    // the rejected queries of every chunk accumulate in one redo list
-    CU(h->cand_idx.ensure(sizeof(int) * (size_t)m * kKnnCand));
-    CU(h->cand_worst.ensure(sizeof(float) * (size_t)m));
-    CU(h->qnorm.ensure(sizeof(float) * (size_t)m));
+  }
+  // candidates: only the tensor-core filter takes the caller's bound (start thresholds); the other scans ignore it
+  KnnStage s;
+  if (h->scan == kScanTc16) {
+    int rc = knn_stage_tc16(h, q, m, bound, s);
+    if (rc) return rc;
+  } else if (h->scan == kScanFp32) {
+    CU(knn_scan(h->dp, h->train32.as<float>(), h->n, q, m, h->d, h->cand_idx.as<int>(), h->cand_worst.as<float>(),
+                h->qnorm.as<float>(), c->stream));
+    s.launches = 1;
+    s.err_rel = (double)(h->d + 4) * 1.1920929e-7;
+    s.refine_cap = (h->dp == 16 && h->k < kKnnCand) ? (int)std::min<int64_t>(m, 65536) : 0;
+  } else if (h->scan == kScanDense) {
+    // tensor-core candidate scan in chunks of queries (bounded staging); one rerank then certifies all of them
     const int64_t chunk = std::min<int64_t>(m, kKnnDenseQueryChunk);
     CU(h->qpacked.ensure(knn_dense_packed_bytes(chunk, h->d, false)));
     CU(h->qnorm_chunk.ensure(sizeof(float) * (size_t)knn_dense_padded_rows(chunk, false)));
@@ -1068,26 +1049,42 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
       CU(cudaMemcpyAsync(h->qnorm.as<float>() + q0, h->qnorm_chunk.p, sizeof(float) * (size_t)mc, cudaMemcpyDeviceToDevice, c->stream));
       CU(knn_dense_scan(h->qpacked.p, h->tpacked.p, h->tnorm_dense.as<float>(), mc, h->n, h->d,
                         h->cand_idx.as<int>() + q0 * kKnnCand, h->cand_worst.as<float>() + q0, c->sm_count, c->stream));
-      c->launches += 2;
+      s.launches += 2;
     }
     int qflags[2] = {0, 0};
     CU(cudaMemcpyAsync(qflags, h->dense_flags.p, sizeof qflags, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    const bool all_fit = qflags[1] == 0;     // a query value outside the fp16 range: float64 scan for everything
-    if (all_fit) {
-      CU(knn_rerank(h->train64.as<double>(), nullptr, 0, h->n, q, m, h->d, h->k, h->index_base,
-                    h->labels.as<int32_t>(), h->cand_idx.as<int>(), h->cand_worst.as<float>(), h->qnorm.as<float>(),
-                    h->tnorm_max, knn_dense_err_rel(h->d), 0.0, nbr_idx, nbr_sqdist, nbr_label, h->redo_list.as<int32_t>(),
-                    h->redo_count.as<int32_t>(), c->stream));
-    } else {
-      CU(knn_redo_all(h->redo_list.as<int32_t>(), h->redo_count.as<int32_t>(), m, c->stream));
-    }
-    c->launches++;
+    s.redo_all = qflags[1] != 0;     // a query value outside the fp16 range: float64 scan for everything
+    s.err_rel = knn_dense_err_rel(h->d);
+    s.allow_short = true;
   } else {
-    h->refine_cap = 0;
-    // feature dimension beyond both scans (or values outside the fp16 range): exhaustive float64 scan of every query
+    s.redo_all = true;     // feature dimension beyond both scans (or values outside the fp16 range)
+  }
+  // rejected queries: fp32 threshold scan + float64 ranking of the survivors (knn_refine) for up to refine_cap of them,
+  // the exhaustive float64 scan for the rest
+  h->refine_cap = s.refine_cap;
+  if (s.refine_cap) {
+    CU(h->refine_list.ensure(sizeof(int32_t) * (size_t)s.refine_cap));
+    CU(h->refine_thr.ensure(sizeof(float) * (size_t)s.refine_cap));
+    CU(h->surv_count.ensure(sizeof(int32_t) * (size_t)s.refine_cap));
+    CU(h->surv_rows.ensure(sizeof(int32_t) * (size_t)s.refine_cap * knn_refine_survivor_cap()));
+  }
+  if (s.redo_all) {
     CU(knn_redo_all(h->redo_list.as<int32_t>(), h->redo_count.as<int32_t>(), m, c->stream));
-    c->launches++;
+  } else {
+    CU(knn_rerank(h->train64.as<double>(), h->train32.as<float>(), h->dp, h->n, q, m, h->d, h->k, h->index_base,
+                  h->labels.as<int32_t>(), h->cand_idx.as<int>(), h->cand_worst.as<float>(), h->qnorm.as<float>(),
+                  h->tnorm_max, s.err_rel, s.err_floor, nbr_idx, nbr_sqdist, nbr_label, h->redo_list.as<int32_t>(),
+                  h->redo_count.as<int32_t>(), c->stream, s.refine_cap ? h->refine_list.as<int32_t>() : nullptr,
+                  h->refine_thr.as<float>(), s.refine_cap, s.qnorm_limit, s.rerank_bound, s.thr0, s.allow_short));
+  }
+  c->launches += s.launches + 1;
+  if (s.refine_cap) {
+    CU(knn_refine(h->train64.as<double>(), h->train32.as<float>(), h->dp, h->n, q, h->d, h->k, h->index_base,
+                  h->labels.as<int32_t>(), h->refine_list.as<int32_t>(), h->refine_thr.as<float>(), s.refine_cap,
+                  h->surv_count.as<int32_t>(), h->surv_rows.as<int32_t>(), h->redo_count.as<int32_t>(),
+                  h->redo_list.as<int32_t>(), nbr_idx, nbr_sqdist, nbr_label, c->sm_count, c->stream, s.allow_short));
+    c->launches += 2;
   }
   CU(h->part_d.ensure(sizeof(double) * (size_t)knn_rescan_grid(c->sm_count) * kKnnMaxK));
   CU(h->part_i.ensure(sizeof(long long) * (size_t)knn_rescan_grid(c->sm_count) * kKnnMaxK));
@@ -1101,12 +1098,12 @@ int dsp_knn_topk_bounded_device(dsp_knn* h, const double* q, int64_t m, const do
     cudaStreamSynchronize(c->stream);
     fprintf(stderr, "[knn] m=%lld n=%lld exhaustive=%d refined=%d refined->exhaustive=%d\n", (long long)m, (long long)h->n, cnt[0],
             std::min(cnt[1], h->refine_cap), cnt[2]);
-    if (prune_kept) {
+    if (s.prune_kept) {
       unsigned long long kept = 0;
-      cudaMemcpyAsync(&kept, prune_kept, sizeof kept, cudaMemcpyDeviceToHost, c->stream);
+      cudaMemcpyAsync(&kept, s.prune_kept, sizeof kept, cudaMemcpyDeviceToHost, c->stream);
       cudaStreamSynchronize(c->stream);
-      fprintf(stderr, "[knn] prune: tile visits kept=%llu of %lld (%s)\n", kept, (long long)prune_visits,
-              c->knn_prune == 1 && kept > (unsigned long long)(0.85 * (double)prune_visits) ? "every tile walked" : "lists walked");
+      fprintf(stderr, "[knn] prune: tile visits kept=%llu of %lld (%s)\n", kept, (long long)s.prune_visits,
+              c->knn_prune == 1 && kept > (unsigned long long)(0.85 * (double)s.prune_visits) ? "every tile walked" : "lists walked");
     }
   }
   return DSP_OK;
@@ -1241,7 +1238,7 @@ int dsp_knn_last_stats(dsp_knn* h, int64_t* rescanned, int32_t* scan_kind) {
     CU(cudaStreamSynchronize(h->ctx->stream));
   }
   if (rescanned) *rescanned = (int64_t)cnt[0] + std::min(cnt[1], h->refine_cap) - cnt[2];
-  if (scan_kind) *scan_kind = h->dp ? (h->tc16 ? 3 : 1) : (h->dense ? 2 : 0);
+  if (scan_kind) *scan_kind = h->scan;
   return DSP_OK;
 }
 

@@ -975,26 +975,25 @@ frontend_pcm_kernel(const PcmArgs a) {
 
 namespace {
 using PcmKernel = void (*)(const PcmArgs);
-struct Variant { PcmKernel fn; int threads; bool stream; const char* name; };
-// [0] is the shared-memory-resident kernel (any alignment); the rest are streaming builds
+struct Variant { PcmKernel fn; int threads; bool stream; };
+// [0], [8] and [9] are shared-memory-resident builds (any alignment); the rest are streaming builds
 const Variant kVariants[] = {
-    {frontend_pcm_kernel<false, 256, 2, 2>, 256, false, "resident 256x2"},
-    {frontend_pcm_kernel<true, 128, 1, 4>, 128, true, "stream 128 thr, >=4 CTAs/SM"},
-    {frontend_pcm_kernel<true, 128, 1, 5>, 128, true, "stream 128 thr, >=5 CTAs/SM"},
-    {frontend_pcm_kernel<true, 128, 1, 6>, 128, true, "stream 128 thr, >=6 CTAs/SM"},
-    {frontend_pcm_kernel<true, 256, 2, 2>, 256, true, "stream 256 thr, >=2 CTAs/SM"},
-    {frontend_pcm_kernel<true, 256, 2, 3>, 256, true, "stream 256 thr, >=3 CTAs/SM"},
-    {frontend_pcm_kernel<true, 192, 2, 4>, 192, true, "stream 192 thr, >=4 CTAs/SM"},
-    {frontend_pcm_kernel<true, 160, 1, 4>, 160, true, "stream 160 thr, >=4 CTAs/SM"},
-    {frontend_pcm_kernel<false, 256, 1, 2>, 256, false, "resident 256 thr (7 main + 1 stats warps)"},
-    {frontend_pcm_kernel<false, 288, 1, 2>, 288, false, "resident 288 thr (8 main + 1 stats warps)"},
+    {frontend_pcm_kernel<false, 256, 2, 2>, 256, false},
+    {frontend_pcm_kernel<true, 128, 1, 4>, 128, true},
+    {frontend_pcm_kernel<true, 128, 1, 5>, 128, true},
+    {frontend_pcm_kernel<true, 128, 1, 6>, 128, true},
+    {frontend_pcm_kernel<true, 256, 2, 2>, 256, true},
+    {frontend_pcm_kernel<true, 256, 2, 3>, 256, true},
+    {frontend_pcm_kernel<true, 192, 2, 4>, 192, true},
+    {frontend_pcm_kernel<true, 160, 1, 4>, 160, true},
+    {frontend_pcm_kernel<false, 256, 1, 2>, 256, false},
+    {frontend_pcm_kernel<false, 288, 1, 2>, 288, false},
 };
 constexpr int kNumVariants = (int)(sizeof(kVariants) / sizeof(kVariants[0]));
 }  // namespace
 
 int pcm_num_variants() { return kNumVariants; }
 bool pcm_variant_streams(int v) { return kVariants[v].stream; }
-const char* pcm_variant_name(int v) { return kVariants[v].name; }
 
 cudaError_t launch_frontend_pcm(int variant, const PcmArgs& a, int grid, size_t smem, cudaStream_t st) {
   const Variant& v = kVariants[variant];

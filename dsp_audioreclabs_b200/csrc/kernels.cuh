@@ -81,7 +81,6 @@ struct PipePlan { int ring_slots, n_rec, cap_groups; size_t smem; };
 bool pipe_kernel_plan(int64_t max_len, int cap_frames, int fl, size_t smem_limit, PipePlan* plan);
 cudaError_t launch_frontend_pipe(const PcmArgs& a, int grid, size_t smem, cudaStream_t st);
 bool pcm_variant_streams(int variant);
-const char* pcm_variant_name(int variant);
 #ifndef DSP_PCM_THREADS
 #define DSP_PCM_THREADS 256
 #endif

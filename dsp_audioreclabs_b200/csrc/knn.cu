@@ -49,9 +49,8 @@ template <int DP, int QPT>
 __global__ void __launch_bounds__(kScanThreads)
 knn_scan_kernel(const float* __restrict__ train32, int64_t n, const double* __restrict__ queries,
                 int64_t m, int d, int* __restrict__ cand_idx, float* __restrict__ cand_worst,
-                float* __restrict__ qnorm_out, const int* __restrict__ gate) {
+                float* __restrict__ qnorm_out) {
   __shared__ __align__(16) float tile[kTileRows * DP];
-  if (gate && gate[1] == 0) return;
   const int64_t q0 = ((int64_t)blockIdx.x * kScanThreads + threadIdx.x) * QPT;
   float q[QPT][DP - 1];
   float cd[QPT][kKnnCand];
@@ -123,9 +122,8 @@ constexpr int kPairQpt = 2;
 __global__ void __launch_bounds__(kScanThreads)
 knn_scan_pair_kernel(const float* __restrict__ train32, int64_t n, const double* __restrict__ queries,
                      int64_t m, int d, int* __restrict__ cand_idx, float* __restrict__ cand_worst,
-                     float* __restrict__ qnorm_out, const int* __restrict__ gate) {
+                     float* __restrict__ qnorm_out) {
   constexpr int DP = 16;
-  if (gate && gate[1] == 0) return;          // the tensor-core filter served this call
   __shared__ __align__(16) float tile[kTileRows * DP];            // [row pair][column][2]
   const int64_t q0 = ((int64_t)blockIdx.x * kScanThreads + threadIdx.x) * kPairQpt;
   f32x2_t qq[kPairQpt][DP - 1];
@@ -795,18 +793,18 @@ cudaError_t knn_pack(const double* train, int64_t n, int d, int dp, float* train
 }
 
 cudaError_t knn_scan(int dp, const float* train32, int64_t n, const double* q, int64_t m, int d,
-                     int* cand_idx, float* cand_worst, float* qnorm, const int* gate, cudaStream_t st) {
+                     int* cand_idx, float* cand_worst, float* qnorm, cudaStream_t st) {
   if (m == 0) return cudaSuccess;
   if (dp == 16) {
     constexpr int QPT = 2;
     const unsigned grid = (unsigned)((m + (int64_t)kScanThreads * QPT - 1) / ((int64_t)kScanThreads * QPT));
-    knn_scan_pair_kernel<<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);
+    knn_scan_pair_kernel<<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm);
   } else if (dp == 32) {
     const unsigned grid = (unsigned)((m + kScanThreads - 1) / kScanThreads);
-    knn_scan_kernel<32, 1><<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);
+    knn_scan_kernel<32, 1><<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm);
   } else {
     const unsigned grid = (unsigned)((m + kScanThreads - 1) / kScanThreads);
-    knn_scan_kernel<64, 1><<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm, gate);
+    knn_scan_kernel<64, 1><<<grid, kScanThreads, 0, st>>>(train32, n, q, m, d, cand_idx, cand_worst, qnorm);
   }
   return cudaGetLastError();
 }

@@ -13,10 +13,8 @@ constexpr int kKnnMaxK = 16;   // largest supported n_neighbors (certificate nee
 int knn_padded_dim(int d);     // 16 / 32 / 64, or 0 when d is too large for the tiled scan
 cudaError_t knn_pack(const double* train, int64_t n, int d, int dp, float* train32, float* tnorm_max,
                      cudaStream_t st);
-// gate (optional, device): the scan runs only when gate[1] != 0 -- the fp32 stand-in for a tensor-core filter call whose
-// queries left the filter's range (knn_tc16.cu), decided on the device without a host round trip
 cudaError_t knn_scan(int dp, const float* train32, int64_t n, const double* q, int64_t m, int d,
-                     int* cand_idx, float* cand_worst, float* qnorm, const int* gate, cudaStream_t st);
+                     int* cand_idx, float* cand_worst, float* qnorm, cudaStream_t st);
 cudaError_t knn_rerank(const double* train, const float* train32, int dp, int64_t n, const double* q,
                        int64_t m, int d, int k, int64_t index_base, const int32_t* labels,
                        const int* cand_idx, const float* cand_worst, const float* qnorm,

@@ -118,8 +118,10 @@ int dsp_destroy(dsp_context* ctx);
 int dsp_set_stream(dsp_context* ctx, void* cuda_stream);
 int dsp_use_own_stream(dsp_context* ctx);
 int dsp_sync(dsp_context* ctx);
-/* Tuning knobs (not needed for correctness): "pcm_variant" = -1 automatic, 0 the shared-memory
- * resident build of the fused kernel, 1.. the streaming builds; "tma_chunk" = bytes per bulk copy. */
+/* Tuning knobs (not needed for correctness): "pcm_variant" = -1 automatic, 0..9 one build of the
+ * fused kernel (0, 8, 9 shared-memory resident; 1-7 streaming, for 16-byte aligned utterances), 10 the
+ * pipelined kernel (build 0 where its plan does not fit); "tma_chunk" = bytes per bulk copy;
+ * "stagger_ns" = start-up delay per co-resident CTA; "knn_prune" = 0 off, 1 automatic, 2 always. */
 int dsp_set_tuning(dsp_context* ctx, const char* key, int value);
 /* kernels launched by this context since creation (bench.py's gpu_launches) */
 int64_t dsp_launch_count(dsp_context* ctx);
