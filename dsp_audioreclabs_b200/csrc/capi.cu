@@ -280,8 +280,8 @@ FrontRoute route_frontend(dsp_context* c, int dtype, const int64_t* feat_offsets
   return r;
 }
 
-// DSP_PROF: per-phase cycle counters of the fast kernels, printed to stderr after every launch (tools/cmp_variants.sh
-// reads these lines).  Returns the zeroed counters, or nullptr when DSP_PROF is unset.
+// DSP_PROF: per-phase cycle counters of the fast kernels, printed to stderr after every launch (tools/quick_pipe.py
+// shows them).  Returns the zeroed counters, or nullptr when DSP_PROF is unset.
 long long* prof_begin(dsp_context* c) {
   if (!std::getenv("DSP_PROF") || c->prof.ensure(16 * sizeof(long long)) != cudaSuccess) return nullptr;
   cudaMemsetAsync(c->prof.p, 0, 16 * sizeof(long long), c->stream);
@@ -294,8 +294,10 @@ void prof_report(dsp_context* c, const FrontRoute& r) {
   cudaStreamSynchronize(c->stream);
   if (r.kind == FrontRoute::kPipe) {
     const char* nm[12] = {"S.wait_full", "S.passA", "S.bar1", "S.passB", "S.bar2", "S.wait_rec", "S.passF", "-", "T.wait", "T.decide", "T.window", "T.stats+out"};
-    fprintf(stderr, "[prof pipe R=%d nrec=%d] utterances=%lld (cycles/utt, stream warp 0 / tail warp 0 x nrec)", r.plan.ring_slots, r.plan.n_rec, h[15]);
-    for (int i = 0; i < 12; ++i) fprintf(stderr, "  %s=%.0f", nm[i], (double)h[i] / (double)std::max<long long>(h[15], 1) * (i >= 8 ? r.plan.n_rec : 1));
+    // n_rec holds two batches of records, one per tail warp at work
+    const int tail_warps = r.plan.n_rec / 2;
+    fprintf(stderr, "[prof pipe R=%d nrec=%d] utterances=%lld (cycles/utt, stream warp 0 / tail warp 0 x %d tail warps)", r.plan.ring_slots, r.plan.n_rec, h[15], tail_warps);
+    for (int i = 0; i < 12; ++i) fprintf(stderr, "  %s=%.0f", nm[i], (double)h[i] / (double)std::max<long long>(h[15], 1) * (i >= 8 ? tail_warps : 1));
     fprintf(stderr, "\n");
   } else {
     const char* nm[12] = {"load_wait", "P1", "feat_empty_wait", "P2", "P2b", "P3tail(searches)", "P4", "fixup+handoff", "P3a(select passes)", "P3b(gather)", "P3c(rank+thresholds)", "P3d(N3N4)"};

@@ -35,35 +35,15 @@ constexpr int kGroup = 64;                 // samples per group-sum record
 constexpr int kChunkSamples = 2048;        // samples per ring slot
 constexpr int kChunkBytes = 2 * kChunkSamples;
 constexpr int kGroupsPerChunk = kChunkSamples / kGroup;   // 32: one group per stream lane
-#ifndef DSP_PIPE_STREAM_WARPS
-#define DSP_PIPE_STREAM_WARPS 8
-#endif
 // 8 stream warps (512 threads, 128 registers each) measure best with the batch hand-off below: 3.12 ms per 100k
 // utterances against 3.26 (12 warps), 3.69 (16) and 3.57 (4) -- every stream warp repeats ~140 instructions of
-// per-utterance set-up, and 22 chunks split 3/3/3/3/3/3/2/2 over 8 warps.  More than 8 use the register split.
-constexpr int kStreamWarps = DSP_PIPE_STREAM_WARPS;       // a multiple of 4: whole warpgroups (setmaxnreg)
-#ifndef DSP_PIPE_TAIL_WARPS
-#define DSP_PIPE_TAIL_WARPS 7
-#endif
-// 7 tail warps: with 11 (-DDSP_PIPE_TAIL_WARPS=11 -DDSP_PIPE_STREAM_REGS=72: 640 threads, stream warps at 72 and tail warps at
-// 112 registers, 22 records, a 24-slot ring) the kernel is parity-green and slower, 3.81 against 3.43 ms per 100k utterances
-constexpr int kMaxTailWarps = DSP_PIPE_TAIL_WARPS;        // tail warps + the control warp: whole warpgroups too
+// per-utterance set-up, and 22 chunks split 3/3/3/3/3/3/2/2 over 8 warps.
+constexpr int kStreamWarps = 8;
+// 7 tail warps: with 11 (640 threads, a register split with stream warps at 72 and tail warps at 112 registers, 22
+// records, a 24-slot ring) the kernel is parity-green and slower, 3.81 against 3.43 ms per 100k utterances
+constexpr int kMaxTailWarps = 7;
 constexpr int kPipeWarps = kStreamWarps + kMaxTailWarps + 1;
 constexpr int kPipeThreads = 32 * kPipeWarps;             // 512
-// Register split (setmaxnreg, per warpgroup; only for kStreamWarps > 8): the stream warps run short integer loops and give their
-// registers to the tail warps, which keep whole sequences in registers.  The launch allocates
-// kLaunchRegs = 65536 / kPipeThreads registers per thread (rounded down to 8) and the CTA owns only those:
-// setmaxnreg.inc can take no more than the stream warps have given back, or it waits forever.
-constexpr bool kSplitRegs = kPipeWarps > 16;              // more than 512 threads: 128 registers each no longer fit
-constexpr int kLaunchRegs = (65536 / kPipeThreads) & ~7;
-#ifndef DSP_PIPE_STREAM_REGS
-#define DSP_PIPE_STREAM_REGS (DSP_PIPE_STREAM_WARPS == 16 ? 56 : 64)
-#endif
-constexpr int kStreamRegs = DSP_PIPE_STREAM_REGS;
-constexpr int kTailRegs = ((kLaunchRegs * kPipeThreads - kStreamWarps * 32 * kStreamRegs) / ((kMaxTailWarps + 1) * 32)) & ~7;
-static_assert(kStreamWarps % 4 == 0 && (kMaxTailWarps + 1) % 4 == 0, "roles must cover whole warpgroups");
-static_assert(!kSplitRegs || kStreamWarps * 32 * kStreamRegs + (kMaxTailWarps + 1) * 32 * kTailRegs <= kLaunchRegs * kPipeThreads, "register pool of the CTA");
-static_assert(!kSplitRegs || kTailRegs >= 104, "tail warps keep whole sequences in registers");
 constexpr int kStreamThreads = 32 * kStreamWarps;
 constexpr int kDescRing = 64;              // > max ring slots: the producer can never lap a reader
 constexpr int kMaxRingSlots = 56;
@@ -79,23 +59,12 @@ constexpr int kMetaE = 8, kMetaO = 13, kMetaP = 17, kMetaL = 18;
 __host__ __device__ constexpr int meta_bit(int i) { return (i & 1) ? kMetaO + (i >> 1) : kMetaE + (i >> 1); }
 
 constexpr int kBarStream = 1;              // named barrier of the stream warps
-// record hand-offs use named barriers too (a warp parked on bar.sync costs no issue slots, a warp polling an
-// mbarrier does): kBarRecFull + r is "record r is complete" (stream warps arrive, its tail warp syncs),
-// kBarRecEmpty + r is "record r is free again" (the tail warp arrives, the stream warps sync)
-constexpr int kBarRecFull = 2, kBarRecEmpty = 9;
-constexpr int kRecBarThreads = 32 * (kStreamWarps + 1);   // the stream warps + the record's tail warp
-// Batch mode: records are handed over kBatch at a time (one per tail warp), double-buffered: the stream warps arrive on
+// Records go to the tail warps through named barriers (a warp parked on bar.sync costs no issue slots, a warp polling an
+// mbarrier does), kBatch at a time (one per tail warp), double-buffered: the stream warps arrive on
 // kBarBatchFull + b after the last record of batch b, ALL tail warps sync on it and therefore run decision / window /
 // statistics at the same time -- one walk through the tail's ~25 KB of code then serves kBatch utterances instead of one
 // (the instruction-miss path, gcc, runs at 94 % of its peak with staggered tail warps).  kBarBatchEmpty + b: the tail
 // warps arrive when they are done with batch b, the stream warps sync before they refill it.
-#ifndef DSP_PIPE_BATCH
-#define DSP_PIPE_BATCH 1
-#endif
-#ifndef DSP_CHAIN_PACKED
-#define DSP_CHAIN_PACKED 1          // window chain on packed fp32x2 arithmetic (0: the scalar FFMA build)
-#endif
-constexpr bool kBatchMode = DSP_PIPE_BATCH != 0;
 constexpr int kBatch = kMaxTailWarps;
 constexpr int kBarBatchFull = 2, kBarBatchEmpty = 4;
 constexpr int kBatchBarThreads = 32 * (kStreamWarps + kMaxTailWarps);
@@ -107,7 +76,7 @@ struct PipeLayout {
 
 __host__ __device__ inline int al16(int x) { return (x + 15) & ~15; }
 
-// R ring slots, capG groups / capF frames per utterance, nrec records (= active tail warps)
+// R ring slots, capG groups / capF frames per utterance, nrec records (two batches of one per active tail warp)
 __host__ __device__ inline PipeLayout make_pipe_layout(int R, int capG, int capF, int fl, int nrec) {
   PipeLayout L;
   int o = 0;
@@ -408,9 +377,8 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
   // =========================================================================================
   // CONTROL WARP: work distribution + TMA producer
   // =========================================================================================
-  // The two register regimes never meet again: everything inside this branch ends in a return.
+  // The roles never meet again: everything inside this branch ends in a return.
   if (wid >= kStreamWarps) {
-  if constexpr (kSplitRegs) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kTailRegs));
   if (wid == kPipeWarps - 1) {
     // Lane 0 schedules and issues the bulk copies.  Bulk copies need 16-byte aligned addresses on both sides (and the
     // tiled tensor-map form faults on an inner coordinate that is not a multiple of 16 bytes, tools/tma_probe.cu), so an
@@ -486,7 +454,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
   // tail warps get the issue slots they can use, the throughput-bound stream warps fill the rest)
   const int twid = wid - kStreamWarps;
   if (twid >= 0 && twid < kMaxTailWarps) {
-    if (!kBatchMode && twid >= nrec) return;
     double* cand = reinterpret_cast<double*>(smem + L.scratch + (size_t)twid * 256);
 
     // Window coefficients of the hop-128 / length-256 chain.  The chain reads 16-byte ALIGNED vectors whatever the
@@ -499,11 +466,11 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
     long long tp[5] = {0, 0, 0, 0, 0}, tprev = clock64();
     auto tick = [&](int i) { if (a.prof) { const long long t = clock64(); tp[i] += t - tprev; tprev = t; } };
     for (int it = 0;; ++it) {
-      const int batch = kBatchMode ? (it & 1) : 0;
+      const int batch = it & 1;
       // nb = records per batch = tail warps at work (7 unless the per-utterance records of a many-frame geometry leave
       // room for fewer: pipe_kernel_plan); the other tail warps only keep the batch barriers' head counts
-      const int nb = kBatchMode ? (nrec >> 1) : nrec;
-      unsigned char* rec = smem + L.rec + (size_t)(kBatchMode ? batch * nb + min(twid, nb - 1) : twid) * L.rec_bytes;
+      const int nb = nrec >> 1;
+      unsigned char* rec = smem + L.rec + (size_t)(batch * nb + min(twid, nb - 1)) * L.rec_bytes;
       int* r_int = reinterpret_cast<int*>(rec);
       double* r_dbl = reinterpret_cast<double*>(rec + 64);
       double* r_e = reinterpret_cast<double*>(rec + L.rec_e);
@@ -511,16 +478,11 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
       unsigned short* r_zf = reinterpret_cast<unsigned short*>(rec + L.rec_zf);
       float* s_fe = reinterpret_cast<float*>(rec + L.rec_fe);   // indexed by full-utterance frame number
       float* s_fm = reinterpret_cast<float*>(rec + L.rec_fm);
-      if constexpr (kBatchMode) bar_sync(kBarBatchFull + batch, kBatchBarThreads);
-      else bar_sync(kBarRecFull + twid, kRecBarThreads);
+      bar_sync(kBarBatchFull + batch, kBatchBarThreads);
       int u = r_int[0];
-      if constexpr (kBatchMode) {
-        if (u == -2) break;                                   // the closing batch: every tail warp leaves
-        if (twid >= nb) u = -1;                               // a tail warp without a record slot
-        if (u < 0) { __syncwarp(); bar_arrive(kBarBatchEmpty + batch, kBatchBarThreads); continue; }   // padding of the last batch
-      } else {
-        if (u < 0) break;
-      }
+      if (u == -2) break;                                     // the closing batch: every tail warp leaves
+      if (twid >= nb) u = -1;                                 // a tail warp without a record slot
+      if (u < 0) { __syncwarp(); bar_arrive(kBarBatchEmpty + batch, kBatchBarThreads); continue; }   // padding of the last batch
       tick(0);
       const int n = r_int[1], f1 = r_int[2], thr = r_int[4], kmn_s = r_int[5], kmx_s = r_int[6];
       const double phi_d = r_dbl[0], inv_m = r_dbl[1], mu = r_dbl[2];
@@ -742,7 +704,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
           const float scale = hi8 ? (float)sc_m : (float)sc_e;
           float* dst = (hi8 ? s_fm : s_fe) + zbase + fa - 1;   // frame fa + i - 1 at dst[i]
           float* dummy = reinterpret_cast<float*>(cand);
-#if DSP_CHAIN_PACKED
           // Packed fp32x2 arithmetic (sm_100 FFMA2 / FADD2 / FMUL2): the two samples of a 32-bit word travel as one
           // 64-bit register pair from the conversion on -- (x + c1f) - phi, d * d and the four multiply-adds of a word are
           // ONE instruction each instead of two.  Same FMA-pipe time, two thirds of the issue slots (12 instead of 17
@@ -781,44 +742,12 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
             // +50 % in this phase): lanes with nothing to write hit the warp's scratch word
             *((writer && i >= 1 && i <= nfr) ? dst + i : dummy) = vv * scale;
           };
-#else
-          float ce = 0.f, cm = 0.f;                          // first-half partials of the previous block
-          auto step = [&](const int4& q, int i) {
-            const uint32_t w[4] = {(uint32_t)q.x, (uint32_t)q.y, (uint32_t)q.z, (uint32_t)q.w};
-            float e0 = 0.f, m0 = 0.f, e1 = ce, m1 = cm;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const uint32_t ub = w[k] ^ 0x80008000u;
-              const float dlo = (__uint_as_float(__byte_perm(ub, 0x4b000000u, 0x7610)) + c1f) - phi;
-              const float dhi = (__uint_as_float(__byte_perm(ub, 0x4b000000u, 0x7632)) + c1f) - phi;
-              const float qlo = dlo * dlo, qhi = dhi * dhi;
-              const float alo = fabsf(dlo), ahi = fabsf(dhi);
-              e0 = fmaf(cw2[0][2 * k], qlo, e0); m0 = fmaf(cw[0][2 * k], alo, m0);
-              e1 = fmaf(cw2[1][2 * k], qlo, e1); m1 = fmaf(cw[1][2 * k], alo, m1);
-              e0 = fmaf(cw2[0][2 * k + 1], qhi, e0); m0 = fmaf(cw[0][2 * k + 1], ahi, m0);
-              e1 = fmaf(cw2[1][2 * k + 1], qhi, e1); m1 = fmaf(cw[1][2 * k + 1], ahi, m1);
-            }
-            ce = e0; cm = m0;
-            // transposed reduction of (e1, m1) over the chain's 16 lanes
-            const float send = hi8 ? e1 : m1, keep = hi8 ? m1 : e1;
-            float vv = keep + __shfl_xor_sync(0xffffffffu, send, 8);
-            vv += __shfl_xor_sync(0xffffffffu, vv, 4);
-            vv += __shfl_xor_sync(0xffffffffu, vv, 2);
-            vv += __shfl_xor_sync(0xffffffffu, vv, 1);
-            // one unconditional store (a branch here makes the compiler give up the straight-line schedule of the loop:
-            // +50 % in this phase): lanes with nothing to write hit the warp's scratch word
-            *((writer && i >= 1 && i <= nfr) ? dst + i : dummy) = vv * scale;
-          };
-#endif
           // kInFlight hop blocks in flight per lane (the tail warps run this phase together and wait on L2 / HBM together:
           // 4 -> 6 in flight is 3.65 -> 3.24 ms per 100k utterances; before the batch hand-off the larger loop body cost
           // more in instruction misses than it hid in latency); loads past the chain's last block re-read that block.
           // ld.global.cs: by the time a batch is processed the segment has usually left L2 (hit rate ~10 %) and this is
           // its last use -- streaming loads keep the dead lines from displacing the ring's traffic (-4 % DRAM reads)
-#ifndef DSP_CHAIN_INFLIGHT
-#define DSP_CHAIN_INFLIGHT 6
-#endif
-          constexpr int kInFlight = DSP_CHAIN_INFLIGHT;
+          constexpr int kInFlight = 6;
           int4 q[kInFlight];
           auto load_block = [&](int bi) -> int4 { return __ldcs(ptr + 16 * bi); };
 #pragma unroll
@@ -1005,8 +934,7 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
         if (flagged) { const int s = atomicAdd(a.flag_count, 1); a.flag_list[s] = u; }
       }
       __syncwarp();
-      if constexpr (kBatchMode) bar_arrive(kBarBatchEmpty + batch, kBatchBarThreads);
-      else bar_arrive(kBarRecEmpty + twid, kRecBarThreads);
+      bar_arrive(kBarBatchEmpty + batch, kBatchBarThreads);
       tick(3);
     }
     if (a.prof && twid == 0 && lane == 0) for (int i = 0; i < 4; ++i) atomicAdd((unsigned long long*)&a.prof[8 + i], (unsigned long long)tp[i]);
@@ -1014,13 +942,12 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
   }
   return;
   }   // wid >= kStreamWarps
-  if constexpr (kSplitRegs) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kStreamRegs));
 
   // =========================================================================================
   // STREAM WARPS
   // =========================================================================================
   const int swid = wid, stid = tid;
-  const int nbs = kBatchMode ? (nrec >> 1) : nrec;       // records per batch (pipe_kernel_plan)
+  const int nbs = nrec >> 1;                              // records per batch (pipe_kernel_plan)
   int useq = 0, cslot = 0, clap = 0, rec_id = 0, rec_lap = 0;
   long long sp[8] = {0, 0, 0, 0, 0, 0, 0, 0}, sprev = clock64();
   auto stick = [&](int i) { if (a.prof) { const long long t = clock64(); sp[i] += t - sprev; sprev = t; } };
@@ -1033,14 +960,12 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
     const int par = useq & 1;
     unsigned char* rec = smem + L.rec + (size_t)rec_id * L.rec_bytes;
     int* r_int = reinterpret_cast<int*>(rec);
-    // record slot hand-off with the tail warps: per record, or (batch mode) per batch of kBatch records
+    // record slot hand-off with the tail warps, per batch of kBatch records
     auto rec_acquire = [&]() {
-      if constexpr (kBatchMode) { if (rec_lap > 0 && rec_id % nbs == 0) bar_sync(kBarBatchEmpty + rec_id / nbs, kBatchBarThreads); }
-      else { if (rec_lap > 0) bar_sync(kBarRecEmpty + rec_id, kRecBarThreads); }
+      if (rec_lap > 0 && rec_id % nbs == 0) bar_sync(kBarBatchEmpty + rec_id / nbs, kBatchBarThreads);
     };
     auto rec_publish = [&]() {
-      if constexpr (kBatchMode) { if (rec_id % nbs == nbs - 1) bar_arrive(kBarBatchFull + rec_id / nbs, kBatchBarThreads); }
-      else bar_arrive(kBarRecFull + rec_id, kRecBarThreads);
+      if (rec_id % nbs == nbs - 1) bar_arrive(kBarBatchFull + rec_id / nbs, kBatchBarThreads);
       if (++rec_id == nrec) { rec_id = 0; ++rec_lap; }
     };
     // The ring holds the 16-byte aligned stream around the utterance: sample i sits at stream position i + sh
@@ -1484,8 +1409,10 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
     stick(6);
   }
   if (a.prof && stid == 0) { for (int i = 0; i < 7; ++i) atomicAdd((unsigned long long*)&a.prof[i], (unsigned long long)sp[i]); atomicAdd((unsigned long long*)&a.prof[15], (unsigned long long)useq); }
-  if constexpr (kBatchMode) {
-    // pad the open batch with "skip" records, then one closing batch that makes every tail warp leave
+  // Pad the open batch with "skip" records, then one closing batch that makes every tail warp leave.  (A block of its
+  // own: with `mark` at function scope the compiler numbers the registers of the stream warps' record hand-off
+  // differently.)
+  {
     auto mark = [&](int code) {
       if (rec_lap > 0 && rec_id % nbs == 0) bar_sync(kBarBatchEmpty + rec_id / nbs, kBatchBarThreads);
       if (stid == 0) *reinterpret_cast<int*>(smem + L.rec + (size_t)rec_id * L.rec_bytes) = code;
@@ -1497,16 +1424,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) frontend_pipe_kernel(const Pc
     while (rec_id % nbs != 0) mark(-1);
 #pragma unroll 1
     for (int k = 0; k < nbs; ++k) mark(-2);
-    return;
-  }
-  // tell the tail warps to stop: one terminator record each
-#pragma unroll 1
-  for (int k = 0; k < nrec; ++k) {
-    if (rec_lap > 0) bar_sync(kBarRecEmpty + rec_id, kRecBarThreads);
-    if (stid == 0) *reinterpret_cast<int*>(smem + L.rec + (size_t)rec_id * L.rec_bytes) = -1;
-    __syncwarp();
-    bar_arrive(kBarRecFull + rec_id, kRecBarThreads);
-    if (++rec_id == nrec) { rec_id = 0; ++rec_lap; }
   }
 }
 
@@ -1518,35 +1435,19 @@ bool pipe_kernel_plan(int64_t max_len, int cap_frames, int fl, size_t smem_limit
   if (max_len > 65535 || cap_frames > 65535 || fl > 65535) return false;      // 16-bit crossing counts, int32 sums
   const int chunks = (int)std::max<int64_t>((max_len + 7 + kChunkSamples - 1) / kChunkSamples, 1);   // + the <= 7 samples below a misaligned start
   const int capG = chunks * kGroupsPerChunk;
-  if (kBatchMode) {
-    // two batches of records, as many per batch (= tail warps at work) as leave the ring the utterance in flight plus
-    // at least two chunks of the next one: 7 for the usual geometries, fewer when hops under ~100 samples make the
-    // per-utterance records large (64/32 at 1 s: 1,377 frames, 16.6 KB per record -> 2 per batch)
-    for (int nb = kBatch; nb >= 1; --nb) {
-      const int nrec = 2 * nb;
-      const PipeLayout fixed = make_pipe_layout(0, capG, cap_frames, fl, nrec);
-      const long long room = (long long)smem_limit - fixed.total - 1024;
-      int R = (int)(room / (kChunkBytes + 16));
-      if (R > kMaxRingSlots) R = kMaxRingSlots;
-      if (R < chunks + 2) continue;
-      plan->ring_slots = R; plan->n_rec = nrec; plan->cap_groups = capG;
-      plan->smem = (size_t)make_pipe_layout(R, capG, cap_frames, fl, nrec).total;
-      return true;
-    }
-    return false;
-  }
-  for (int nrec = kMaxTailWarps; nrec >= 2; --nrec) {
+  // two batches of records, as many per batch (= tail warps at work) as leave the ring the utterance in flight plus
+  // at least two chunks of the next one: 7 for the usual geometries, fewer when hops under ~100 samples make the
+  // per-utterance records large (64/32 at 1 s: 1,377 frames, 16.6 KB per record -> 2 per batch)
+  for (int nb = kBatch; nb >= 1; --nb) {
+    const int nrec = 2 * nb;
     const PipeLayout fixed = make_pipe_layout(0, capG, cap_frames, fl, nrec);
     const long long room = (long long)smem_limit - fixed.total - 1024;        // static shared memory + slack
     int R = (int)(room / (kChunkBytes + 16));
     if (R > kMaxRingSlots) R = kMaxRingSlots;
-    // two utterances in flight if possible; give up tail warps for ring slots otherwise
-    const bool roomy = R >= 2 * chunks - 2 || R == kMaxRingSlots;
-    if (R >= chunks + 1 && (roomy || nrec == 2)) {
-      plan->ring_slots = R; plan->n_rec = nrec; plan->cap_groups = capG;
-      plan->smem = (size_t)make_pipe_layout(R, capG, cap_frames, fl, nrec).total;
-      return true;
-    }
+    if (R < chunks + 2) continue;
+    plan->ring_slots = R; plan->n_rec = nrec; plan->cap_groups = capG;
+    plan->smem = (size_t)make_pipe_layout(R, capG, cap_frames, fl, nrec).total;
+    return true;
   }
   return false;
 }
