@@ -98,6 +98,11 @@ SIGNATURES = {
     "dsp_knn_merge_vote_device": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _I32, _P, _P, _P]),
     "dsp_mfcc_batch_host": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, C.POINTER(MfccParams), _P, _P, _P, _P, _P]),
     "dsp_dtw_topk_host": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P, _I64, _I32, _I32, _I64, _P, _P, _P, _P]),
+    "dsp_mfcc_batch_device": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, C.POINTER(MfccParams), _P, _P, _P, _P, _P]),
+    "dsp_dtw_fit_device": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I32, _I32, _I64, C.POINTER(_P)]),
+    "dsp_dtw_topk_device": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _P]),
+    "dsp_dtw_last_stats": (C.c_int, [_P, C.POINTER(_I64), C.POINTER(_I64)]),
+    "dsp_dtw_free": (C.c_int, [_P]),
     "dsp_wav_scan": (C.c_int, [_P, _I64, _I32, _P]),
     "dsp_wav_read": (C.c_int, [_P, _I64, _I32, _P, _P, _P, _I64]),
     "dsp_host_alloc": (C.c_int, [_I64, C.POINTER(_P)]),

@@ -126,6 +126,24 @@ struct dsp_context {
   int occ = 0;
   Slot slot[2];
   DevBuf tmp[16];
+  // device tables of dsp_mfcc_batch_device, kept per (parameters, filterbank, DCT): a repeated call copies nothing
+  struct MfccEntry {
+    int frame_length, window, n_fft, n_mels, n_ceps;
+    std::vector<float> fb, dct;                 // the caller's tables (the key) ...
+    std::vector<float> win, tw;                 // ... and the derived host tables, alive until their copies are done
+    std::vector<int> range;
+    DevBuf d_win, d_tw, d_fb, d_range, d_dct;
+  };
+  std::vector<MfccEntry*> mfcc_tables;
+  DevBuf mfcc_work;  // work counter of the device MFCC call
+};
+
+struct dsp_dtw {
+  dsp_context* ctx = nullptr;
+  int64_t nt = 0, index_base = 0;
+  int dim = 0, k = 0, max_t = 0, warps = 1;
+  std::vector<int32_t> h_len;                   // source of the t_len upload
+  DevBuf feats, offsets, t_len, labels, cand_d, cand_i, stats;
 };
 
 struct dsp_knn {
@@ -365,6 +383,79 @@ int frontend_device(dsp_context* c, const void* samples, int dtype, const int64_
                       a.flag_list ? 0 : B, max_len, p, out, ex, r.replay_grid);
 }
 
+int check_mfcc_params(const dsp_mfcc_params* p) {
+  if (p->frame_length < 1 || p->frame_shift < 1 || p->n_mels < 1 || p->n_ceps < 1 || p->n_ceps > p->n_mels)
+    return fail(DSP_ERR_INVALID, "bad MFCC geometry");
+  if (p->n_fft < 32 || (p->n_fft & (p->n_fft - 1)) || p->n_fft < p->frame_length || p->n_fft > 16384)
+    return fail(DSP_ERR_INVALID, "n_fft must be a power of two in [max(32, frame_length), 16384]");
+  if (mfcc_smem_bytes(p->n_fft, p->n_mels) > kMaxSmemPerCta) return fail(DSP_ERR_UNSUPPORTED, "n_fft too large for shared memory");
+  return DSP_OK;
+}
+
+// the tables mfcc_kernel reads besides the caller's filterbank / DCT: float32 window, twiddles, filter bin ranges
+int mfcc_host_tables(const dsp_mfcc_params* p, const float* filterbank, std::vector<float>& wf, std::vector<float>& tw,
+                     std::vector<int>& range) {
+  std::vector<double> w;
+  int rc = host_window(p->window, p->frame_length, w);
+  if (rc) return rc;
+  wf.assign(w.begin(), w.end());
+  const int n_bins = p->n_fft / 2 + 1;
+  tw.assign((size_t)p->n_fft, 0.f);                                               // W[k] = exp(-2 pi i k / n_fft), k < n_fft / 2
+  for (int k = 0; k < p->n_fft / 2; ++k) {
+    const double a = -2.0 * M_PI * (double)k / (double)p->n_fft;
+    tw[2 * (size_t)k] = (float)std::cos(a); tw[2 * (size_t)k + 1] = (float)std::sin(a);
+  }
+  range.assign(2 * (size_t)p->n_mels, 0);                                         // non-zero bins of every filter
+  for (int m = 0; m < p->n_mels; ++m) {
+    int lo = n_bins, hi = 0;
+    for (int b = 0; b < n_bins; ++b) if (filterbank[(size_t)m * n_bins + b] != 0.f) { lo = std::min(lo, b); hi = std::max(hi, b + 1); }
+    range[2 * (size_t)m] = std::min(lo, hi); range[2 * (size_t)m + 1] = hi;
+  }
+  return DSP_OK;
+}
+
+// The context's device tables for these parameters and host tables, uploaded on first use (stream-ordered copies from
+// host vectors the entry keeps).  A hit compares the tables on the host and copies nothing.
+int ensure_mfcc_tables(dsp_context* c, const dsp_mfcc_params* p, const float* filterbank, const float* dct,
+                       dsp_context::MfccEntry** out) {
+  const size_t n_fb = (size_t)p->n_mels * (p->n_fft / 2 + 1), n_dct = (size_t)p->n_ceps * p->n_mels;
+  for (auto* e : c->mfcc_tables)
+    if (e->frame_length == p->frame_length && e->window == p->window && e->n_fft == p->n_fft && e->n_mels == p->n_mels &&
+        e->n_ceps == p->n_ceps && !std::memcmp(e->fb.data(), filterbank, n_fb * sizeof(float)) &&
+        !std::memcmp(e->dct.data(), dct, n_dct * sizeof(float))) { *out = e; return DSP_OK; }
+  if (c->mfcc_tables.size() >= 16) {           // a sweep over many geometries: drop the tables once nothing can be reading them
+    CU(cudaDeviceSynchronize());
+    for (auto* e : c->mfcc_tables) { e->d_win.release(); e->d_tw.release(); e->d_fb.release(); e->d_range.release(); e->d_dct.release(); delete e; }
+    c->mfcc_tables.clear();
+  }
+  auto* e = new dsp_context::MfccEntry{p->frame_length, p->window, p->n_fft, p->n_mels, p->n_ceps,
+                                       std::vector<float>(filterbank, filterbank + n_fb), std::vector<float>(dct, dct + n_dct),
+                                       {}, {}, {}, {}, {}, {}, {}, {}};
+  int rc = mfcc_host_tables(p, filterbank, e->win, e->tw, e->range);
+  if (rc) { delete e; return rc; }
+  auto drop = [&](int code) { e->d_win.release(); e->d_tw.release(); e->d_fb.release(); e->d_range.release(); e->d_dct.release(); delete e; return code; };
+  if (e->d_win.ensure(sizeof(float) * e->win.size()) != cudaSuccess || e->d_tw.ensure(sizeof(float) * e->tw.size()) != cudaSuccess ||
+      e->d_fb.ensure(sizeof(float) * n_fb) != cudaSuccess || e->d_range.ensure(sizeof(int) * e->range.size()) != cudaSuccess ||
+      e->d_dct.ensure(sizeof(float) * n_dct) != cudaSuccess)
+    return drop(fail(DSP_ERR_NOMEM, "device allocation failed"));
+  const std::pair<DevBuf*, std::pair<const void*, size_t>> copies[] = {
+      {&e->d_win, {e->win.data(), sizeof(float) * e->win.size()}}, {&e->d_tw, {e->tw.data(), sizeof(float) * e->tw.size()}},
+      {&e->d_fb, {e->fb.data(), sizeof(float) * n_fb}}, {&e->d_range, {e->range.data(), sizeof(int) * e->range.size()}},
+      {&e->d_dct, {e->dct.data(), sizeof(float) * n_dct}}};
+  for (const auto& cp : copies) {
+    const cudaError_t err = cudaMemcpyAsync(cp.first->p, cp.second.first, cp.second.second, cudaMemcpyHostToDevice, c->stream);
+    if (err != cudaSuccess) return drop(fail(DSP_ERR_CUDA, "MFCC table upload: %s", cudaGetErrorString(err)));
+  }
+  c->mfcc_tables.push_back(e);
+  *out = e;
+  return DSP_OK;
+}
+
+void dtw_release(dsp_dtw* h) {
+  DevBuf* all[] = {&h->feats, &h->offsets, &h->t_len, &h->labels, &h->cand_d, &h->cand_i, &h->stats};
+  for (DevBuf* b : all) b->release();
+}
+
 // small helper for the single-signal host entry points
 struct OneShot {
   dsp_context* c;
@@ -432,6 +523,9 @@ int dsp_destroy(dsp_context* c) {
   for (auto& b : c->tmp) b.release();
   for (auto* e : c->windows) { e->w64.release(); e->w32.release(); delete e; }
   c->windows.clear();
+  for (auto* e : c->mfcc_tables) { e->d_win.release(); e->d_tw.release(); e->d_fb.release(); e->d_range.release(); e->d_dct.release(); delete e; }
+  c->mfcc_tables.clear();
+  c->mfcc_work.release();
   c->counters.release(); c->flag_list.release(); c->prof.release();
   c->zbuf.release(); c->seqbuf.release();
   if (c->own) cudaStreamDestroy(c->own);
@@ -1118,29 +1212,15 @@ int dsp_mfcc_batch_host(dsp_context* c, const int16_t* samples, const int64_t* o
                         int32_t* n_frames_out) {
   if (!c || !p || n_utts < 0 || (n_utts && (!samples || !offsets || !seg_start || !seg_end || !filterbank || !dct || !mfcc_offsets || !mfcc_out)))
     return fail(DSP_ERR_INVALID, "bad argument");
-  if (p->frame_length < 1 || p->frame_shift < 1 || p->n_mels < 1 || p->n_ceps < 1 || p->n_ceps > p->n_mels)
-    return fail(DSP_ERR_INVALID, "bad MFCC geometry");
-  if (p->n_fft < 32 || (p->n_fft & (p->n_fft - 1)) || p->n_fft < p->frame_length || p->n_fft > 16384)
-    return fail(DSP_ERR_INVALID, "n_fft must be a power of two in [max(32, frame_length), 16384]");
-  if (mfcc_smem_bytes(p->n_fft, p->n_mels) > kMaxSmemPerCta) return fail(DSP_ERR_UNSUPPORTED, "n_fft too large for shared memory");
+  int rc = check_mfcc_params(p);
+  if (rc) return rc;
   if (n_utts == 0) return DSP_OK;
   CU(cudaSetDevice(c->device));
-  std::vector<double> w;
-  int rc = host_window(p->window, p->frame_length, w);
+  std::vector<float> wf, tw;
+  std::vector<int> range;
+  rc = mfcc_host_tables(p, filterbank, wf, tw, range);
   if (rc) return rc;
-  std::vector<float> wf(w.begin(), w.end());
   const int n_bins = p->n_fft / 2 + 1;
-  std::vector<float> tw((size_t)p->n_fft);                                       // W[k] = exp(-2 pi i k / n_fft), k < n_fft / 2
-  for (int k = 0; k < p->n_fft / 2; ++k) {
-    const double a = -2.0 * M_PI * (double)k / (double)p->n_fft;
-    tw[2 * (size_t)k] = (float)std::cos(a); tw[2 * (size_t)k + 1] = (float)std::sin(a);
-  }
-  std::vector<int> range(2 * (size_t)p->n_mels);                                  // non-zero bins of every filter
-  for (int m = 0; m < p->n_mels; ++m) {
-    int lo = n_bins, hi = 0;
-    for (int b = 0; b < n_bins; ++b) if (filterbank[(size_t)m * n_bins + b] != 0.f) { lo = std::min(lo, b); hi = std::max(hi, b + 1); }
-    range[2 * (size_t)m] = std::min(lo, hi); range[2 * (size_t)m + 1] = hi;
-  }
   const int64_t total_samples = lengths ? offsets[n_utts - 1] + lengths[n_utts - 1] : offsets[n_utts];
   int64_t span = 0;
   for (int64_t b = 0; b < n_utts; ++b) span = std::max<int64_t>(span, offsets[b] + (lengths ? lengths[b] : offsets[b + 1] - offsets[b]));
@@ -1225,6 +1305,115 @@ int dsp_dtw_topk_host(dsp_context* c, const float* q_feats, const int64_t* q_off
   if (nbr_idx) CU(cudaMemcpyAsync(nbr_idx, d_ni, sizeof(int64_t) * (size_t)nq * k, cudaMemcpyDeviceToHost, st));
   if (nbr_label) CU(cudaMemcpyAsync(nbr_label, d_nl, sizeof(int32_t) * (size_t)nq * k, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
+  return DSP_OK;
+}
+
+int dsp_mfcc_batch_device(dsp_context* c, const int16_t* samples, const int64_t* offsets, const int32_t* lengths,
+                          const int32_t* seg_start, const int32_t* seg_end, int64_t n_utts, const dsp_mfcc_params* p,
+                          const float* filterbank, const float* dct, const int64_t* mfcc_offsets, float* mfcc_out,
+                          int32_t* n_frames_out) {
+  if (!c || !p || n_utts < 0 || (n_utts && (!samples || !offsets || !seg_start || !seg_end || !filterbank || !dct || !mfcc_offsets || !mfcc_out)))
+    return fail(DSP_ERR_INVALID, "bad argument");
+  int rc = check_mfcc_params(p);
+  if (rc) return rc;
+  if (n_utts == 0) return DSP_OK;
+  CU(cudaSetDevice(c->device));
+  dsp_context::MfccEntry* t = nullptr;
+  rc = ensure_mfcc_tables(c, p, filterbank, dct, &t);
+  if (rc) return rc;
+  CU(c->mfcc_work.ensure(sizeof(unsigned int)));
+  MfccArgs a{p->frame_length, p->frame_shift, p->n_fft, p->n_mels, p->n_ceps, p->pre_emphasis, (float)p->log_floor};
+  CU(launch_mfcc(samples, offsets, lengths, seg_start, seg_end, n_utts, a, t->d_win.as<float>(), t->d_tw.as<float2>(),
+                 t->d_fb.as<float>(), t->d_range.as<int2>(), t->d_dct.as<float>(), mfcc_offsets, mfcc_out, n_frames_out,
+                 c->mfcc_work.as<unsigned int>(), c->sm_count, c->stream));
+  c->launches++;
+  return DSP_OK;
+}
+
+int dsp_dtw_fit_device(dsp_context* c, const float* t_feats, const int64_t* t_offsets, const int32_t* t_lengths,
+                       const int32_t* t_labels, int64_t nt, int32_t dim, int32_t k, int64_t index_base, dsp_dtw** out) {
+  if (!c || !out || nt < 1 || dim < 1 || k < 1 || !t_offsets) return fail(DSP_ERR_INVALID, "bad argument");
+  *out = nullptr;
+  if (k > kKnnMaxK) return fail(DSP_ERR_UNSUPPORTED, "k > %d is not supported", kKnnMaxK);
+  if (dim > dtw_max_dim()) return fail(DSP_ERR_UNSUPPORTED, "feature dimension > %d is not supported by the DTW kernel", dtw_max_dim());
+  if (nt > INT32_MAX) return fail(DSP_ERR_UNSUPPORTED, "more than 2^31 templates per handle");
+  CU(cudaSetDevice(c->device));
+  // the one synchronisation: template lengths on the host, for the longest template and the extent of the copy
+  std::vector<int64_t> off((size_t)nt + 1);
+  std::vector<int32_t> len((size_t)nt);
+  CU(cudaMemcpyAsync(off.data(), t_offsets, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, c->stream));
+  if (t_lengths) CU(cudaMemcpyAsync(len.data(), t_lengths, sizeof(int32_t) * len.size(), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  int64_t extent = 0, max_t = 0;
+  for (int64_t i = 0; i < nt; ++i) {
+    const int64_t n = t_lengths ? (int64_t)len[(size_t)i] : off[(size_t)i + 1] - off[(size_t)i];
+    if (off[(size_t)i] < 0 || n < 0 || n > INT32_MAX) return fail(DSP_ERR_INVALID, "template %lld: bad offset / length", (long long)i);
+    len[(size_t)i] = (int32_t)n;
+    max_t = std::max(max_t, n);
+    extent = std::max(extent, off[(size_t)i] + n);
+  }
+  if (extent > 0 && !t_feats) return fail(DSP_ERR_INVALID, "bad argument");
+  const size_t per_warp = dtw_fused_smem_per_warp((int)max_t, dim);
+  if (per_warp > c->smem_optin)
+    return fail(DSP_ERR_UNSUPPORTED, "template sequence too long for shared memory (%lld frames x %d features)", (long long)max_t, dim);
+  dsp_dtw* h = new dsp_dtw();
+  h->ctx = c; h->nt = nt; h->index_base = index_base; h->dim = dim; h->k = k; h->max_t = (int)max_t;
+  h->warps = (int)std::min<size_t>(dtw_fused_max_warps(), c->smem_optin / per_warp);
+  h->h_len = std::move(len);
+  auto bail = [&](int code) { dtw_release(h); delete h; return code; };
+  if (h->feats.ensure(sizeof(float) * (size_t)std::max<int64_t>(extent, 1) * dim) != cudaSuccess ||
+      h->offsets.ensure(sizeof(int64_t) * (size_t)nt) != cudaSuccess || h->t_len.ensure(sizeof(int32_t) * (size_t)nt) != cudaSuccess ||
+      h->labels.ensure(sizeof(int32_t) * (size_t)nt) != cudaSuccess || h->stats.ensure(2 * sizeof(unsigned long long)) != cudaSuccess)
+    return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
+  cudaError_t e = cudaSuccess;
+  if (extent > 0) e = cudaMemcpyAsync(h->feats.p, t_feats, sizeof(float) * (size_t)extent * dim, cudaMemcpyDeviceToDevice, c->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(h->offsets.p, t_offsets, sizeof(int64_t) * (size_t)nt, cudaMemcpyDeviceToDevice, c->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(h->t_len.p, h->h_len.data(), sizeof(int32_t) * (size_t)nt, cudaMemcpyHostToDevice, c->stream);
+  if (e == cudaSuccess)
+    e = t_labels ? cudaMemcpyAsync(h->labels.p, t_labels, sizeof(int32_t) * (size_t)nt, cudaMemcpyDeviceToDevice, c->stream)
+                 : cudaMemsetAsync(h->labels.p, 0, sizeof(int32_t) * (size_t)nt, c->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(h->stats.p, 0, 2 * sizeof(unsigned long long), c->stream);
+  if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "dtw fit: %s", cudaGetErrorString(e)));
+  *out = h;
+  return DSP_OK;
+}
+
+int dsp_dtw_topk_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offsets, const int32_t* q_lengths, int64_t nq,
+                        int32_t max_q_frames, double* nbr_cost, int64_t* nbr_idx, int32_t* nbr_label) {
+  if (!h || nq < 0 || (nq && !q_offsets)) return fail(DSP_ERR_INVALID, "bad argument");   // q_feats: NULL when every query is empty
+  dsp_context* c = h->ctx;
+  CU(cudaSetDevice(c->device));
+  const int slices = dtw_fused_slices(nq, h->nt, c->sm_count);
+  const size_t cand = (size_t)dtw_fused_units(nq, c->sm_count) * h->k;   // >= nq * slices * k
+  if (nq > 0) {
+    CU(h->cand_d.ensure(sizeof(float) * cand));
+    CU(h->cand_i.ensure(sizeof(int64_t) * cand));
+  }
+  CU(launch_dtw_topk_fused(q_feats, q_offsets, q_lengths, nq, max_q_frames, h->feats.as<float>(), h->offsets.as<int64_t>(),
+                           h->t_len.as<int32_t>(), h->nt, h->max_t, h->dim, h->k, slices, h->warps, h->index_base,
+                           h->labels.as<int32_t>(), h->cand_d.as<float>(), h->cand_i.as<int64_t>(),
+                           h->stats.as<unsigned long long>(), nbr_cost, nbr_idx, nbr_label, c->stream));
+  c->launches += nq > 0 ? 3 : 1;
+  return DSP_OK;
+}
+
+int dsp_dtw_last_stats(dsp_dtw* h, int64_t* pairs_scored, int64_t* pairs_abandoned) {
+  if (!h) return fail(DSP_ERR_INVALID, "bad argument");
+  CU(cudaSetDevice(h->ctx->device));
+  unsigned long long cnt[2] = {0, 0};
+  CU(cudaMemcpyAsync(cnt, h->stats.p, sizeof cnt, cudaMemcpyDeviceToHost, h->ctx->stream));
+  CU(cudaStreamSynchronize(h->ctx->stream));
+  if (pairs_scored) *pairs_scored = (int64_t)cnt[0];
+  if (pairs_abandoned) *pairs_abandoned = (int64_t)cnt[1];
+  return DSP_OK;
+}
+
+int dsp_dtw_free(dsp_dtw* h) {
+  if (!h) return DSP_OK;
+  cudaSetDevice(h->ctx->device);
+  cudaStreamSynchronize(h->ctx->stream);
+  dtw_release(h);
+  delete h;
   return DSP_OK;
 }
 

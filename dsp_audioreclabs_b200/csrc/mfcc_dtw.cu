@@ -14,8 +14,13 @@
 //                 free), query frames live in registers.  Cost matrix [queries x templates] in fp32.
 //   dtw_topk      one warp per query: the k smallest costs (ties to the lower template index) -> candidates in the
 //                 layout knn_merge_vote consumes, so the row-sharded multi-GPU exchange is the KNN one.
+//   dtw_topk_fused  the same top k without the cost matrix: one warp per (query, slice of templates) keeps the slice's k
+//                 best in registers and abandons a pair once a lower bound on its cost exceeds the k-th;
+//                 dtw_merge_kernel combines the slices with dtw_topk's selection.  Same cell arithmetic
+//                 (dtw_lane_column), so the same bits as the matrix path.
 #include <algorithm>
 #include <cfloat>
+#include <type_traits>
 
 #include <climits>
 #include "kernels.cuh"
@@ -86,7 +91,8 @@ mfcc_kernel(const int16_t* __restrict__ samples, const int64_t* __restrict__ off
     const double scale = M > 0 ? (double)N / (double)M : 1.0 / 32768.0;   // all samples equal: x - mean = 0 anyway
     const int start = seg_start[u], end = min(seg_end[u], n);
     const int seg = end - start;
-    const int nf = (int)frame_count_host_device(seg, a.frame_length, a.frame_shift);
+    // rows [mfcc_offsets[u], mfcc_offsets[u + 1]) belong to the utterance: never more frames than that capacity
+    const int nf = (int)std::min<int64_t>(frame_count_host_device(seg, a.frame_length, a.frame_shift), mfcc_offsets[u + 1] - mfcc_offsets[u]);
     if (tid == 0 && n_frames_out) n_frames_out[u] = nf;
     const int64_t obase = mfcc_offsets[u];
     for (int f = 0; f < nf; ++f) {
@@ -142,7 +148,7 @@ mfcc_kernel(const int16_t* __restrict__ samples, const int64_t* __restrict__ off
 }
 
 // ---------------------------------------------------------------------------------------
-// DTW: one warp-sized CTA per (query, template) pair
+// DTW: one warp per (query, template) pair
 // ---------------------------------------------------------------------------------------
 // Lane L owns R consecutive query frames of a STRIP of 32 R rows (in registers) and runs one column behind lane L - 1:
 // D[i-1][j] crosses the lane boundary by one shfl_up per step.  Queries longer than a strip are processed strip by
@@ -151,6 +157,125 @@ mfcc_kernel(const int16_t* __restrict__ samples, const int64_t* __restrict__ off
 // the feature dimension held in registers (R * DMAX <= 128 floats per lane): 16 for the 13 MFCCs, 32 / 64 / 128 for
 // stacked delta features or other embeddings.
 constexpr int kDtwMaxDim = 128;
+constexpr int kDtwFusedWarps = 4;               // warps per CTA of dtw_topk_fused_kernel (fewer when shared memory is short)
+
+// The R cells a lane owns in column j: D[i][j] = |q_i - t_j| + min(D[i-1][j], D[i][j-1], D[i-1][j-1]).  The one
+// definition of the cell arithmetic (fmaf order, sqrtf, fminf nesting) behind every DTW cost this library reports, so
+// the cost-matrix and the fused top-k paths agree bit for bit.  up / diag: D[i-1][j] / D[i-1][j-1] of the lane's first
+// row; prev: D[i][j-1] of its rows, replaced by D[i][j].  Returns min_r D[i][j] over the lane's rows.
+template <int R, int DMAX>
+__device__ __forceinline__ float dtw_lane_column(const float (&q)[R][DMAX], const float* __restrict__ tj, int dim, int i_lane,
+                                                 int n, int i_last, int j, float up, float diag, float (&prev)[R], float& cur_r) {
+  float t[DMAX];
+#pragma unroll
+  for (int c = 0; c < DMAX; ++c) t[c] = c < dim ? tj[c] : 0.f;
+  float row_min = INFINITY;
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int i = i_lane + r;
+    float d2 = 0.f;
+#pragma unroll
+    for (int c = 0; c < DMAX; ++c) { const float e = q[r][c] - t[c]; d2 = fmaf(e, e, d2); }
+    const float d = sqrtf(d2);
+    float best = fminf(fminf(up, prev[r]), diag);
+    if (i == 0 && j == 0) best = 0.f;
+    const float v = i < n ? d + best : INFINITY;
+    diag = prev[r];                             // D[i][j-1] is the diagonal of the row below
+    up = v;
+    prev[r] = v;
+    row_min = fminf(row_min, v);
+    if (i == i_last) cur_r = v;
+  }
+  return row_min;
+}
+
+// D[n-1][m-1] of one pair on one warp: query rows qp[n][dim] (global), template st[m][dim] and the boundary row
+// brow[m] in shared memory.  q / q_strip: the caller's registers holding the strip of rows starting at q_strip (a warp
+// that keeps one query for many templates loads a one-strip query once).  With PRUNE the pair is abandoned -- the call
+// returns false -- as soon as a lower bound on its final cost is strictly greater than `kth`; sufmin[m] is scratch.
+template <int R, int DMAX, bool PRUNE>
+__device__ __forceinline__ bool dtw_pair(const float* __restrict__ qp, int n, const float* st, int m, int dim, float* brow,
+                                         float* sufmin, float kth, float (&q)[R][DMAX], int& q_strip, float& cost) {
+  const int lane = threadIdx.x & 31;
+  for (int j = lane; j < m; j += 32) brow[j] = INFINITY;      // "row -1"
+  __syncwarp();
+  float result = INFINITY;
+  constexpr int kStrip = 32 * R;
+#pragma unroll 1
+  for (int i0 = 0; i0 < n; i0 += kStrip) {
+    const int ns = min(kStrip, n - i0);         // rows of this strip
+    if (q_strip != i0) {                        // this lane's rows of the strip in registers
+#pragma unroll
+      for (int r = 0; r < R; ++r) {
+        const int i = i0 + lane * R + r;
+#pragma unroll
+        for (int c = 0; c < DMAX; ++c) q[r][c] = (i < n && c < dim) ? qp[(size_t)i * dim + c] : 0.f;
+      }
+      q_strip = i0;
+    }
+    if (PRUNE && i0 > 0) {                      // sufmin[j] = min over columns >= j of the previous strip's last row
+      float carry = INFINITY;
+      for (int base = ((m - 1) >> 5) << 5; base >= 0; base -= 32) {
+        const int j = base + lane;
+        float v = j < m ? brow[j] : INFINITY;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const float w = __shfl_down_sync(0xffffffffu, v, o); if (lane + o < 32) v = fminf(v, w); }
+        v = fminf(v, carry);
+        if (j < m) sufmin[j] = v;
+        carry = __shfl_sync(0xffffffffu, v, 0);
+      }
+      __syncwarp();
+    }
+    const bool final_strip = i0 + ns == n;
+    float prev[R];                              // D[i][j-1] of the lane's rows
+#pragma unroll
+    for (int r = 0; r < R; ++r) prev[r] = INFINITY;
+    float top_cur = INFINITY, top_prev = INFINITY;   // D[i-1][j], D[i-1][j-1] from the lane above (lane 0: the boundary row)
+    float bottom = INFINITY;                    // D[last row of the lane][j] of the previous step
+    float col_min = INFINITY;                   // min of D[i][j] over the strip's rows down to this lane's (PRUNE)
+    float last_row_min = INFINITY;              // min over columns <= j of the strip's last row (PRUNE, last lane)
+    const int last_lane = (ns - 1) / R;
+    const int steps = m + last_lane;
+#pragma unroll 1
+    for (int s = 0; s < steps; ++s) {
+      // the lane above finished column j = s - lane in the previous step
+      const float from_above = __shfl_up_sync(0xffffffffu, bottom, 1);
+      const float min_above = PRUNE ? __shfl_up_sync(0xffffffffu, col_min, 1) : INFINITY;
+      top_prev = top_cur;
+      top_cur = lane == 0 ? (s < m ? brow[s] : INFINITY) : from_above;
+      const int j = s - lane;
+      bool hopeless = false;
+      if (j >= 0 && j < m && lane <= last_lane) {
+        float cur_r = INFINITY;
+        const float row_min = dtw_lane_column<R, DMAX>(q, st + j * dim, dim, i0 + lane * R, n, i0 + ns - 1, j, top_cur, top_prev,
+                                                       prev, cur_r);
+        bottom = prev[R - 1];
+        col_min = lane == 0 ? row_min : fminf(min_above, row_min);
+        if (lane == last_lane) {
+          brow[j] = cur_r;                      // the strip's last row: top boundary of the next strip
+          if (final_strip && j == m - 1) result = cur_r;
+          if (PRUNE) {
+            // Early exit.  In fp32, v = d + best with d >= 0 rounds to a value >= best, so D never decreases along the
+            // predecessor chain of the final cell, and that chain visits every row and every column.  Where it crosses
+            // column j it is either (a) in this strip: D >= col_min, the strip's column minimum; (b) above it: it
+            // still has to cross the previous strip's last row at a column >= j: D >= sufmin[j]; or (c) below it (not
+            // in the final strip): it crossed this strip's last row at a column <= j: D >= last_row_min.  The least
+            // of these bounds D[n-1][m-1]; strictly above the k-th cost the pair cannot enter the top k even through
+            // the index tie-break.
+            last_row_min = fminf(last_row_min, cur_r);
+            float bound = fminf(col_min, i0 > 0 ? sufmin[j] : INFINITY);
+            if (!final_strip) bound = fminf(bound, last_row_min);
+            hopeless = bound > kth;
+          }
+        }
+      }
+      if (PRUNE && __any_sync(0xffffffffu, hopeless)) return false;
+    }
+    __syncwarp();
+  }
+  cost = __shfl_sync(0xffffffffu, result, ((n - 1) % kStrip) / R);
+  return true;
+}
 
 template <int R, int DMAX>
 __global__ void __launch_bounds__(32)
@@ -165,86 +290,32 @@ dtw_kernel(const float* __restrict__ qf, const int64_t* __restrict__ qoff, int64
   if (n == 0 || m == 0) { if (lane == 0) *dst = INFINITY; return; }
   const float* tp = tf + toff[ti] * dim;
   for (int i = lane; i < m * dim; i += 32) st[i] = tp[i];
-  for (int j = lane; j < m; j += 32) brow[j] = INFINITY;      // "row -1"
-  __syncwarp();
-  const float* qp = qf + qoff[qi] * dim;
-  float result = INFINITY;
-  constexpr int kStrip = 32 * R;
-#pragma unroll 1
-  for (int i0 = 0; i0 < n; i0 += kStrip) {
-    const int ns = min(kStrip, n - i0);         // rows of this strip
-    // this lane's rows of the strip in registers
-    float q[R][DMAX];
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const int i = i0 + lane * R + r;
-#pragma unroll
-      for (int c = 0; c < DMAX; ++c) q[r][c] = (i < n && c < dim) ? qp[(size_t)i * dim + c] : 0.f;
-    }
-    float prev[R];                              // D[i][j-1] of the lane's rows
-#pragma unroll
-    for (int r = 0; r < R; ++r) prev[r] = INFINITY;
-    float top_cur = INFINITY, top_prev = INFINITY;   // D[i-1][j], D[i-1][j-1] from the lane above (lane 0: the boundary row)
-    float bottom = INFINITY;                    // D[last row of the lane][j] of the previous step
-    const int last_lane = (ns - 1) / R;
-    const int steps = m + last_lane;
-#pragma unroll 1
-    for (int s = 0; s < steps; ++s) {
-      // the lane above finished column j = s - lane in the previous step
-      const float from_above = __shfl_up_sync(0xffffffffu, bottom, 1);
-      top_prev = top_cur;
-      top_cur = lane == 0 ? (s < m ? brow[s] : INFINITY) : from_above;
-      const int j = s - lane;
-      if (j >= 0 && j < m && lane <= last_lane) {
-        float t[DMAX];
-#pragma unroll
-        for (int c = 0; c < DMAX; ++c) t[c] = c < dim ? st[j * dim + c] : 0.f;
-        float up = top_cur, diag = top_prev;
-        float cur_r = INFINITY;
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-          const int i = i0 + lane * R + r;
-          float d2 = 0.f;
-#pragma unroll
-          for (int c = 0; c < DMAX; ++c) { const float e = q[r][c] - t[c]; d2 = fmaf(e, e, d2); }
-          const float d = sqrtf(d2);
-          float best = fminf(fminf(up, prev[r]), diag);
-          if (i == 0 && j == 0) best = 0.f;
-          const float v = i < n ? d + best : INFINITY;
-          diag = prev[r];                       // D[i][j-1] is the diagonal of the row below
-          up = v;
-          prev[r] = v;
-          if (i == i0 + ns - 1) cur_r = v;
-        }
-        bottom = prev[R - 1];
-        if (lane == last_lane) {
-          brow[j] = cur_r;                      // the strip's last row: top boundary of the next strip
-          if (i0 + ns == n && j == m - 1) result = cur_r;
-        }
-      }
-    }
-    __syncwarp();
-  }
-  result = __shfl_sync(0xffffffffu, result, ((n - 1) % kStrip) / R);
+  float q[R][DMAX];
+  int q_strip = -1;
+  float result;
+  dtw_pair<R, DMAX, false>(qf + qoff[qi] * dim, n, st, m, dim, brow, nullptr, INFINITY, q, q_strip, result);
   if (lane == 0) *dst = result;
 }
 
-// k smallest costs per query (ties to the lower template index): one warp per query
-__global__ void dtw_topk_kernel(const float* __restrict__ cost, int64_t nq, int64_t nt, int k, int64_t index_base,
-                                const int32_t* __restrict__ labels, double* __restrict__ nbr_cost,
-                                int64_t* __restrict__ nbr_idx, int32_t* __restrict__ nbr_label) {
+// (cost, index) order of every top-k here: ties to the lower template index
+__device__ __forceinline__ bool dtw_before(float d, int64_t i, float bd, int64_t bi) { return d < bd || (d == bd && i < bi); }
+
+// The k smallest of `count` candidates (cost, local template index) = get(c) of query qi, on one warp: each lane keeps a
+// sorted list of its share, then k rounds of a warp-wide minimum.  Writes (inf, -1, -1) past the valid candidates.
+template <class Get>
+__device__ __forceinline__ void dtw_warp_select(Get get, int64_t count, int k, int64_t qi, int64_t index_base,
+                                                const int32_t* __restrict__ labels, double* __restrict__ nbr_cost,
+                                                int64_t* __restrict__ nbr_idx, int32_t* __restrict__ nbr_label) {
   const int lane = threadIdx.x & 31;
-  const int64_t qi = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (qi >= nq) return;
-  const float* row = cost + qi * nt;
   float bd[kKnnMaxK]; int64_t bi[kKnnMaxK];
   for (int c = 0; c < k; ++c) { bd[c] = INFINITY; bi[c] = INT64_MAX; }
-  for (int64_t i = lane; i < nt; i += 32) {
-    const float d = row[i];
-    if (d < bd[k - 1] || (d == bd[k - 1] && i < bi[k - 1])) {
+  for (int64_t i = lane; i < count; i += 32) {
+    float d; int64_t ix;
+    get(i, d, ix);
+    if (dtw_before(d, ix, bd[k - 1], bi[k - 1])) {
       int s = k - 1;
-      while (s > 0 && (d < bd[s - 1] || (d == bd[s - 1] && i < bi[s - 1]))) { bd[s] = bd[s - 1]; bi[s] = bi[s - 1]; --s; }
-      bd[s] = d; bi[s] = i;
+      while (s > 0 && dtw_before(d, ix, bd[s - 1], bi[s - 1])) { bd[s] = bd[s - 1]; bi[s] = bi[s - 1]; --s; }
+      bd[s] = d; bi[s] = ix;
     }
   }
   int head = 0;
@@ -257,7 +328,7 @@ __global__ void dtw_topk_kernel(const float* __restrict__ cost, int64_t nq, int6
       const float od = __shfl_xor_sync(0xffffffffu, md, o);
       const int64_t oi = __shfl_xor_sync(0xffffffffu, mi, o);
       const int oo = __shfl_xor_sync(0xffffffffu, owner, o);
-      if (od < md || (od == md && oi < mi)) { md = od; mi = oi; owner = oo; }
+      if (dtw_before(od, oi, md, mi)) { md = od; mi = oi; owner = oo; }
     }
     if (owner == lane && mi != INT64_MAX) ++head;
     if (lane == 0) {
@@ -267,6 +338,82 @@ __global__ void dtw_topk_kernel(const float* __restrict__ cost, int64_t nq, int6
       if (nbr_label) nbr_label[qi * k + c] = valid ? labels[mi] : -1;
     }
   }
+}
+
+// k smallest costs per query (ties to the lower template index): one warp per query
+__global__ void dtw_topk_kernel(const float* __restrict__ cost, int64_t nq, int64_t nt, int k, int64_t index_base,
+                                const int32_t* __restrict__ labels, double* __restrict__ nbr_cost,
+                                int64_t* __restrict__ nbr_idx, int32_t* __restrict__ nbr_label) {
+  const int64_t qi = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (qi >= nq) return;
+  const float* row = cost + qi * nt;
+  dtw_warp_select([&](int64_t i, float& d, int64_t& ix) { d = row[i]; ix = i; }, nt, k, qi, index_base, labels, nbr_cost,
+                  nbr_idx, nbr_label);
+}
+
+// DTW with the top-k fused in and no cost matrix: one warp per (query, slice of templates).  The warp scores its slice's
+// templates one after another (dtw_pair with PRUNE) and keeps the slice's k best (cost, index) pairs in registers, entry
+// c on lane c, so the k-th cost that decides the early exit is one shuffle away.  Output: cand_d / cand_i [unit][k],
+// (inf, INT64_MAX) where the slice has fewer than k, merged per query by dtw_merge_kernel.  stats[0] / [1] count the
+// pairs scored to the last cell / abandoned.
+template <int R, int DMAX>
+__global__ void __launch_bounds__(kDtwFusedWarps * 32, 1)
+dtw_topk_fused_kernel(const float* __restrict__ qf, const int64_t* __restrict__ qoff, const int32_t* __restrict__ qlen, int64_t nq,
+                      const float* __restrict__ tf, const int64_t* __restrict__ toff, const int32_t* __restrict__ tlen,
+                      int64_t nt, int dim, int max_t_frames, int slices, int k, float* __restrict__ cand_d,
+                      int64_t* __restrict__ cand_i, unsigned long long* __restrict__ stats) {
+  extern __shared__ float smem[];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int64_t unit = (int64_t)blockIdx.x * (blockDim.x >> 5) + w;
+  if (unit >= nq * slices) return;              // whole warps only: no CTA-wide barrier below
+  const int64_t qi = unit / slices, sl = unit % slices;
+  float* st = smem + (size_t)w * ((size_t)max_t_frames * (dim + 2));   // template [m][dim], boundary row, suffix minima
+  float* brow = st + (size_t)max_t_frames * dim;
+  float* sufmin = brow + max_t_frames;
+  const int n = qlen ? qlen[qi] : (int)(qoff[qi + 1] - qoff[qi]);
+  const float* qp = qf + qoff[qi] * dim;
+  const int64_t t_end = nt * (sl + 1) / slices;
+  float my_d = INFINITY, kth = INFINITY;
+  int64_t my_i = INT64_MAX;
+  float q[R][DMAX];
+  int q_strip = -1;
+  unsigned long long scored = 0, abandoned = 0;
+#pragma unroll 1
+  for (int64_t ti = nt * sl / slices; ti < t_end; ++ti) {
+    const int m = tlen[ti];
+    float cost = INFINITY;
+    if (n > 0 && m > 0) {
+      const float* tp = tf + toff[ti] * dim;
+      __syncwarp();                             // the previous pair is done with st
+      for (int i = lane; i < m * dim; i += 32) st[i] = tp[i];
+      if (!dtw_pair<R, DMAX, true>(qp, n, st, m, dim, brow, sufmin, kth, q, q_strip, cost)) { ++abandoned; continue; }
+    }
+    ++scored;
+    if (cost <= kth) {                          // insert into the sorted list held one entry per lane
+      const bool before = dtw_before(cost, ti, my_d, my_i);
+      const bool shift = __shfl_up_sync(0xffffffffu, (int)before, 1) && lane > 0;
+      const float up_d = __shfl_up_sync(0xffffffffu, my_d, 1);
+      const int64_t up_i = __shfl_up_sync(0xffffffffu, my_i, 1);
+      if (lane < k) {
+        if (shift) { my_d = up_d; my_i = up_i; }
+        else if (before) { my_d = cost; my_i = ti; }
+      }
+      kth = __shfl_sync(0xffffffffu, my_d, k - 1);
+    }
+  }
+  if (lane < k) { cand_d[unit * k + lane] = my_d; cand_i[unit * k + lane] = my_i; }
+  if (lane == 0) { atomicAdd(stats, scored); atomicAdd(stats + 1, abandoned); }
+}
+
+// the slices' candidates of one query -> its top k: one warp per query, dtw_topk_kernel's selection
+__global__ void dtw_merge_kernel(const float* __restrict__ cand_d, const int64_t* __restrict__ cand_i, int64_t nq, int slices,
+                                 int k, int64_t index_base, const int32_t* __restrict__ labels, double* __restrict__ nbr_cost,
+                                 int64_t* __restrict__ nbr_idx, int32_t* __restrict__ nbr_label) {
+  const int64_t qi = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (qi >= nq) return;
+  const int64_t base = qi * slices * k;
+  dtw_warp_select([&](int64_t i, float& d, int64_t& ix) { d = cand_d[base + i]; ix = cand_i[base + i]; }, (int64_t)slices * k, k,
+                  qi, index_base, labels, nbr_cost, nbr_idx, nbr_label);
 }
 
 }  // namespace
@@ -292,6 +439,24 @@ int dtw_max_query_frames() { return INT32_MAX; }      // any length: strips of 3
 int dtw_max_dim() { return kDtwMaxDim; }
 size_t dtw_smem_bytes(int max_t_frames, int dim) { return ((size_t)std::max(max_t_frames, 1) * dim + (size_t)std::max(max_t_frames, 1)) * sizeof(float); }
 
+namespace {
+// The (R, DMAX) build for a feature dimension and a query length: DMAX the smallest register row that holds a frame,
+// R the largest strip the registers allow (R * DMAX <= 128), and for the 13 MFCCs the smallest strip that holds the
+// longest query -- a strip with idle lanes costs R per step where one of 32 R rows costs 1.  Any build gives the same
+// bits: padded features add fmaf(0, 0, d2) = d2, and strips only change where a row is held.
+template <class F>
+cudaError_t dtw_build(int dim, int max_q_frames, F&& f) {
+  using std::integral_constant;
+  if (dim > 64) return f(integral_constant<int, 1>{}, integral_constant<int, 128>{});
+  if (dim > 32) return f(integral_constant<int, 2>{}, integral_constant<int, 64>{});
+  if (dim > 16) return f(integral_constant<int, 4>{}, integral_constant<int, 32>{});
+  if (max_q_frames <= 32) return f(integral_constant<int, 1>{}, integral_constant<int, 16>{});
+  if (max_q_frames <= 64) return f(integral_constant<int, 2>{}, integral_constant<int, 16>{});
+  if (max_q_frames <= 128) return f(integral_constant<int, 4>{}, integral_constant<int, 16>{});
+  return f(integral_constant<int, 8>{}, integral_constant<int, 16>{});
+}
+}  // namespace
+
 cudaError_t launch_dtw(const float* qf, const int64_t* qoff, int64_t nq, int max_q_frames, const float* tf, const int64_t* toff,
                        int64_t nt, int max_t_frames, int dim, float* cost, cudaStream_t st) {
   if (nq == 0 || nt == 0) return cudaSuccess;
@@ -302,23 +467,54 @@ cudaError_t launch_dtw(const float* qf, const int64_t* qoff, int64_t nq, int max
     const int64_t qc = std::min<int64_t>(65535, nq - q0);
     const dim3 grid((unsigned)nt, (unsigned)qc);
     const float* cq = qf; const int64_t* oq = qoff + q0; float* cc = cost + q0 * nt;
-    auto run = [&](auto kern) -> cudaError_t {
+    cudaError_t e = dtw_build(dim, max_q_frames, [&](auto r, auto d) -> cudaError_t {
+      auto kern = dtw_kernel<decltype(r)::value, decltype(d)::value>;
       cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) return e;
       kern<<<grid, 32, smem, st>>>(cq, oq, qc, tf, toff, nt, dim, std::max(max_t_frames, 1), cc);
       return cudaGetLastError();
-    };
-    cudaError_t e;
-    if (dim > 64) e = run(dtw_kernel<1, 128>);
-    else if (dim > 32) e = run(dtw_kernel<2, 64>);
-    else if (dim > 16) e = run(dtw_kernel<4, 32>);
-    else if (max_q_frames <= 32) e = run(dtw_kernel<1, 16>);
-    else if (max_q_frames <= 64) e = run(dtw_kernel<2, 16>);
-    else if (max_q_frames <= 128) e = run(dtw_kernel<4, 16>);
-    else e = run(dtw_kernel<8, 16>);
+    });
     if (e != cudaSuccess) return e;
   }
   return cudaSuccess;
+}
+
+size_t dtw_fused_smem_per_warp(int max_t_frames, int dim) { return (size_t)std::max(max_t_frames, 1) * (dim + 2) * sizeof(float); }
+int dtw_fused_max_warps() { return kDtwFusedWarps; }
+
+int64_t dtw_fused_units(int64_t nq, int sm_count) { return std::max<int64_t>(nq, (int64_t)sm_count * 32); }
+
+int dtw_fused_slices(int64_t nq, int64_t nt, int sm_count) {
+  // enough (query, slice) warps for a few waves when queries are few, but slices of >= 32 templates so that the k-th
+  // cost is known early; nq * slices <= dtw_fused_units(nq): scratch sized for nq serves every smaller call
+  if (nq < 1) return 1;
+  const int64_t by_units = dtw_fused_units(nq, sm_count) / nq;
+  return (int)std::max<int64_t>(1, std::min<int64_t>(by_units, nt / 32));
+}
+
+cudaError_t launch_dtw_topk_fused(const float* qf, const int64_t* qoff, const int32_t* qlen, int64_t nq, int max_q_frames,
+                                  const float* tf, const int64_t* toff, const int32_t* tlen, int64_t nt, int max_t_frames, int dim,
+                                  int k, int slices, int warps, int64_t index_base, const int32_t* labels, float* cand_d,
+                                  int64_t* cand_i, unsigned long long* stats, double* nbr_cost, int64_t* nbr_idx,
+                                  int32_t* nbr_label, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(stats, 0, 2 * sizeof(unsigned long long), st);
+  if (e != cudaSuccess || nq == 0) return e;
+  if (dim > kDtwMaxDim || k < 1 || k > kKnnMaxK || warps < 1 || warps > kDtwFusedWarps) return cudaErrorInvalidValue;
+  const int mt = std::max(max_t_frames, 1);
+  const size_t smem = dtw_fused_smem_per_warp(mt, dim) * warps;
+  const int64_t units = nq * slices;
+  e = dtw_build(dim, max_q_frames > 0 ? max_q_frames : 128, [&](auto r, auto d) -> cudaError_t {
+    auto kern = dtw_topk_fused_kernel<decltype(r)::value, decltype(d)::value>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<(unsigned)((units + warps - 1) / warps), 32 * warps, smem, st>>>(qf, qoff, qlen, nq, tf, toff, tlen, nt, dim, mt,
+                                                                            slices, k, cand_d, cand_i, stats);
+    return cudaGetLastError();
+  });
+  if (e != cudaSuccess) return e;
+  dtw_merge_kernel<<<(unsigned)((nq + 7) / 8), 256, 0, st>>>(cand_d, cand_i, nq, slices, k, index_base, labels, nbr_cost, nbr_idx,
+                                                            nbr_label);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_dtw_topk(const float* cost, int64_t nq, int64_t nt, int k, int64_t index_base, const int32_t* labels,

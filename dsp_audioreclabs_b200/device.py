@@ -211,3 +211,147 @@ def zscore_apply_f32(stats, mean, std, out=None, ctx=None):
         out = torch.empty(n, d, dtype=torch.float64, device=stats.device)
     check(ctx.lib.dsp_zscore_apply_f32_device(ctx.handle, _dp(stats), n, d, _dp(mean), _dp(std), _dp(out)))
     return out
+
+
+class DeviceMFCC:
+    """MFCC of the trimmed segments [start, end) of one packed int16 batch layout, on device tensors.
+
+    The output rows are planned on the host from `offsets` alone: utterance b may use rows
+    [mfcc_offsets[b], mfcc_offsets[b + 1]), its untrimmed frame count (dsp_frontend_plan), which bounds the frame count
+    of any segment of it.  So the front end's start / end never leave the device.  Parameters as mfcc_dtw.DEFAULTS."""
+
+    def __init__(self, offsets, frame_length=1102, frame_shift=441, lengths=None, ctx=None, device=None, **params):
+        from . import mfcc_dtw
+        p = dict(mfcc_dtw.DEFAULTS)
+        p.update(params, frame_length=int(frame_length), frame_shift=int(frame_shift))
+        if p["window_type"] not in _capi.WINDOW_IDS:
+            raise ValueError(f"unsupported window type: {p['window_type']}")
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.ctx = ctx or default_context(self.device.index or 0)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        self.n_utts = len(offsets) - 1
+        h_lengths = None if lengths is None else np.ascontiguousarray(lengths, dtype=np.int32)
+        self.h_mfcc_offsets, _, _ = plan(offsets, make_params(frame_length, frame_shift), h_lengths)
+        self.total_frames = int(self.h_mfcc_offsets[-1])
+        self.n_ceps = int(p["n_ceps"])
+        self.filterbank = mfcc_dtw.mel_filterbank(p["n_mels"], p["n_fft"], p["sample_rate"])
+        self.dct = mfcc_dtw.dct_matrix(p["n_ceps"], p["n_mels"])
+        self.params = _capi.MfccParams(p["frame_length"], p["frame_shift"], p["n_fft"], p["n_mels"], p["n_ceps"],
+                                       _capi.WINDOW_IDS[p["window_type"]], p["pre_emphasis"], p["log_floor"])
+        dev = self.device
+        self.offsets = torch.from_numpy(offsets).to(dev)
+        self.lengths = None if h_lengths is None else torch.from_numpy(h_lengths).to(dev)
+        self.mfcc_offsets = torch.from_numpy(self.h_mfcc_offsets).to(dev)
+        # the uploads above were enqueued on torch's current stream; run() may use another one
+        self._ready = torch.cuda.Event()
+        self._ready.record(torch.cuda.current_stream(dev))
+        self._waited = set()
+
+    def run(self, samples, start, end, out=None):
+        """Enqueue the MFCC of `samples` (1-D int16 CUDA tensor laid out by `offsets`) over the segments given by the
+        int32 CUDA tensors start / end (e.g. DeviceFrontend's) on torch's current stream.  Returns (mfcc float32
+        [total_frames, n_ceps], mfcc_offsets int64 [B + 1], n_frames int32 [B]): utterance b's frames are rows
+        mfcc_offsets[b] .. + n_frames[b]; the rest of its rows are left as they were in `out` (if given)."""
+        if not samples.is_cuda or samples.dtype != torch.int16:
+            raise ValueError("samples must be an int16 CUDA tensor")
+        for name, t in (("start", start), ("end", end)):
+            if not t.is_cuda or t.dtype != torch.int32 or not t.is_contiguous() or t.numel() != self.n_utts:
+                raise ValueError(f"{name} must be a contiguous int32 CUDA tensor of {self.n_utts} entries")
+        rows = max(self.total_frames, 1)
+        if out is None:
+            out = torch.empty(rows, self.n_ceps, dtype=torch.float32, device=self.device)
+        elif out.dtype != torch.float32 or not out.is_contiguous() or tuple(out.shape) != (rows, self.n_ceps):
+            raise ValueError(f"out must be a contiguous float32 tensor of shape ({rows}, {self.n_ceps})")
+        n_frames = torch.empty(self.n_utts, dtype=torch.int32, device=self.device)
+        st = torch.cuda.current_stream(self.device)
+        if st.cuda_stream not in self._waited:
+            st.wait_event(self._ready)
+            self._waited.add(st.cuda_stream)
+        self.ctx.set_stream(st.cuda_stream)
+        check(self.ctx.lib.dsp_mfcc_batch_device(
+            self.ctx.handle, _dp(samples.contiguous()), _dp(self.offsets), _dp(self.lengths), _dp(start), _dp(end),
+            self.n_utts, C.byref(self.params), self.filterbank.ctypes.data_as(C.c_void_p),
+            self.dct.ctypes.data_as(C.c_void_p), _dp(self.mfcc_offsets), _dp(out), _dp(n_frames)))
+        return out[:self.total_frames], self.mfcc_offsets, n_frames
+
+
+class DeviceDTW:
+    """k cheapest templates under DTW for device-resident sequences: fit keeps a device copy of the templates, topk
+    scores every (query, template) pair without a cost matrix and abandons pairs that cannot enter the top k."""
+
+    def __init__(self, n_neighbors=1, ctx=None, device=None, index_base=0):
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.ctx = ctx or default_context(self.device.index or 0)
+        self.k = int(n_neighbors)
+        self.index_base = int(index_base)
+        self.handle = None
+
+    def _stream(self):
+        self.ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
+
+    @staticmethod
+    def _check_seqs(feats, offsets, lengths):
+        if not feats.is_cuda or feats.dtype != torch.float32 or feats.dim() != 2 or not feats.is_contiguous():
+            raise ValueError("feats must be a contiguous float32 CUDA tensor [frames, dim]")
+        if not offsets.is_cuda or offsets.dtype != torch.int64 or offsets.dim() != 1 or not offsets.is_contiguous():
+            raise ValueError("offsets must be a contiguous int64 CUDA tensor [n + 1] (in frames)")
+        if lengths is not None and (not lengths.is_cuda or lengths.dtype != torch.int32 or not lengths.is_contiguous()
+                                    or lengths.numel() != offsets.numel() - 1):
+            raise ValueError("lengths must be a contiguous int32 CUDA tensor [n]")
+
+    def fit(self, feats, offsets, labels, lengths=None):
+        """Templates: sequence i is lengths[i] (default offsets[i + 1] - offsets[i]) rows of feats from offsets[i];
+        labels int32 [n] (None: 0).  Synchronises once."""
+        self._check_seqs(feats, offsets, lengths)
+        if labels is not None and (not labels.is_cuda or labels.dtype != torch.int32 or not labels.is_contiguous()):
+            raise ValueError("labels must be a contiguous int32 CUDA tensor")
+        self._stream()
+        self.free()
+        h = C.c_void_p()
+        check(self.ctx.lib.dsp_dtw_fit_device(self.ctx.handle, _dp(feats), _dp(offsets), _dp(lengths), _dp(labels),
+                                              offsets.numel() - 1, feats.shape[1], self.k, self.index_base, C.byref(h)))
+        self.handle = h
+        self.dim = feats.shape[1]
+        return self
+
+    def topk(self, feats, offsets, lengths=None, max_q_frames=None):
+        """(cost float64, template index int64, label int32), each [nq, k], ties to the lower index, (inf, -1, -1)
+        where fewer than k templates have a finite cost.  max_q_frames (optional) only picks the kernel build."""
+        self._check_seqs(feats, offsets, lengths)
+        if feats.shape[1] != self.dim:
+            raise ValueError(f"queries have {feats.shape[1]} features, the templates {self.dim}")
+        self._stream()
+        nq = offsets.numel() - 1
+        cost = torch.empty(nq, self.k, dtype=torch.float64, device=self.device)
+        idx = torch.empty(nq, self.k, dtype=torch.int64, device=self.device)
+        lab = torch.empty(nq, self.k, dtype=torch.int32, device=self.device)
+        check(self.ctx.lib.dsp_dtw_topk_device(self.handle, _dp(feats), _dp(offsets), _dp(lengths), nq,
+                                               int(max_q_frames or 0), _dp(cost), _dp(idx), _dp(lab)))
+        return cost, idx, lab
+
+    def predict(self, feats, offsets, lengths=None, max_q_frames=None):
+        """Majority label of the k cheapest templates, ties to the smallest label: int32 [nq]."""
+        cost, idx, lab = self.topk(feats, offsets, lengths, max_q_frames)
+        nq = cost.shape[0]
+        out = torch.empty(nq, dtype=torch.int32, device=self.device)
+        if nq:
+            check(self.ctx.lib.dsp_knn_merge_vote_device(self.ctx.handle, _dp(cost), _dp(idx), _dp(lab), 1, nq, self.k,
+                                                         _dp(out), None, None))
+        return out
+
+    def last_stats(self):
+        """(pairs scored to their last cell, pairs abandoned early) of the last topk / predict call."""
+        scored, abandoned = C.c_int64(), C.c_int64()
+        check(self.ctx.lib.dsp_dtw_last_stats(self.handle, C.byref(scored), C.byref(abandoned)))
+        return int(scored.value), int(abandoned.value)
+
+    def free(self):
+        if self.handle:
+            self.ctx.lib.dsp_dtw_free(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass

@@ -7,13 +7,19 @@
         samples, plan.offsets, plan.feat_offsets, plan.n_utts, plan.max_len, plan.total_frames, 256, 128, 1, True, 0.5, 0.1, 1.5)
     qn = torch.ops.dsp_audioreclabs.zscore_apply(stats, mean, std)
     labels = torch.ops.dsp_audioreclabs.knn_predict(train_norm, train_labels, qn, 3)
+    p5 = torch_ops.plan(offsets, 1102, 441)            # MFCC rows: the untrimmed frame counts bound every segment's
+    mfcc, n_frames = torch.ops.dsp_audioreclabs.mfcc_batch(   # (start / end of a frontend_batch at 1102 / 441)
+        samples, p5.offsets, start, end, p5.feat_offsets, p5.total_frames, 1102, 441, 2048, 26, 13, 1, 0.97, 1e-10)
+    cost, idx, label = torch.ops.dsp_audioreclabs.dtw_topk(t_feats, t_offsets, t_labels, q_feats, q_offsets, 1)
 
 Each op enqueues libdspfront kernels on torch's CURRENT stream with the tensors' device pointers -- no host copies,
 no torch arithmetic on the path -- and has a fake (meta) implementation, so the ops trace under torch.compile /
 torch.export as opaque calls.  They are tensor-in / tensor-out mirrors of src/audio_processing.py:336-396 +
-src/feature_extraction.py:91-112 (front end), :157-181 (z-score) and src/models.py:52-58 (KNN predict).
+src/feature_extraction.py:91-112 (front end), :157-181 (z-score) and src/models.py:52-58 (KNN predict), plus the
+self-specified MFCC + DTW template matching of mfcc_dtw.py.
 """
 import ctypes as C
+import functools
 from collections import OrderedDict
 from typing import Tuple
 
@@ -171,3 +177,74 @@ def knn_topk(train: torch.Tensor, labels: torch.Tensor, queries: torch.Tensor, k
 def _(train, labels, queries, k):
     m = queries.shape[0]
     return (queries.new_empty((m, k)), queries.new_empty((m, k), dtype=torch.int64), queries.new_empty((m, k), dtype=torch.int32))
+
+
+@functools.lru_cache(maxsize=8)
+def _mfcc_tables(n_fft, n_mels, n_ceps):
+    from .mfcc_dtw import DEFAULTS, dct_matrix, mel_filterbank
+    return mel_filterbank(n_mels, n_fft, DEFAULTS["sample_rate"]), dct_matrix(n_ceps, n_mels)
+
+
+@torch.library.custom_op(f"{NS}::mfcc_batch", mutates_args=(), device_types="cuda")
+def mfcc_batch(samples: torch.Tensor, offsets: torch.Tensor, start: torch.Tensor, end: torch.Tensor, mfcc_offsets: torch.Tensor,
+               total_frames: int, frame_length: int, frame_shift: int, n_fft: int, n_mels: int, n_ceps: int, window: int,
+               pre_emphasis: float, log_floor: float) -> Tuple[torch.Tensor, torch.Tensor]:
+    """MFCC of the segments [start, end) of a packed int16 batch (mfcc_dtw.mfcc_batch, on device tensors; HTK-mel
+    filterbank at 44.1 kHz and orthonormal DCT-II from mfcc_dtw).  mfcc_offsets [B+1] are row capacities, e.g.
+    plan(offsets, frame_length, frame_shift).feat_offsets.  -> (mfcc f32 [total_frames, n_ceps], n_frames i32 [B]);
+    rows of an utterance past its n_frames are zero."""
+    if samples.dtype != torch.int16:
+        raise ValueError("mfcc_batch takes 16-bit PCM")
+    dev = samples.device
+    ctx = _ctx_for(samples)
+    fb, dct = _mfcc_tables(n_fft, n_mels, n_ceps)
+    p = _capi.MfccParams(frame_length, frame_shift, n_fft, n_mels, n_ceps, window, pre_emphasis, log_floor)
+    b = offsets.numel() - 1
+    mfcc = torch.zeros(max(total_frames, 1), n_ceps, dtype=torch.float32, device=dev)
+    n_frames = torch.zeros(b, dtype=torch.int32, device=dev)
+    check(ctx.lib.dsp_mfcc_batch_device(ctx.handle, _dp(samples.contiguous()), _dp(offsets.contiguous()), None,
+                                        _dp(start.contiguous()), _dp(end.contiguous()), b, C.byref(p),
+                                        fb.ctypes.data_as(C.c_void_p), dct.ctypes.data_as(C.c_void_p),
+                                        _dp(mfcc_offsets.contiguous()), _dp(mfcc), _dp(n_frames)))
+    return mfcc[:total_frames], n_frames
+
+
+@mfcc_batch.register_fake
+def _(samples, offsets, start, end, mfcc_offsets, total_frames, frame_length, frame_shift, n_fft, n_mels, n_ceps, window,
+      pre_emphasis, log_floor):
+    return (samples.new_empty((total_frames, n_ceps), dtype=torch.float32),
+            samples.new_empty(offsets.shape[0] - 1, dtype=torch.int32))
+
+
+_dtw_cache = OrderedDict()
+
+
+def _dtw_handle(t_feats, t_offsets, t_labels, k):
+    """Fitted handles are kept per (storage, version, k), like _knn_handle: a query batch against the same templates
+    does not copy them again."""
+    from .device import DeviceDTW
+    key = (t_feats.data_ptr(), tuple(t_feats.shape), t_feats._version, t_offsets.data_ptr(), t_offsets.numel(),
+           t_offsets._version, t_labels.data_ptr(), t_labels._version, int(k), t_feats.device.index)
+    dtw = _dtw_cache.get(key)
+    if dtw is None:
+        dtw = DeviceDTW(k, device=t_feats.device).fit(t_feats.contiguous(), t_offsets.contiguous(), t_labels.contiguous())
+        _dtw_cache[key] = dtw
+        while len(_dtw_cache) > 4:
+            _dtw_cache.popitem(last=False)[1].free()
+    return dtw
+
+
+@torch.library.custom_op(f"{NS}::dtw_topk", mutates_args=(), device_types="cuda")
+def dtw_topk(t_feats: torch.Tensor, t_offsets: torch.Tensor, t_labels: torch.Tensor, q_feats: torch.Tensor,
+             q_offsets: torch.Tensor, k: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """k cheapest templates of each query under DTW (mfcc_dtw.DTWClassifier.kneighbors on device tensors): sequences
+    are float32 [frames, dim] with int64 offsets [n+1] in frames; -> (cost f64 [nq,k], template index i64 [nq,k],
+    label i32 [nq,k]), ties to the lower index, (inf, -1, -1) where fewer than k templates have a finite cost."""
+    return _dtw_handle(t_feats, t_offsets, t_labels, k).topk(q_feats.contiguous(), q_offsets.contiguous())
+
+
+@dtw_topk.register_fake
+def _(t_feats, t_offsets, t_labels, q_feats, q_offsets, k):
+    nq = q_offsets.shape[0] - 1
+    return (q_feats.new_empty((nq, k), dtype=torch.float64), q_feats.new_empty((nq, k), dtype=torch.int64),
+            q_feats.new_empty((nq, k), dtype=torch.int32))

@@ -271,6 +271,47 @@ int dsp_dtw_topk_host(dsp_context* ctx, const float* q_feats, const int64_t* q_o
                       int64_t nt, int32_t dim, int32_t k, int64_t index_base, float* cost_out,
                       double* nbr_cost, int64_t* nbr_idx, int32_t* nbr_label);
 
+/* dsp_mfcc_batch_host on DEVICE pointers (samples, offsets, lengths, seg_start, seg_end,
+ * mfcc_offsets, mfcc_out, n_frames_out), enqueued on the context stream without synchronising.
+ * mfcc_offsets[B+1] are capacities: utterance b writes n_frames_out[b] rows from
+ * mfcc_offsets[b] and leaves the rest of [mfcc_offsets[b], mfcc_offsets[b+1]) untouched (never
+ * more rows than that).  frame_signal's frame count is monotone in the segment length and the
+ * segment lies inside the utterance, so the untrimmed counts of dsp_frontend_plan (feat_offsets
+ * for the same frame_length / frame_shift) are valid capacities: front end -> MFCC needs no host
+ * copy of start / end.  filterbank / dct stay HOST pointers; the tables derived from them and from
+ * the parameters (window, twiddles, filter bin ranges) are kept in the context, so a repeated call
+ * with the same tables copies nothing from the host. */
+int dsp_mfcc_batch_device(dsp_context* ctx, const int16_t* samples, const int64_t* offsets,
+                          const int32_t* lengths, const int32_t* seg_start, const int32_t* seg_end,
+                          int64_t n_utts, const dsp_mfcc_params* params, const float* filterbank,
+                          const float* dct, const int64_t* mfcc_offsets, float* mfcc_out,
+                          int32_t* n_frames_out);
+
+/* DTW top-k over resident templates, without the [nq][nt] cost matrix.  Fit copies the templates
+ * (device pointers: ragged [frames][dim] float32, t_offsets[nt+1] in frames, t_lengths[nt] or
+ * NULL = t_offsets[i+1] - t_offsets[i], t_labels[nt] or NULL = 0) into library-owned device
+ * memory, device to device; it synchronises once to learn the longest template.  Limits as
+ * dsp_dtw_topk_host: k <= 16, dim <= 128 (DSP_ERR_UNSUPPORTED before any copy), and
+ * (longest template) x (dim + 2) floats within one CTA's shared memory. */
+typedef struct dsp_dtw dsp_dtw;
+int dsp_dtw_fit_device(dsp_context* ctx, const float* t_feats, const int64_t* t_offsets,
+                       const int32_t* t_lengths, const int32_t* t_labels, int64_t nt, int32_t dim,
+                       int32_t k, int64_t index_base, dsp_dtw** out);
+/* The k cheapest templates of each query (device pointers; q_offsets[nq+1], q_lengths[nq] or
+ * NULL), with the meaning of dsp_dtw_topk_host's outputs: float64 of the fp32 cost -- bit-identical
+ * to its cost matrix entry -- ties to the lower template index, (inf, -1, -1) past nt and for
+ * empty sequences, index_base added.  A pair is abandoned once a lower bound on its cost exceeds
+ * the k-th best of its slice of templates.  Enqueued on the context stream; no synchronisation,
+ * and no allocation once an earlier call had as many queries or more.  max_q_frames is a hint for
+ * the kernel build (<= 0: unknown); any query length is correct.  Any output may be NULL. */
+int dsp_dtw_topk_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offsets,
+                        const int32_t* q_lengths, int64_t nq, int32_t max_q_frames, double* nbr_cost,
+                        int64_t* nbr_idx, int32_t* nbr_label);
+/* Pairs of the last dsp_dtw_topk_device call scored to their last cell / abandoned early (waits
+ * for that call). */
+int dsp_dtw_last_stats(dsp_dtw* h, int64_t* pairs_scored, int64_t* pairs_abandoned);
+int dsp_dtw_free(dsp_dtw* h);
+
 /* ---- batched WAV ingest (SURVEY.md 8 f1) ----------------------------------
  * Replaces the per-file `wave.open` / `readframes` / `np.frombuffer` of load_wav
  * (src/audio_processing.py:21-40) for whole file lists.  Host-only I/O: no CUDA device is
