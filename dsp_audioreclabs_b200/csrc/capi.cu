@@ -7,7 +7,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <iterator>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "kernels.cuh"
@@ -39,36 +42,61 @@ int fail(int code, const char* fmt, ...) {
                   __FILE__, __LINE__);                                                   \
   } while (0)
 
-struct DevBuf {
+// Owners of the library's device memory, pinned memory, streams and events: each one frees what it holds when it is
+// destroyed, so a handle or table entry releases everything with it, on an error return too.  Every destruction keeps
+// two rules:
+//  - the owner's device is current: dsp_destroy, dsp_knn_free and dsp_dtw_free call cudaSetDevice first, and every
+//    other destruction happens inside an entry point that has already set the device;
+//  - no queued work still uses it: those three synchronise before they free, and the window / MFCC table caches are
+//    emptied only after cudaDeviceSynchronize.
+// Host vectors that are sources of stream-ordered copies (MfccEntry::win / tw / range, dsp_dtw::h_len) belong to the
+// owner of the device buffers they fill, so they live as long as those buffers.
+template <bool kPinned>
+struct Buf {
   void* p = nullptr;
   size_t cap = 0;
+  Buf() = default;
+  Buf(const Buf&) = delete;
+  Buf& operator=(const Buf&) = delete;
+  Buf(Buf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  Buf& operator=(Buf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+  ~Buf() { reset(); }
+  // device buffers grow with 1/8 headroom, pinned staging buffers by 256 bytes
   cudaError_t ensure(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
-    size_t want = bytes + bytes / 8 + 256;
-    cudaError_t e = cudaMalloc(&p, want);
+    reset();
+    const size_t want = kPinned ? bytes + 256 : bytes + bytes / 8 + 256;
+    const cudaError_t e = kPinned ? cudaMallocHost(&p, want) : cudaMalloc(&p, want);
     if (e == cudaSuccess) cap = want;
     return e;
   }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
   template <class T> T* as() const { return reinterpret_cast<T*>(p); }
-};
 
-struct PinBuf {
-  void* p = nullptr;
-  size_t cap = 0;
-  cudaError_t ensure(size_t bytes) {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFreeHost(p);
-    p = nullptr; cap = 0;
-    cudaError_t e = cudaMallocHost(&p, bytes + 256);
-    if (e == cudaSuccess) cap = bytes + 256;
-    return e;
+ private:
+  void reset() {
+    if (p && kPinned) cudaFreeHost(p);
+    if (p && !kPinned) cudaFree(p);
+    p = nullptr;
+    cap = 0;
   }
-  void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
-  template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
+using DevBuf = Buf<false>;
+using PinBuf = Buf<true>;
+
+// a stream or event the library created (dsp_context::stream is not one: it may be the caller's)
+template <class T, cudaError_t (*Destroy)(T)>
+struct Owned {
+  T h = nullptr;
+  Owned() = default;
+  Owned(const Owned&) = delete;
+  Owned& operator=(const Owned&) = delete;
+  Owned(Owned&& o) noexcept : h(o.h) { o.h = nullptr; }
+  Owned& operator=(Owned&& o) noexcept { std::swap(h, o.h); return *this; }
+  ~Owned() { if (h) Destroy(h); }
+  operator T() const { return h; }
+};
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
 
 constexpr size_t kMaxSmemPerCta = 227 * 1024;
 constexpr int64_t kFastMaxLen = 1 << 20;          // exact-integer bounds of the fast kernel
@@ -93,10 +121,9 @@ size_t dtype_size(int dtype) {
 }
 
 struct Slot {
-  DevBuf samples, off, foff, eoff, ints, stats, feat, epd_e, epd_z, f64;
+  DevBuf samples, off, ints, stats, feat, epd_e, epd_z, f64;
   PinBuf h_off;
-  cudaEvent_t ev_in = nullptr, ev_k = nullptr, ev_out = nullptr;
-  bool busy = false;
+  Event ev_in, ev_k, ev_out;
 };
 
 }  // namespace
@@ -105,13 +132,14 @@ struct dsp_context {
   int device = 0;
   int sm_count = 0;
   size_t smem_optin = 0;        // opt-in shared memory per block (227 KB on sm_100), static + dynamic
-  cudaStream_t own = nullptr, stream = nullptr, s_in = nullptr, s_out = nullptr;
+  Stream own, s_in, s_out;
+  cudaStream_t stream = nullptr;
   int64_t launches = 0;
   // window tables stay resident per (type, length): a context that alternates windows (three front ends sharing one
   // context, a sweep over frame lengths) never re-uploads or synchronises, and kernels still running on a previously
   // installed stream keep reading the table they were launched with
   struct WinEntry { int type, len; DevBuf w64, w32; };
-  std::vector<WinEntry*> windows;
+  std::vector<std::unique_ptr<WinEntry>> windows;
   const double* win64 = nullptr;
   const float* win32 = nullptr;
   DevBuf counters;   // [0] work counter (u32)  [1] flag count (i32)
@@ -134,7 +162,7 @@ struct dsp_context {
     std::vector<int> range;
     DevBuf d_win, d_tw, d_fb, d_range, d_dct;
   };
-  std::vector<MfccEntry*> mfcc_tables;
+  std::vector<std::unique_ptr<MfccEntry>> mfcc_tables;
   DevBuf mfcc_work;  // work counter of the device MFCC call
 };
 
@@ -182,7 +210,7 @@ int host_window(int type, int n, std::vector<double>& w) {
 }
 
 int ensure_window(dsp_context* c, int type, int fl) {
-  for (auto* e : c->windows)
+  for (const auto& e : c->windows)
     if (e->type == type && e->len == fl) { c->win64 = e->w64.as<double>(); c->win32 = e->w32.as<float>(); return DSP_OK; }
   std::vector<double> w;
   int rc = host_window(type, fl, w);
@@ -190,19 +218,18 @@ int ensure_window(dsp_context* c, int type, int fl) {
   std::vector<float> wf(w.begin(), w.end());
   if (c->windows.size() >= 256) {            // a pathological sweep: drop the tables once nothing can be reading them
     CU(cudaDeviceSynchronize());
-    for (auto* e : c->windows) { e->w64.release(); e->w32.release(); delete e; }
     c->windows.clear();
   }
-  auto* e = new dsp_context::WinEntry{type, fl, {}, {}};
-  if (e->w64.ensure(sizeof(double) * (size_t)fl + 16) != cudaSuccess || e->w32.ensure(sizeof(float) * (size_t)fl + 16) != cudaSuccess) {
-    e->w64.release(); e->w32.release(); delete e;
+  auto e = std::make_unique<dsp_context::WinEntry>();
+  e->type = type;
+  e->len = fl;
+  if (e->w64.ensure(sizeof(double) * (size_t)fl + 16) != cudaSuccess || e->w32.ensure(sizeof(float) * (size_t)fl + 16) != cudaSuccess)
     return fail(DSP_ERR_NOMEM, "device allocation failed");
-  }
   // a fresh table nobody reads yet: blocking copies from the stack vectors are safe and happen once per (type, length)
   CU(cudaMemcpy(e->w64.p, w.data(), sizeof(double) * (size_t)fl, cudaMemcpyHostToDevice));
   CU(cudaMemcpy(e->w32.p, wf.data(), sizeof(float) * (size_t)fl, cudaMemcpyHostToDevice));
-  c->windows.push_back(e);
   c->win64 = e->w64.as<double>(); c->win32 = e->w32.as<float>();
+  c->windows.push_back(std::move(e));
   return DSP_OK;
 }
 
@@ -419,49 +446,45 @@ int mfcc_host_tables(const dsp_mfcc_params* p, const float* filterbank, std::vec
 int ensure_mfcc_tables(dsp_context* c, const dsp_mfcc_params* p, const float* filterbank, const float* dct,
                        dsp_context::MfccEntry** out) {
   const size_t n_fb = (size_t)p->n_mels * (p->n_fft / 2 + 1), n_dct = (size_t)p->n_ceps * p->n_mels;
-  for (auto* e : c->mfcc_tables)
+  for (const auto& e : c->mfcc_tables)
     if (e->frame_length == p->frame_length && e->window == p->window && e->n_fft == p->n_fft && e->n_mels == p->n_mels &&
         e->n_ceps == p->n_ceps && !std::memcmp(e->fb.data(), filterbank, n_fb * sizeof(float)) &&
-        !std::memcmp(e->dct.data(), dct, n_dct * sizeof(float))) { *out = e; return DSP_OK; }
+        !std::memcmp(e->dct.data(), dct, n_dct * sizeof(float))) { *out = e.get(); return DSP_OK; }
   if (c->mfcc_tables.size() >= 16) {           // a sweep over many geometries: drop the tables once nothing can be reading them
     CU(cudaDeviceSynchronize());
-    for (auto* e : c->mfcc_tables) { e->d_win.release(); e->d_tw.release(); e->d_fb.release(); e->d_range.release(); e->d_dct.release(); delete e; }
     c->mfcc_tables.clear();
   }
-  auto* e = new dsp_context::MfccEntry{p->frame_length, p->window, p->n_fft, p->n_mels, p->n_ceps,
-                                       std::vector<float>(filterbank, filterbank + n_fb), std::vector<float>(dct, dct + n_dct),
-                                       {}, {}, {}, {}, {}, {}, {}, {}};
+  auto e = std::make_unique<dsp_context::MfccEntry>();
+  e->frame_length = p->frame_length;
+  e->window = p->window;
+  e->n_fft = p->n_fft;
+  e->n_mels = p->n_mels;
+  e->n_ceps = p->n_ceps;
+  e->fb.assign(filterbank, filterbank + n_fb);
+  e->dct.assign(dct, dct + n_dct);
   int rc = mfcc_host_tables(p, filterbank, e->win, e->tw, e->range);
-  if (rc) { delete e; return rc; }
-  auto drop = [&](int code) { e->d_win.release(); e->d_tw.release(); e->d_fb.release(); e->d_range.release(); e->d_dct.release(); delete e; return code; };
+  if (rc) return rc;
   if (e->d_win.ensure(sizeof(float) * e->win.size()) != cudaSuccess || e->d_tw.ensure(sizeof(float) * e->tw.size()) != cudaSuccess ||
       e->d_fb.ensure(sizeof(float) * n_fb) != cudaSuccess || e->d_range.ensure(sizeof(int) * e->range.size()) != cudaSuccess ||
       e->d_dct.ensure(sizeof(float) * n_dct) != cudaSuccess)
-    return drop(fail(DSP_ERR_NOMEM, "device allocation failed"));
-  const std::pair<DevBuf*, std::pair<const void*, size_t>> copies[] = {
-      {&e->d_win, {e->win.data(), sizeof(float) * e->win.size()}}, {&e->d_tw, {e->tw.data(), sizeof(float) * e->tw.size()}},
-      {&e->d_fb, {e->fb.data(), sizeof(float) * n_fb}}, {&e->d_range, {e->range.data(), sizeof(int) * e->range.size()}},
-      {&e->d_dct, {e->dct.data(), sizeof(float) * n_dct}}};
-  for (const auto& cp : copies) {
-    const cudaError_t err = cudaMemcpyAsync(cp.first->p, cp.second.first, cp.second.second, cudaMemcpyHostToDevice, c->stream);
-    if (err != cudaSuccess) return drop(fail(DSP_ERR_CUDA, "MFCC table upload: %s", cudaGetErrorString(err)));
-  }
-  c->mfcc_tables.push_back(e);
-  *out = e;
+    return fail(DSP_ERR_NOMEM, "device allocation failed");
+  CU(cudaMemcpyAsync(e->d_win.p, e->win.data(), sizeof(float) * e->win.size(), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(e->d_tw.p, e->tw.data(), sizeof(float) * e->tw.size(), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(e->d_fb.p, e->fb.data(), sizeof(float) * n_fb, cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(e->d_range.p, e->range.data(), sizeof(int) * e->range.size(), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(e->d_dct.p, e->dct.data(), sizeof(float) * n_dct, cudaMemcpyHostToDevice, c->stream));
+  *out = e.get();
+  c->mfcc_tables.push_back(std::move(e));
   return DSP_OK;
 }
 
-void dtw_release(dsp_dtw* h) {
-  DevBuf* all[] = {&h->feats, &h->offsets, &h->t_len, &h->labels, &h->cand_d, &h->cand_i, &h->stats};
-  for (DevBuf* b : all) b->release();
-}
-
-// small helper for the single-signal host entry points
+// small helper for the single-signal host entry points: scratch buffers from the context, nullptr past the last one
 struct OneShot {
   dsp_context* c;
   int n_tmp = 0;
   explicit OneShot(dsp_context* ctx) : c(ctx) {}
   template <class T> T* dev(size_t count) {
+    if (n_tmp == (int)std::size(c->tmp)) return nullptr;
     DevBuf& b = c->tmp[n_tmp++];
     if (b.ensure(sizeof(T) * std::max<size_t>(count, 1)) != cudaSuccess) return nullptr;
     return b.as<T>();
@@ -489,49 +512,31 @@ int dsp_create(int device, dsp_context** out) {
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   if (prop.major < 10) return fail(DSP_ERR_NO_DEVICE, "device %d is sm_%d%d; this library is built for sm_100a only", device, prop.major, prop.minor);
-  dsp_context* c = new dsp_context();
+  auto c = std::make_unique<dsp_context>();
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
   c->smem_optin = prop.sharedMemPerBlockOptin;
-  CU(cudaStreamCreateWithFlags(&c->own, cudaStreamNonBlocking));
-  CU(cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
-  CU(cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
+  CU(cudaStreamCreateWithFlags(&c->own.h, cudaStreamNonBlocking));
+  CU(cudaStreamCreateWithFlags(&c->s_in.h, cudaStreamNonBlocking));
+  CU(cudaStreamCreateWithFlags(&c->s_out.h, cudaStreamNonBlocking));
   c->stream = c->own;
   if (const char* e = std::getenv("DSP_PCM_VARIANT")) { int v = std::atoi(e); if (v >= -1 && v <= pcm_num_variants()) c->pcm_variant = v; }
   if (const char* e = std::getenv("DSP_STAGGER_NS")) c->stagger_ns = std::atoi(e);
   if (const char* e = std::getenv("DSP_TMA_CHUNK")) { int v = std::atoi(e); if (v >= 16 && v % 16 == 0) c->tma_chunk = v; }
   for (auto& s : c->slot) {
-    CU(cudaEventCreateWithFlags(&s.ev_in, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&s.ev_k, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&s.ev_out, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&s.ev_in.h, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&s.ev_k.h, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&s.ev_out.h, cudaEventDisableTiming));
   }
-  *out = c;
+  *out = c.release();
   return DSP_OK;
 }
 
 int dsp_destroy(dsp_context* c) {
   if (!c) return DSP_OK;
+  const std::unique_ptr<dsp_context> owner(c);   // its members free the buffers, tables, events and streams
   cudaSetDevice(c->device);
   cudaDeviceSynchronize();
-  for (auto& s : c->slot) {
-    s.samples.release(); s.off.release(); s.foff.release(); s.eoff.release(); s.ints.release();
-    s.stats.release(); s.feat.release(); s.epd_e.release(); s.epd_z.release(); s.f64.release(); s.h_off.release();
-    if (s.ev_in) cudaEventDestroy(s.ev_in);
-    if (s.ev_k) cudaEventDestroy(s.ev_k);
-    if (s.ev_out) cudaEventDestroy(s.ev_out);
-  }
-  for (auto& b : c->tmp) b.release();
-  for (auto* e : c->windows) { e->w64.release(); e->w32.release(); delete e; }
-  c->windows.clear();
-  for (auto* e : c->mfcc_tables) { e->d_win.release(); e->d_tw.release(); e->d_fb.release(); e->d_range.release(); e->d_dct.release(); delete e; }
-  c->mfcc_tables.clear();
-  c->mfcc_work.release();
-  c->counters.release(); c->flag_list.release(); c->prof.release();
-  c->zbuf.release(); c->seqbuf.release();
-  if (c->own) cudaStreamDestroy(c->own);
-  if (c->s_in) cudaStreamDestroy(c->s_in);
-  if (c->s_out) cudaStreamDestroy(c->s_out);
-  delete c;
   return DSP_OK;
 }
 
@@ -640,6 +645,11 @@ int dsp_frontend_batch_host(dsp_context* c, const void* samples, int dtype, cons
   rc = ensure_window(c, p->window, p->frame_length);
   if (rc) return rc;
 
+  // every return, an error inside the chunk loop included, waits until no download into the caller's arrays is in flight
+  struct DrainDownloads {
+    cudaStream_t s_out;
+    ~DrainDownloads() { cudaStreamSynchronize(s_out); }
+  } drain_on_return{c->s_out};
   const unsigned char* src = reinterpret_cast<const unsigned char*>(samples);
   int64_t b0 = 0;
   int chunk = 0;
@@ -649,7 +659,7 @@ int dsp_frontend_batch_host(dsp_context* c, const void* samples, int dtype, cons
     while (b1 < B && (size_t)(offsets[b1 + 1] - offsets[b0]) * esz <= host_chunk_bytes()) ++b1;
     const int64_t bc = b1 - b0;
     Slot& s = c->slot[chunk & 1];
-    if (s.busy) { CU(cudaEventSynchronize(s.ev_out)); s.busy = false; }
+    if (chunk >= 2) CU(cudaEventSynchronize(s.ev_out));   // the downloads of chunk - 2 read this slot's buffers
     const int64_t e0 = offsets[b0], e1 = offsets[b1];
     const int64_t f0 = foff[(size_t)b0], f1 = foff[(size_t)b1], g0 = eoff[(size_t)b0], g1 = eoff[(size_t)b1];
     CU(s.h_off.ensure(sizeof(int64_t) * 4 * (size_t)(bc + 1)));
@@ -730,12 +740,10 @@ int dsp_frontend_batch_host(dsp_context* c, const void* samples, int dtype, cons
     CU(d2h(out->epd_zcr_f64 ? out->epd_zcr_f64 + g0 : nullptr, o.epd_zcr_f64, sizeof(double) * (size_t)(g1 - g0)));
     CU(d2h(out->frames_f64 ? out->frames_f64 + (size_t)f0 * (size_t)p->frame_length : nullptr, o.frames_f64, sizeof(double) * (size_t)(f1 - f0) * (size_t)p->frame_length));
     CU(cudaEventRecord(s.ev_out, c->s_out));
-    s.busy = true;
     b0 = b1;
     ++chunk;
   }
-  for (auto& s : c->slot)
-    if (s.busy) { CU(cudaEventSynchronize(s.ev_out)); s.busy = false; }
+  CU(cudaStreamSynchronize(c->s_out));
   return DSP_OK;
 }
 
@@ -926,35 +934,24 @@ int dsp_zscore_host(dsp_context* c, const double* x, int64_t n, int32_t d, int f
 }
 
 // ---- KNN ----------------------------------------------------------------------------------------
-static void knn_release(dsp_knn* k) {
-  DevBuf* all[] = {&k->train64, &k->train32, &k->labels, &k->tnorm, &k->cand_idx, &k->cand_worst, &k->qnorm,
-                   &k->redo_list, &k->redo_count, &k->nbr_label, &k->q, &k->o_idx, &k->o_dist, &k->o_lab,
-                   &k->tpacked, &k->tnorm_dense, &k->qpacked, &k->qnorm_chunk, &k->dense_flags, &k->part_d, &k->part_i,
-                   &k->tc_train, &k->tc_train_rows, &k->tc_q, &k->tc_flags, &k->refine_list, &k->refine_thr, &k->surv_count, &k->surv_rows, &k->thr0,
-                   &k->prune_perm, &k->prune_geom, &k->prune_box, &k->prune_ws, &k->prune_bound};
-  for (DevBuf* b : all) b->release();
-}
-
 int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* labels, int64_t n, int32_t d, int32_t k,
                        int64_t index_base, dsp_knn** out) {
   if (!c || !out || n < 1 || d < 1 || k < 1 || !train || !labels) return fail(DSP_ERR_INVALID, "bad argument");
   if (k > kKnnMaxK) return fail(DSP_ERR_UNSUPPORTED, "n_neighbors > %d is not supported", kKnnMaxK);
   if (n > INT32_MAX) return fail(DSP_ERR_UNSUPPORTED, "more than 2^31 train rows per shard");
   CU(cudaSetDevice(c->device));
-  dsp_knn* h = new dsp_knn();
+  auto h = std::make_unique<dsp_knn>();
   h->ctx = c; h->n = n; h->d = d; h->k = k; h->index_base = index_base; h->dp = knn_padded_dim(d);
-  auto bail = [&](int code) { knn_release(h); delete h; return code; };
   if (h->train64.ensure(sizeof(double) * (size_t)n * d) != cudaSuccess || h->labels.ensure(sizeof(int32_t) * (size_t)n) != cudaSuccess ||
       h->tnorm.ensure(64) != cudaSuccess || h->redo_count.ensure(64) != cudaSuccess)
-    return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
-  cudaMemcpyAsync(h->train64.p, train, sizeof(double) * (size_t)n * d, cudaMemcpyDeviceToDevice, c->stream);
-  cudaMemcpyAsync(h->labels.p, labels, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToDevice, c->stream);
+    return fail(DSP_ERR_NOMEM, "device allocation failed");
+  CU(cudaMemcpyAsync(h->train64.p, train, sizeof(double) * (size_t)n * d, cudaMemcpyDeviceToDevice, c->stream));
+  CU(cudaMemcpyAsync(h->labels.p, labels, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToDevice, c->stream));
   if (h->dp) {
-    if (h->train32.ensure(sizeof(float) * (size_t)n * h->dp) != cudaSuccess) return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
-    cudaError_t e = knn_pack(h->train64.as<double>(), n, d, h->dp, h->train32.as<float>(), h->tnorm.as<float>(), c->stream);
+    if (h->train32.ensure(sizeof(float) * (size_t)n * h->dp) != cudaSuccess) return fail(DSP_ERR_NOMEM, "device allocation failed");
+    CU(knn_pack(h->train64.as<double>(), n, d, h->dp, h->train32.as<float>(), h->tnorm.as<float>(), c->stream));
     c->launches++;
-    if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "knn_pack: %s", cudaGetErrorString(e)));
-    cudaMemcpyAsync(&h->tnorm_max, h->tnorm.p, sizeof(float), cudaMemcpyDeviceToHost, c->stream);
+    CU(cudaMemcpyAsync(&h->tnorm_max, h->tnorm.p, sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   }
   int tc_flags[2] = {0, 1};
   if (h->dp == 16 && n >= 64 && k < kKnnCand && std::getenv("DSP_KNN_NO_TC16") == nullptr) {
@@ -962,9 +959,8 @@ int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* label
     // holds the rows in the tile order of the pruning plan (principal-axis median splits), train64 / train32 keep the
     // original order
     std::vector<double> host((size_t)n * d);
-    if (cudaMemcpyAsync(host.data(), h->train64.p, sizeof(double) * host.size(), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
-        cudaStreamSynchronize(c->stream) != cudaSuccess)
-      return bail(fail(DSP_ERR_CUDA, "knn fit: %s", cudaGetErrorString(cudaGetLastError())));
+    CU(cudaMemcpyAsync(host.data(), h->train64.p, sizeof(double) * host.size(), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
     KnnPrunePlan plan;
     knn_prune_plan(host.data(), n, d, plan);
     h->prune_tiles = (int64_t)plan.slack.size();
@@ -972,25 +968,22 @@ int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* label
     if (h->tc_train.ensure(knn_tc16_packed_bytes(n, false)) != cudaSuccess || h->tc_flags.ensure(64) != cudaSuccess ||
         h->prune_perm.ensure(sizeof(int) * (size_t)n) != cudaSuccess || h->prune_geom.ensure(sizeof(KnnPruneGeom)) != cudaSuccess ||
         h->prune_box.ensure(2 * box + sizeof(double) * plan.slack.size()) != cudaSuccess)
-      return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
+      return fail(DSP_ERR_NOMEM, "device allocation failed");
     unsigned char* pb = h->prune_box.as<unsigned char>();
-    cudaMemcpyAsync(h->prune_perm.p, plan.perm.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(h->prune_geom.p, &plan.geom, sizeof(KnnPruneGeom), cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(pb, plan.lo.data(), box, cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(pb + box, plan.hi.data(), box, cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(pb + 2 * box, plan.slack.data(), sizeof(double) * plan.slack.size(), cudaMemcpyHostToDevice, c->stream);
-    if (h->tc_train_rows.ensure(knn_tc16_packed_bytes(n, false)) != cudaSuccess) return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
+    CU(cudaMemcpyAsync(h->prune_perm.p, plan.perm.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(h->prune_geom.p, &plan.geom, sizeof(KnnPruneGeom), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(pb, plan.lo.data(), box, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(pb + box, plan.hi.data(), box, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(pb + 2 * box, plan.slack.data(), sizeof(double) * plan.slack.size(), cudaMemcpyHostToDevice, c->stream));
+    if (h->tc_train_rows.ensure(knn_tc16_packed_bytes(n, false)) != cudaSuccess) return fail(DSP_ERR_NOMEM, "device allocation failed");
     // row order for unpruned calls: a walk over spatially ordered tiles finds its neighbours late, and the filter pays
     // for the insertions (2x on the bench's features)
-    cudaError_t e = knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train_rows.p, nullptr, h->tc_flags.as<int>(), c->stream);
-    if (e == cudaSuccess)
-      e = knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train.p, nullptr, h->tc_flags.as<int>(), c->stream,
-                        h->prune_perm.as<int>());
+    CU(knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train_rows.p, nullptr, h->tc_flags.as<int>(), c->stream));
+    CU(knn_tc16_pack(h->train64.as<double>(), n, d, false, h->tc_train.p, nullptr, h->tc_flags.as<int>(), c->stream,
+                     h->prune_perm.as<int>()));
     c->launches++;
-    if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "knn_tc16_pack: %s", cudaGetErrorString(e)));
-    cudaMemcpyAsync(tc_flags, h->tc_flags.p, sizeof tc_flags, cudaMemcpyDeviceToHost, c->stream);
-    if (cudaStreamSynchronize(c->stream) != cudaSuccess)        // (the plan's host vectors are sources of the copies above)
-      return bail(fail(DSP_ERR_CUDA, "knn fit: %s", cudaGetErrorString(cudaGetLastError())));
+    CU(cudaMemcpyAsync(tc_flags, h->tc_flags.p, sizeof tc_flags, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));        // (the plan's host vectors are sources of the copies above)
   }
   int dense_flags[2] = {0, 0};
   if (!h->dp && d <= kKnnDenseMaxDim && std::getenv("DSP_KNN_NO_DENSE") == nullptr) {
@@ -998,19 +991,17 @@ int dsp_knn_fit_device(dsp_context* c, const double* train, const int32_t* label
     if (h->tpacked.ensure(knn_dense_packed_bytes(n, d, true)) != cudaSuccess ||
         h->tnorm_dense.ensure(sizeof(float) * (size_t)knn_dense_padded_rows(n, true)) != cudaSuccess ||
         h->dense_flags.ensure(64) != cudaSuccess)
-      return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
-    cudaError_t e = knn_dense_pack(h->train64.as<double>(), n, d, true, h->tpacked.p, h->tnorm_dense.as<float>(), INFINITY,
-                                   h->dense_flags.as<int>(), true, c->stream);
+      return fail(DSP_ERR_NOMEM, "device allocation failed");
+    CU(knn_dense_pack(h->train64.as<double>(), n, d, true, h->tpacked.p, h->tnorm_dense.as<float>(), INFINITY,
+                      h->dense_flags.as<int>(), true, c->stream));
     c->launches++;
-    if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "knn_dense_pack: %s", cudaGetErrorString(e)));
-    cudaMemcpyAsync(dense_flags, h->dense_flags.p, sizeof dense_flags, cudaMemcpyDeviceToHost, c->stream);
+    CU(cudaMemcpyAsync(dense_flags, h->dense_flags.p, sizeof dense_flags, cudaMemcpyDeviceToHost, c->stream));
   }
-  cudaError_t e = cudaStreamSynchronize(c->stream);
-  if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "knn fit: %s", cudaGetErrorString(e)));
+  CU(cudaStreamSynchronize(c->stream));
   if (h->tpacked.p) std::memcpy(&h->tnorm_max, &dense_flags[0], sizeof(float));
   if (h->dp) h->scan = h->tc_train.p && tc_flags[1] == 0 ? kScanTc16 : kScanFp32;
   else h->scan = h->tpacked.p && dense_flags[1] == 0 ? kScanDense : kScanF64;
-  *out = h;
+  *out = h.release();
   return DSP_OK;
 }
 
@@ -1030,10 +1021,9 @@ int dsp_knn_fit_host(dsp_context* c, const double* train, const int32_t* labels,
 
 int dsp_knn_free(dsp_knn* k) {
   if (!k) return DSP_OK;
+  const std::unique_ptr<dsp_knn> owner(k);
   cudaSetDevice(k->ctx->device);
   cudaStreamSynchronize(k->ctx->stream);
-  knn_release(k);
-  delete k;
   return DSP_OK;
 }
 
@@ -1216,32 +1206,19 @@ int dsp_mfcc_batch_host(dsp_context* c, const int16_t* samples, const int64_t* o
   if (rc) return rc;
   if (n_utts == 0) return DSP_OK;
   CU(cudaSetDevice(c->device));
-  std::vector<float> wf, tw;
-  std::vector<int> range;
-  rc = mfcc_host_tables(p, filterbank, wf, tw, range);
-  if (rc) return rc;
-  const int n_bins = p->n_fft / 2 + 1;
-  const int64_t total_samples = lengths ? offsets[n_utts - 1] + lengths[n_utts - 1] : offsets[n_utts];
   int64_t span = 0;
   for (int64_t b = 0; b < n_utts; ++b) span = std::max<int64_t>(span, offsets[b] + (lengths ? lengths[b] : offsets[b + 1] - offsets[b]));
   const int64_t total_frames = mfcc_offsets[n_utts];
-  (void)total_samples;
   OneShot os(c);
   int16_t* d_s = os.dev<int16_t>((size_t)span);
   int64_t* d_off = os.dev<int64_t>((size_t)n_utts + 1);
   int32_t* d_len = lengths ? os.dev<int32_t>((size_t)n_utts) : nullptr;
   int32_t* d_st = os.dev<int32_t>((size_t)n_utts);
   int32_t* d_en = os.dev<int32_t>((size_t)n_utts);
-  float* d_w = os.dev<float>(wf.size());
-  float* d_tw = os.dev<float>(tw.size());
-  float* d_fb = os.dev<float>((size_t)p->n_mels * n_bins);
-  int* d_rg = os.dev<int>(range.size());
-  float* d_dct = os.dev<float>((size_t)p->n_ceps * p->n_mels);
   int64_t* d_mo = os.dev<int64_t>((size_t)n_utts + 1);
   float* d_out = os.dev<float>((size_t)std::max<int64_t>(total_frames, 1) * p->n_ceps);
   int32_t* d_nf = os.dev<int32_t>((size_t)n_utts);
-  unsigned int* d_cnt = os.dev<unsigned int>(4);
-  if (!d_s || !d_off || (lengths && !d_len) || !d_st || !d_en || !d_w || !d_tw || !d_fb || !d_rg || !d_dct || !d_mo || !d_out || !d_nf || !d_cnt)
+  if (!d_s || !d_off || (lengths && !d_len) || !d_st || !d_en || !d_mo || !d_out || !d_nf)
     return fail(DSP_ERR_NOMEM, "device allocation failed");
   cudaStream_t st = c->stream;
   CU(cudaMemcpyAsync(d_s, samples, sizeof(int16_t) * (size_t)span, cudaMemcpyHostToDevice, st));
@@ -1249,16 +1226,10 @@ int dsp_mfcc_batch_host(dsp_context* c, const int16_t* samples, const int64_t* o
   if (lengths) CU(cudaMemcpyAsync(d_len, lengths, sizeof(int32_t) * (size_t)n_utts, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(d_st, seg_start, sizeof(int32_t) * (size_t)n_utts, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(d_en, seg_end, sizeof(int32_t) * (size_t)n_utts, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_w, wf.data(), sizeof(float) * wf.size(), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_tw, tw.data(), sizeof(float) * tw.size(), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_fb, filterbank, sizeof(float) * (size_t)p->n_mels * n_bins, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_rg, range.data(), sizeof(int) * range.size(), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d_dct, dct, sizeof(float) * (size_t)p->n_ceps * p->n_mels, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(d_mo, mfcc_offsets, sizeof(int64_t) * ((size_t)n_utts + 1), cudaMemcpyHostToDevice, st));
-  MfccArgs a{p->frame_length, p->frame_shift, p->n_fft, p->n_mels, p->n_ceps, p->pre_emphasis, (float)p->log_floor};
-  CU(launch_mfcc(d_s, d_off, d_len, d_st, d_en, n_utts, a, d_w, reinterpret_cast<const float2*>(d_tw), d_fb,
-                 reinterpret_cast<const int2*>(d_rg), d_dct, d_mo, d_out, d_nf, d_cnt, c->sm_count, st));
-  c->launches++;
+  // tables come from the context's cache: a repeated call uploads only its inputs
+  rc = dsp_mfcc_batch_device(c, d_s, d_off, d_len, d_st, d_en, n_utts, p, filterbank, dct, d_mo, d_out, d_nf);
+  if (rc) return rc;
   if (total_frames > 0) CU(cudaMemcpyAsync(mfcc_out, d_out, sizeof(float) * (size_t)total_frames * p->n_ceps, cudaMemcpyDeviceToHost, st));
   if (n_frames_out) CU(cudaMemcpyAsync(n_frames_out, d_nf, sizeof(int32_t) * (size_t)n_utts, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
@@ -1356,25 +1327,21 @@ int dsp_dtw_fit_device(dsp_context* c, const float* t_feats, const int64_t* t_of
   const size_t per_warp = dtw_fused_smem_per_warp((int)max_t, dim);
   if (per_warp > c->smem_optin)
     return fail(DSP_ERR_UNSUPPORTED, "template sequence too long for shared memory (%lld frames x %d features)", (long long)max_t, dim);
-  dsp_dtw* h = new dsp_dtw();
+  auto h = std::make_unique<dsp_dtw>();
   h->ctx = c; h->nt = nt; h->index_base = index_base; h->dim = dim; h->k = k; h->max_t = (int)max_t;
   h->warps = (int)std::min<size_t>(dtw_fused_max_warps(), c->smem_optin / per_warp);
   h->h_len = std::move(len);
-  auto bail = [&](int code) { dtw_release(h); delete h; return code; };
   if (h->feats.ensure(sizeof(float) * (size_t)std::max<int64_t>(extent, 1) * dim) != cudaSuccess ||
       h->offsets.ensure(sizeof(int64_t) * (size_t)nt) != cudaSuccess || h->t_len.ensure(sizeof(int32_t) * (size_t)nt) != cudaSuccess ||
       h->labels.ensure(sizeof(int32_t) * (size_t)nt) != cudaSuccess || h->stats.ensure(2 * sizeof(unsigned long long)) != cudaSuccess)
-    return bail(fail(DSP_ERR_NOMEM, "device allocation failed"));
-  cudaError_t e = cudaSuccess;
-  if (extent > 0) e = cudaMemcpyAsync(h->feats.p, t_feats, sizeof(float) * (size_t)extent * dim, cudaMemcpyDeviceToDevice, c->stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(h->offsets.p, t_offsets, sizeof(int64_t) * (size_t)nt, cudaMemcpyDeviceToDevice, c->stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(h->t_len.p, h->h_len.data(), sizeof(int32_t) * (size_t)nt, cudaMemcpyHostToDevice, c->stream);
-  if (e == cudaSuccess)
-    e = t_labels ? cudaMemcpyAsync(h->labels.p, t_labels, sizeof(int32_t) * (size_t)nt, cudaMemcpyDeviceToDevice, c->stream)
-                 : cudaMemsetAsync(h->labels.p, 0, sizeof(int32_t) * (size_t)nt, c->stream);
-  if (e == cudaSuccess) e = cudaMemsetAsync(h->stats.p, 0, 2 * sizeof(unsigned long long), c->stream);
-  if (e != cudaSuccess) return bail(fail(DSP_ERR_CUDA, "dtw fit: %s", cudaGetErrorString(e)));
-  *out = h;
+    return fail(DSP_ERR_NOMEM, "device allocation failed");
+  if (extent > 0) CU(cudaMemcpyAsync(h->feats.p, t_feats, sizeof(float) * (size_t)extent * dim, cudaMemcpyDeviceToDevice, c->stream));
+  CU(cudaMemcpyAsync(h->offsets.p, t_offsets, sizeof(int64_t) * (size_t)nt, cudaMemcpyDeviceToDevice, c->stream));
+  CU(cudaMemcpyAsync(h->t_len.p, h->h_len.data(), sizeof(int32_t) * (size_t)nt, cudaMemcpyHostToDevice, c->stream));
+  if (t_labels) CU(cudaMemcpyAsync(h->labels.p, t_labels, sizeof(int32_t) * (size_t)nt, cudaMemcpyDeviceToDevice, c->stream));
+  else CU(cudaMemsetAsync(h->labels.p, 0, sizeof(int32_t) * (size_t)nt, c->stream));
+  CU(cudaMemsetAsync(h->stats.p, 0, 2 * sizeof(unsigned long long), c->stream));
+  *out = h.release();
   return DSP_OK;
 }
 
@@ -1410,10 +1377,9 @@ int dsp_dtw_last_stats(dsp_dtw* h, int64_t* pairs_scored, int64_t* pairs_abandon
 
 int dsp_dtw_free(dsp_dtw* h) {
   if (!h) return DSP_OK;
+  const std::unique_ptr<dsp_dtw> owner(h);
   cudaSetDevice(h->ctx->device);
   cudaStreamSynchronize(h->ctx->stream);
-  dtw_release(h);
-  delete h;
   return DSP_OK;
 }
 

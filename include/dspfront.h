@@ -248,7 +248,9 @@ int dsp_knn_merge_vote_device(dsp_context* ctx, const double* cand_sqdist, const
  * (:299-333), then pre-emphasis, window, power spectrum of an n_fft-point FFT, the caller's
  * mel filterbank [n_mels][n_fft/2+1], log(max(., log_floor)) and the caller's DCT matrix
  * [n_ceps][n_mels].  mfcc_offsets[B+1] (in frames, from dsp_frame_count(end-start, ...))
- * addresses the ragged output [frames][n_ceps]. */
+ * addresses the ragged output [frames][n_ceps].  dsp_mfcc_batch_host uploads its inputs and runs
+ * dsp_mfcc_batch_device, so it shares the context's table cache: a repeated call with the same
+ * parameters and tables uploads only the samples and the per-utterance arrays. */
 typedef struct {
   int32_t frame_length, frame_shift, n_fft, n_mels, n_ceps;
   int32_t window;        /* dsp_window_type */
