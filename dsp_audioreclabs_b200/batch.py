@@ -85,12 +85,17 @@ def _host_ctx(ctx):
     return ctx
 
 
+def _window_id(window_type):
+    """The C ABI's id of a window name; an unknown name raises the reference's ValueError (audio_processing.py:296)."""
+    if window_type not in WINDOW_IDS:
+        raise ValueError(f"unsupported window type: {window_type}")
+    return WINDOW_IDS[window_type]
+
+
 def make_params(frame_length, frame_shift, window_type="hamming", do_endpoint_detection=True,
                 energy_high_ratio=0.5, energy_low_ratio=0.1, zcr_threshold_ratio=1.5, channels=1,
                 force_exact=False):
-    if window_type not in WINDOW_IDS:
-        raise ValueError(f"unsupported window type: {window_type}")     # audio_processing.py:296
-    return FrontendParams(int(frame_length), int(frame_shift), WINDOW_IDS[window_type],
+    return FrontendParams(int(frame_length), int(frame_shift), _window_id(window_type),
                           int(bool(do_endpoint_detection)), float(energy_high_ratio),
                           float(energy_low_ratio), float(zcr_threshold_ratio), int(channels),
                           int(bool(force_exact)), 0)
@@ -211,10 +216,9 @@ def _f64(x):
 
 
 def window(window_type, length):
-    if window_type not in WINDOW_IDS:
-        raise ValueError(f"unsupported window type: {window_type}")
+    w = _window_id(window_type)
     out = np.empty(int(length), np.float64)
-    check(load_library().dsp_window(WINDOW_IDS[window_type], int(length), _ptr(out)))
+    check(load_library().dsp_window(w, int(length), _ptr(out)))
     return out
 
 
@@ -245,14 +249,13 @@ def endpoint_detection(x, frame_length, frame_shift, energy_high_ratio=0.5, ener
 
 def frame_signal(x, frame_length, frame_shift, window_type="hamming", ctx=None):
     ctx = _host_ctx(ctx)
-    if window_type not in WINDOW_IDS:
-        raise ValueError(f"unsupported window type: {window_type}")
+    w = _window_id(window_type)
     x = _f64(x)
     nf = int(load_library().dsp_frame_count(x.size, int(frame_length), int(frame_shift)))
     out = np.zeros((nf, int(frame_length)), np.float64)
     if nf:
         check(ctx.lib.dsp_frame_signal_host(ctx.handle, _ptr(x), x.size, int(frame_length),
-                                            int(frame_shift), WINDOW_IDS[window_type], _ptr(out)))
+                                            int(frame_shift), w, _ptr(out)))
     return out
 
 
@@ -368,7 +371,7 @@ class KNN:
 
     def last_stats(self):
         """(queries rescanned in float64, scan kind) of the last kneighbors / predict call: 0 float64 only,
-        1 fp32 tiled scan, 2 tensor-core scan."""
+        1 fp32 tiled scan, 2 dense tensor-core scan, 3 tensor-core filter (D <= 15)."""
         n, kind = C.c_int64(), C.c_int32()
         check(self.ctx.lib.dsp_knn_last_stats(self.handle, C.byref(n), C.byref(kind)))
         return int(n.value), int(kind.value)

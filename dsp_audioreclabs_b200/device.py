@@ -10,7 +10,8 @@ import torch
 
 from . import _capi
 from ._capi import FrontendOutputs, check
-from .batch import _axis0_is_inner, default_context, make_params, plan
+from .batch import _axis0_is_inner, _window_id, default_context, make_params, plan
+from .mfcc_dtw import DEFAULTS, _mfcc_setup
 
 _TORCH_DTYPES = {torch.int16: _capi.DSP_S16, torch.uint8: _capi.DSP_U8,
                  torch.float32: _capi.DSP_F32, torch.float64: _capi.DSP_F64}
@@ -18,6 +19,47 @@ _TORCH_DTYPES = {torch.int16: _capi.DSP_S16, torch.uint8: _capi.DSP_U8,
 
 def _dp(t):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def _device(device):
+    """torch.device of `device`, by default torch's current CUDA device."""
+    return torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+
+
+def _bind(device, ctx=None, stream=None):
+    """`ctx` (default: the default context of `device`) with `stream` (default: torch's current stream of `device`)
+    installed, so the C entry points called with it enqueue there."""
+    ctx = ctx or default_context(device.index or 0)
+    ctx.set_stream((torch.cuda.current_stream(device) if stream is None else stream).cuda_stream)
+    return ctx
+
+
+class _Uploads:
+    """Orders launches after the work a constructor enqueued on torch's current stream.  Each stream waits once, before
+    its first launch: a CUDA graph captured on a stream that has already run records no wait on this event."""
+
+    def __init__(self, device):
+        self._done = torch.cuda.Event()
+        self._done.record(torch.cuda.current_stream(device))
+        self._waited = set()
+
+    def wait(self, stream):
+        if stream.cuda_stream not in self._waited:
+            stream.wait_event(self._done)
+            self._waited.add(stream.cuda_stream)
+
+
+def _frontend_outputs(n_utts, n_frames, n_epd, device, epd_lists):
+    """Zero-filled outputs of one front-end batch (n_frames per-frame rows, n_epd endpoint-detection rows when
+    epd_lists) by FrontendOutputs field name, and the FrontendOutputs of their device pointers."""
+    i32 = lambda *shape: torch.zeros(*shape, dtype=torch.int32, device=device)
+    f32 = lambda *shape: torch.zeros(*shape, dtype=torch.float32, device=device)
+    nf, ne = max(n_frames, 1), max(n_epd, 1)
+    outs = dict(start=i32(n_utts), end=i32(n_utts), n_epd_frames=i32(n_utts), n_frames=i32(n_utts), status=i32(n_utts),
+                energy=f32(nf), magnitude=f32(nf), zcr=f32(nf), stats=f32(n_utts, 15),
+                epd_energy=torch.zeros(ne, dtype=torch.float64, device=device) if epd_lists else None,
+                epd_zcr=f32(ne) if epd_lists else None)
+    return outs, FrontendOutputs(**{name: _dp(t) for name, t in outs.items()})
 
 
 class DeviceFrontend:
@@ -31,8 +73,8 @@ class DeviceFrontend:
                  do_endpoint_detection=True, energy_high_ratio=0.5, energy_low_ratio=0.1,
                  zcr_threshold_ratio=1.5, emit_epd_lists=False, force_exact=False, device=None, ctx=None,
                  lengths=None):
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        self.ctx = ctx or default_context(self.device.index or 0)
+        self.device = _device(device)
+        self.ctx = _bind(self.device, ctx)
         self.params = make_params(frame_length, frame_shift, window_type, do_endpoint_detection,
                                   energy_high_ratio, energy_low_ratio, zcr_threshold_ratio, 1, force_exact)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -45,30 +87,13 @@ class DeviceFrontend:
         self.lengths = None if self.h_lengths is None else torch.from_numpy(self.h_lengths).to(dev)
         self.feat_offsets = torch.from_numpy(self.h_feat_offsets).to(dev)
         self.epd_offsets = torch.from_numpy(self.h_epd_offsets).to(dev)
-        b, nf, ne = self.n_utts, int(self.h_feat_offsets[-1]), int(self.h_epd_offsets[-1])
-        i32 = dict(dtype=torch.int32, device=dev)
-        f32 = dict(dtype=torch.float32, device=dev)
-        self.start = torch.zeros(b, **i32)
-        self.end = torch.zeros(b, **i32)
-        self.n_epd_frames = torch.zeros(b, **i32)
-        self.n_frames = torch.zeros(b, **i32)
-        self.status = torch.zeros(b, **i32)
-        self.energy = torch.zeros(max(nf, 1), **f32)
-        self.magnitude = torch.zeros(max(nf, 1), **f32)
-        self.zcr = torch.zeros(max(nf, 1), **f32)
-        self.stats = torch.zeros(b, 15, **f32)
-        self.epd_energy = torch.zeros(max(ne, 1), dtype=torch.float64, device=dev) if emit_epd_lists else None
-        self.epd_zcr = torch.zeros(max(ne, 1), **f32) if emit_epd_lists else None
-        self._out = FrontendOutputs(_dp(self.start), _dp(self.end), _dp(self.n_epd_frames), _dp(self.n_frames),
-                                    _dp(self.status), _dp(self.energy), _dp(self.magnitude), _dp(self.zcr),
-                                    _dp(self.stats), _dp(self.epd_energy), _dp(self.epd_zcr))
-        # the uploads and fills above were enqueued on torch's current stream; run() may use another one
-        self._ready = torch.cuda.Event()
-        self._ready.record(torch.cuda.current_stream(dev))
-        self._waited = set()
+        outs, self._out = _frontend_outputs(self.n_utts, int(self.h_feat_offsets[-1]), int(self.h_epd_offsets[-1]), dev,
+                                            emit_epd_lists)
+        vars(self).update(outs)                   # self.start, self.end, ..., self.epd_zcr
+        self._uploads = _Uploads(dev)
 
     def set_window(self, window_type):
-        self.params.window = _capi.WINDOW_IDS[window_type]
+        self.params.window = _window_id(window_type)
 
     def algorithmic_bytes(self, sample_bytes=2):
         """SURVEY.md section 8(d): s*L + 4*(3*F2 + 15 + 2) [+ 8*F1 when the EPD lists are written],
@@ -88,10 +113,8 @@ class DeviceFrontend:
         self.params.aligned16 = int(samples.data_ptr() % 16 == 0 and
                                     bool(np.all(self.h_offsets[:-1] * samples.element_size() % 16 == 0)))
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
-        if st.cuda_stream not in self._waited:            # once per stream: order the launch after the construction work
-            st.wait_event(self._ready)
-            self._waited.add(st.cuda_stream)
-        self.ctx.set_stream(st.cuda_stream)
+        self._uploads.wait(st)
+        _bind(self.device, self.ctx, st)
         check(self.ctx.lib.dsp_frontend_batch_device(
             self.ctx.handle, _dp(samples), _TORCH_DTYPES[samples.dtype], _dp(self.offsets), _dp(self.lengths),
             _dp(self.feat_offsets), _dp(self.epd_offsets), self.n_utts, self.max_len,
@@ -104,19 +127,16 @@ class DeviceKNN:
     device-resident queries."""
 
     def __init__(self, n_neighbors=3, ctx=None, device=None, index_base=0):
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        self.ctx = ctx or default_context(self.device.index or 0)
+        self.device = _device(device)
+        self.ctx = _bind(self.device, ctx)
         self.k = int(n_neighbors)
         self.index_base = int(index_base)
         self.handle = None
 
-    def _stream(self):
-        self.ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
-
     def fit(self, train, labels):
         assert train.is_cuda and train.dtype == torch.float64 and train.is_contiguous()
         assert labels.is_cuda and labels.dtype == torch.int32
-        self._stream()
+        _bind(self.device, self.ctx)
         self.free()
         h = C.c_void_p()
         check(self.ctx.lib.dsp_knn_fit_device(self.ctx.handle, _dp(train), _dp(labels), train.shape[0],
@@ -129,7 +149,7 @@ class DeviceKNN:
         distance in the WHOLE train set when this handle holds a row shard of it (dsp_knn_topk_bounded_device): the
         shard returns its rows inside that radius -- possibly fewer than k, the rest (-1, inf, -1)."""
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.is_contiguous()
-        self._stream()
+        _bind(self.device, self.ctx)
         m = queries.shape[0]
         idx = torch.empty(m, self.k, dtype=torch.int64, device=self.device)
         d2 = torch.empty(m, self.k, dtype=torch.float64, device=self.device)
@@ -143,21 +163,21 @@ class DeviceKNN:
 
     def predict(self, queries):
         assert queries.is_cuda and queries.dtype == torch.float64 and queries.is_contiguous()
-        self._stream()
+        _bind(self.device, self.ctx)
         out = torch.empty(queries.shape[0], dtype=torch.int32, device=self.device)
         check(self.ctx.lib.dsp_knn_predict_device(self.handle, _dp(queries), queries.shape[0], _dp(out)))
         return out
 
     def last_stats(self):
-        """(queries rescanned in float64, scan kind: 0 float64 only / 1 fp32 tiled / 2 tensor cores) of the last call."""
-        import ctypes as C
+        """(queries rescanned in float64, scan kind) of the last call: 0 float64 only, 1 fp32 tiled scan, 2 dense
+        tensor-core scan, 3 tensor-core filter (D <= 15)."""
         n, kind = C.c_int64(), C.c_int32()
         check(self.ctx.lib.dsp_knn_last_stats(self.handle, C.byref(n), C.byref(kind)))
         return int(n.value), int(kind.value)
 
     def merge_vote(self, cand_d2, cand_idx, cand_lab):
         """[R, m, k] candidate lists (e.g. all-gathered from R row shards) -> labels, idx, d2."""
-        self._stream()
+        _bind(self.device, self.ctx)
         r, m, k = cand_d2.shape
         labels = torch.empty(m, dtype=torch.int32, device=self.device)
         idx = torch.empty(m, k, dtype=torch.int64, device=self.device)
@@ -183,16 +203,12 @@ def zscore_device(x, mean=None, std=None, ctx=None):
     """normalize_features on a CUDA float64 [n, d] tensor: the result of normalize_features(x.cpu().numpy()), whose
     column sums follow the tensor's layout (batch._axis0_is_inner), e.g. pairwise for a transposed tensor."""
     assert x.is_cuda and x.dtype == torch.float64 and x.dim() == 2
-    ctx = ctx or default_context(x.device.index or 0)
-    ctx.set_stream(torch.cuda.current_stream(x.device).cuda_stream)
+    ctx = _bind(x.device, ctx)
     pairwise = _axis0_is_inner(x)
     x = x.contiguous()
     n, d = x.shape
-    fit = mean is None or std is None
-    fm = torch.empty(d, dtype=torch.float64, device=x.device)
-    fs = torch.empty(d, dtype=torch.float64, device=x.device)
-    if fit:
-        check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 2 if pairwise else 1, _dp(fm), _dp(fs), None))
+    fm, fs = _zscore_fit(ctx, x, pairwise) if mean is None or std is None else (None, None)
+    # the apply kernel replaces std == 0 with 1 in place (csrc/misc.cu), so a caller's mean and std are copied first
     m = fm if mean is None else mean.clone()
     s = fs if std is None else std.clone()
     out = torch.empty_like(x)
@@ -200,12 +216,21 @@ def zscore_device(x, mean=None, std=None, ctx=None):
     return out, m, s
 
 
+def _zscore_fit(ctx, x, pairwise):
+    """Column (mean, std) of a contiguous float64 [n, d] CUDA tensor, std == 0 kept; the column sums are pairwise or
+    row by row (batch._axis0_is_inner of the caller's layout)."""
+    n, d = x.shape
+    mean = torch.empty(d, dtype=torch.float64, device=x.device)
+    std = torch.empty(d, dtype=torch.float64, device=x.device)
+    check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 2 if pairwise else 1, _dp(mean), _dp(std), None))
+    return mean, std
+
+
 def zscore_apply_f32(stats, mean, std, out=None, ctx=None):
     """(float32 [n, d] statistics of the fused front end) -> float64 z-scores with the given train mean / std:
     one kernel between DeviceFrontend.stats and DeviceKNN.predict, no torch arithmetic on the path."""
     assert stats.is_cuda and stats.dtype == torch.float32 and stats.is_contiguous() and stats.dim() == 2
-    ctx = ctx or default_context(stats.device.index or 0)
-    ctx.set_stream(torch.cuda.current_stream(stats.device).cuda_stream)
+    ctx = _bind(stats.device, ctx)
     n, d = stats.shape
     if out is None:
         out = torch.empty(n, d, dtype=torch.float64, device=stats.device)
@@ -221,31 +246,22 @@ class DeviceMFCC:
     of any segment of it.  So the front end's start / end never leave the device.  Parameters as mfcc_dtw.DEFAULTS."""
 
     def __init__(self, offsets, frame_length=1102, frame_shift=441, lengths=None, ctx=None, device=None, **params):
-        from . import mfcc_dtw
-        p = dict(mfcc_dtw.DEFAULTS)
+        p = dict(DEFAULTS)
         p.update(params, frame_length=int(frame_length), frame_shift=int(frame_shift))
-        if p["window_type"] not in _capi.WINDOW_IDS:
-            raise ValueError(f"unsupported window type: {p['window_type']}")
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        self.ctx = ctx or default_context(self.device.index or 0)
+        self.params, self.filterbank, self.dct = _mfcc_setup(p)
+        self.device = _device(device)
+        self.ctx = _bind(self.device, ctx)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         self.n_utts = len(offsets) - 1
         h_lengths = None if lengths is None else np.ascontiguousarray(lengths, dtype=np.int32)
         self.h_mfcc_offsets, _, _ = plan(offsets, make_params(frame_length, frame_shift), h_lengths)
         self.total_frames = int(self.h_mfcc_offsets[-1])
         self.n_ceps = int(p["n_ceps"])
-        self.filterbank = mfcc_dtw.mel_filterbank(p["n_mels"], p["n_fft"], p["sample_rate"])
-        self.dct = mfcc_dtw.dct_matrix(p["n_ceps"], p["n_mels"])
-        self.params = _capi.MfccParams(p["frame_length"], p["frame_shift"], p["n_fft"], p["n_mels"], p["n_ceps"],
-                                       _capi.WINDOW_IDS[p["window_type"]], p["pre_emphasis"], p["log_floor"])
         dev = self.device
         self.offsets = torch.from_numpy(offsets).to(dev)
         self.lengths = None if h_lengths is None else torch.from_numpy(h_lengths).to(dev)
         self.mfcc_offsets = torch.from_numpy(self.h_mfcc_offsets).to(dev)
-        # the uploads above were enqueued on torch's current stream; run() may use another one
-        self._ready = torch.cuda.Event()
-        self._ready.record(torch.cuda.current_stream(dev))
-        self._waited = set()
+        self._uploads = _Uploads(dev)
 
     def run(self, samples, start, end, out=None):
         """Enqueue the MFCC of `samples` (1-D int16 CUDA tensor laid out by `offsets`) over the segments given by the
@@ -264,15 +280,19 @@ class DeviceMFCC:
             raise ValueError(f"out must be a contiguous float32 tensor of shape ({rows}, {self.n_ceps})")
         n_frames = torch.empty(self.n_utts, dtype=torch.int32, device=self.device)
         st = torch.cuda.current_stream(self.device)
-        if st.cuda_stream not in self._waited:
-            st.wait_event(self._ready)
-            self._waited.add(st.cuda_stream)
-        self.ctx.set_stream(st.cuda_stream)
-        check(self.ctx.lib.dsp_mfcc_batch_device(
-            self.ctx.handle, _dp(samples.contiguous()), _dp(self.offsets), _dp(self.lengths), _dp(start), _dp(end),
-            self.n_utts, C.byref(self.params), self.filterbank.ctypes.data_as(C.c_void_p),
-            self.dct.ctypes.data_as(C.c_void_p), _dp(self.mfcc_offsets), _dp(out), _dp(n_frames)))
+        self._uploads.wait(st)
+        _mfcc_device(_bind(self.device, self.ctx, st), samples.contiguous(), self.offsets, self.lengths, start, end,
+                     self.params, self.filterbank, self.dct, self.mfcc_offsets, out, n_frames)
         return out[:self.total_frames], self.mfcc_offsets, n_frames
+
+
+def _mfcc_device(ctx, samples, offsets, lengths, start, end, params, filterbank, dct, mfcc_offsets, out, n_frames):
+    """dsp_mfcc_batch_device over contiguous CUDA tensors: int16 samples, int64 offsets / mfcc_offsets [B + 1], int32
+    lengths (or None) / start / end / n_frames [B], float32 out; MfccParams and the host tables of mfcc_dtw."""
+    check(ctx.lib.dsp_mfcc_batch_device(
+        ctx.handle, _dp(samples), _dp(offsets), _dp(lengths), _dp(start), _dp(end), offsets.numel() - 1,
+        C.byref(params), filterbank.ctypes.data_as(C.c_void_p), dct.ctypes.data_as(C.c_void_p), _dp(mfcc_offsets),
+        _dp(out), _dp(n_frames)))
 
 
 class DeviceDTW:
@@ -280,14 +300,11 @@ class DeviceDTW:
     scores every (query, template) pair without a cost matrix and abandons pairs that cannot enter the top k."""
 
     def __init__(self, n_neighbors=1, ctx=None, device=None, index_base=0):
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        self.ctx = ctx or default_context(self.device.index or 0)
+        self.device = _device(device)
+        self.ctx = _bind(self.device, ctx)
         self.k = int(n_neighbors)
         self.index_base = int(index_base)
         self.handle = None
-
-    def _stream(self):
-        self.ctx.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
 
     @staticmethod
     def _check_seqs(feats, offsets, lengths):
@@ -305,7 +322,7 @@ class DeviceDTW:
         self._check_seqs(feats, offsets, lengths)
         if labels is not None and (not labels.is_cuda or labels.dtype != torch.int32 or not labels.is_contiguous()):
             raise ValueError("labels must be a contiguous int32 CUDA tensor")
-        self._stream()
+        _bind(self.device, self.ctx)
         self.free()
         h = C.c_void_p()
         check(self.ctx.lib.dsp_dtw_fit_device(self.ctx.handle, _dp(feats), _dp(offsets), _dp(lengths), _dp(labels),
@@ -320,7 +337,7 @@ class DeviceDTW:
         self._check_seqs(feats, offsets, lengths)
         if feats.shape[1] != self.dim:
             raise ValueError(f"queries have {feats.shape[1]} features, the templates {self.dim}")
-        self._stream()
+        _bind(self.device, self.ctx)
         nq = offsets.numel() - 1
         cost = torch.empty(nq, self.k, dtype=torch.float64, device=self.device)
         idx = torch.empty(nq, self.k, dtype=torch.int64, device=self.device)

@@ -6,11 +6,12 @@ rule as the reference's front end, then the textbook MFCC chain and classic DTW.
 (mel filterbank, DCT matrix) are built here on the host; the arithmetic per sample runs in csrc/mfcc_dtw.cu.
 """
 import ctypes as C
+import functools
 
 import numpy as np
 
 from . import _capi
-from .batch import _host_ctx, _ptr, check, WINDOW_IDS
+from .batch import _host_ctx, _ptr, _window_id, check
 
 DEFAULTS = dict(frame_length=1102, frame_shift=441, n_fft=2048, n_mels=26, n_ceps=13, pre_emphasis=0.97,
                 log_floor=1e-10, sample_rate=44100, window_type="hamming")
@@ -40,6 +41,21 @@ def dct_matrix(n_ceps, n_mels):
     return np.ascontiguousarray(d, dtype=np.float32)
 
 
+@functools.lru_cache(maxsize=8)
+def _mfcc_tables(n_fft, n_mels, n_ceps, sample_rate):
+    fb, dct = mel_filterbank(n_mels, n_fft, sample_rate), dct_matrix(n_ceps, n_mels)
+    fb.flags.writeable = dct.flags.writeable = False          # shared by every caller with these parameters
+    return fb, dct
+
+
+def _mfcc_setup(p):
+    """(MfccParams, filterbank, dct) of a parameter dict with the keys of DEFAULTS; an unknown window type raises
+    ValueError.  The tables are built once per (n_fft, n_mels, n_ceps, sample_rate)."""
+    cp = _capi.MfccParams(p["frame_length"], p["frame_shift"], p["n_fft"], p["n_mels"], p["n_ceps"],
+                          _window_id(p["window_type"]), p["pre_emphasis"], p["log_floor"])
+    return (cp,) + _mfcc_tables(p["n_fft"], p["n_mels"], p["n_ceps"], p["sample_rate"])
+
+
 def mfcc_batch(samples, offsets, start, end, lengths=None, ctx=None, **params):
     """MFCC frames of the segments [start[b], end[b]) of a packed int16 batch (the endpoints come from
     batch.frontend_batch).  Returns (mfcc float32 [total_frames, n_ceps], mfcc_offsets int64 [B + 1])."""
@@ -54,8 +70,7 @@ def mfcc_batch(samples, offsets, start, end, lengths=None, ctx=None, **params):
     end = np.ascontiguousarray(end, dtype=np.int32)
     if lengths is not None:
         lengths = np.ascontiguousarray(lengths, dtype=np.int32)
-    if p["window_type"] not in WINDOW_IDS:
-        raise ValueError(f"unsupported window type: {p['window_type']}")
+    cp, fb, dct = _mfcc_setup(p)
     lib = ctx.lib
     # frame_signal's frame count in closed form (dsp_frame_count; src/audio_processing.py:320-331), vectorised
     seg = np.maximum(end.astype(np.int64) - start.astype(np.int64), 0)
@@ -64,10 +79,6 @@ def mfcc_batch(samples, offsets, start, end, lengths=None, ctx=None, **params):
     mo = np.zeros(b + 1, dtype=np.int64)
     np.cumsum(nfr, out=mo[1:])
     out = np.zeros((int(mo[-1]), p["n_ceps"]), dtype=np.float32)
-    fb = mel_filterbank(p["n_mels"], p["n_fft"], p["sample_rate"])
-    dct = dct_matrix(p["n_ceps"], p["n_mels"])
-    cp = _capi.MfccParams(p["frame_length"], p["frame_shift"], p["n_fft"], p["n_mels"], p["n_ceps"],
-                          WINDOW_IDS[p["window_type"]], p["pre_emphasis"], p["log_floor"])
     got = np.zeros(b, dtype=np.int32)
     check(lib.dsp_mfcc_batch_host(ctx.handle, _ptr(samples), _ptr(offsets), _ptr(lengths), _ptr(start), _ptr(end), b,
                                   C.byref(cp), _ptr(fb), _ptr(dct), _ptr(mo), _ptr(out), _ptr(got)))

@@ -19,30 +19,19 @@ src/feature_extraction.py:91-112 (front end), :157-181 (z-score) and src/models.
 self-specified MFCC + DTW template matching of mfcc_dtw.py.
 """
 import ctypes as C
-import functools
 from collections import OrderedDict
 from typing import Tuple
 
 import numpy as np
 import torch
 
-from . import _capi
-from ._capi import FrontendOutputs, check
-from .batch import _axis0_is_inner, default_context, make_params, plan as _host_plan
+from ._capi import check
+from .batch import _axis0_is_inner, make_params, plan as _host_plan
+from .device import (_TORCH_DTYPES, DeviceDTW, DeviceKNN, _bind, _dp, _frontend_outputs, _mfcc_device, _zscore_fit,
+                     zscore_apply_f32, zscore_device)
+from .mfcc_dtw import DEFAULTS, _mfcc_setup
 
 NS = "dsp_audioreclabs"
-_WINDOWS = ("rectangular", "hamming", "hanning")
-_TORCH_DTYPES = {torch.int16: _capi.DSP_S16, torch.uint8: _capi.DSP_U8, torch.float32: _capi.DSP_F32, torch.float64: _capi.DSP_F64}
-
-
-def _dp(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-def _ctx_for(t):
-    ctx = default_context(t.device.index or 0)
-    ctx.set_stream(torch.cuda.current_stream(t.device).cuda_stream)
-    return ctx
 
 
 class BatchPlan:
@@ -71,20 +60,16 @@ def frontend_batch(samples: torch.Tensor, offsets: torch.Tensor, feat_offsets: t
     """-> (start[B] i32, end[B] i32, n_frames[B] i32, status[B] i32, stats[B,15] f32, energy, magnitude, zcr [total_frames] f32)."""
     if samples.dtype not in _TORCH_DTYPES:
         raise ValueError("samples must be int16 / uint8 / float32 / float64")
-    dev = samples.device
-    ctx = _ctx_for(samples)
-    p = make_params(frame_length, frame_shift, _WINDOWS[window], do_endpoint_detection, energy_high_ratio, energy_low_ratio,
+    ctx = _bind(samples.device)
+    p = make_params(frame_length, frame_shift, "hamming", do_endpoint_detection, energy_high_ratio, energy_low_ratio,
                     zcr_threshold_ratio)
-    i32 = dict(dtype=torch.int32, device=dev)
-    f32 = dict(dtype=torch.float32, device=dev)
-    start, end, n_epd, n_frames, status = (torch.zeros(n_utts, **i32) for _ in range(5))
-    stats = torch.zeros(n_utts, 15, **f32)
-    energy, magnitude, zcr = (torch.zeros(max(total_frames, 1), **f32) for _ in range(3))
-    out = FrontendOutputs(_dp(start), _dp(end), _dp(n_epd), _dp(n_frames), _dp(status), _dp(energy), _dp(magnitude), _dp(zcr),
-                          _dp(stats), None, None)
+    p.window = window                             # an id; the C ABI rejects one outside 0..2
+    # aligned16 stays 0: only device offsets are known here (DeviceFrontend.run decides it from its host offsets)
+    o, out = _frontend_outputs(n_utts, total_frames, 0, samples.device, False)
     check(ctx.lib.dsp_frontend_batch_device(ctx.handle, _dp(samples.contiguous()), _TORCH_DTYPES[samples.dtype], _dp(offsets), None,
                                             _dp(feat_offsets), None, n_utts, max_len, C.byref(p), C.byref(out)))
-    return start, end, n_frames, status, stats, energy[:total_frames], magnitude[:total_frames], zcr[:total_frames]
+    return (o["start"], o["end"], o["n_frames"], o["status"], o["stats"], o["energy"][:total_frames],
+            o["magnitude"][:total_frames], o["zcr"][:total_frames])
 
 
 @frontend_batch.register_fake
@@ -100,13 +85,8 @@ def zscore_fit(x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
     """normalize_features' statistics (feature_extraction.py:171-177): (mean[d], std[d] with 0 -> 1), float64; the
     column sums follow x's layout like NumPy's on x.cpu().numpy() (batch._axis0_is_inner)."""
     assert x.dtype == torch.float64 and x.dim() == 2
-    ctx = _ctx_for(x)
-    pairwise = _axis0_is_inner(x)
-    x = x.contiguous()
-    n, d = x.shape
-    mean = torch.empty(d, dtype=torch.float64, device=x.device)
-    std = torch.empty(d, dtype=torch.float64, device=x.device)
-    check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 2 if pairwise else 1, _dp(mean), _dp(std), None))
+    mean, std = _zscore_fit(_bind(x.device), x.contiguous(), _axis0_is_inner(x))
+    # the rule zscore_device's std gets from the apply kernel
     return mean, torch.where(std == 0, torch.ones_like(std), std)
 
 
@@ -119,17 +99,10 @@ def _(x):
 def zscore_apply(x: torch.Tensor, mean: torch.Tensor, std: torch.Tensor) -> torch.Tensor:
     """(x - mean) / std in float64 (feature_extraction.py:179); x is float64, or the float32 statistics of the front end."""
     assert x.dim() == 2 and mean.dtype == torch.float64 and std.dtype == torch.float64
-    ctx = _ctx_for(x)
     x = x.contiguous()
-    n, d = x.shape
-    out = torch.empty(n, d, dtype=torch.float64, device=x.device)
     if x.dtype == torch.float32:
-        check(ctx.lib.dsp_zscore_apply_f32_device(ctx.handle, _dp(x), n, d, _dp(mean.contiguous()), _dp(std.contiguous()), _dp(out)))
-    else:
-        assert x.dtype == torch.float64
-        m, s = mean.clone(), std.clone()
-        check(ctx.lib.dsp_zscore_device(ctx.handle, _dp(x), n, d, 0, _dp(m), _dp(s), _dp(out)))
-    return out
+        return zscore_apply_f32(x, mean.contiguous(), std.contiguous())
+    return zscore_device(x, mean, std)[0]
 
 
 @zscore_apply.register_fake
@@ -137,20 +110,23 @@ def _(x, mean, std):
     return x.new_empty(x.shape, dtype=torch.float64)
 
 
-_knn_cache = OrderedDict()
+_knn_cache, _dtw_cache = OrderedDict(), OrderedDict()
+
+
+def _fitted(cache, key, fit):
+    """The handle `cache` holds for `key`, or fit()'s: a call on the same tensors (storage, version, k) does not copy or
+    re-pack them again.  A cache keeps the 4 handles fitted last and frees the others."""
+    h = cache.get(key)
+    if h is None:
+        h = cache[key] = fit()
+        while len(cache) > 4:
+            cache.popitem(last=False)[1].free()
+    return h
 
 
 def _knn_handle(train, labels, k):
-    """Fitted handles are kept per (storage, version, k): a predict on the same train tensor does not re-pack it."""
-    from .device import DeviceKNN
     key = (train.data_ptr(), tuple(train.shape), train._version, labels.data_ptr(), labels._version, int(k), train.device.index)
-    knn = _knn_cache.get(key)
-    if knn is None:
-        knn = DeviceKNN(k, device=train.device).fit(train.contiguous(), labels.contiguous())
-        _knn_cache[key] = knn
-        while len(_knn_cache) > 4:
-            _knn_cache.popitem(last=False)[1].free()
-    return knn
+    return _fitted(_knn_cache, key, lambda: DeviceKNN(k, device=train.device).fit(train.contiguous(), labels.contiguous()))
 
 
 @torch.library.custom_op(f"{NS}::knn_predict", mutates_args=(), device_types="cuda")
@@ -179,12 +155,6 @@ def _(train, labels, queries, k):
     return (queries.new_empty((m, k)), queries.new_empty((m, k), dtype=torch.int64), queries.new_empty((m, k), dtype=torch.int32))
 
 
-@functools.lru_cache(maxsize=8)
-def _mfcc_tables(n_fft, n_mels, n_ceps):
-    from .mfcc_dtw import DEFAULTS, dct_matrix, mel_filterbank
-    return mel_filterbank(n_mels, n_fft, DEFAULTS["sample_rate"]), dct_matrix(n_ceps, n_mels)
-
-
 @torch.library.custom_op(f"{NS}::mfcc_batch", mutates_args=(), device_types="cuda")
 def mfcc_batch(samples: torch.Tensor, offsets: torch.Tensor, start: torch.Tensor, end: torch.Tensor, mfcc_offsets: torch.Tensor,
                total_frames: int, frame_length: int, frame_shift: int, n_fft: int, n_mels: int, n_ceps: int, window: int,
@@ -196,16 +166,15 @@ def mfcc_batch(samples: torch.Tensor, offsets: torch.Tensor, start: torch.Tensor
     if samples.dtype != torch.int16:
         raise ValueError("mfcc_batch takes 16-bit PCM")
     dev = samples.device
-    ctx = _ctx_for(samples)
-    fb, dct = _mfcc_tables(n_fft, n_mels, n_ceps)
-    p = _capi.MfccParams(frame_length, frame_shift, n_fft, n_mels, n_ceps, window, pre_emphasis, log_floor)
-    b = offsets.numel() - 1
+    # the tables at DEFAULTS["sample_rate"], which the op does not take (DeviceMFCC has a sample_rate parameter)
+    p, fb, dct = _mfcc_setup(dict(DEFAULTS, frame_length=frame_length, frame_shift=frame_shift, n_fft=n_fft, n_mels=n_mels,
+                                  n_ceps=n_ceps, pre_emphasis=pre_emphasis, log_floor=log_floor))
+    p.window = window                             # an id; the C ABI rejects one outside 0..2
+    # zero-filled, as documented above (DeviceMFCC.run leaves the rows past n_frames as they were)
     mfcc = torch.zeros(max(total_frames, 1), n_ceps, dtype=torch.float32, device=dev)
-    n_frames = torch.zeros(b, dtype=torch.int32, device=dev)
-    check(ctx.lib.dsp_mfcc_batch_device(ctx.handle, _dp(samples.contiguous()), _dp(offsets.contiguous()), None,
-                                        _dp(start.contiguous()), _dp(end.contiguous()), b, C.byref(p),
-                                        fb.ctypes.data_as(C.c_void_p), dct.ctypes.data_as(C.c_void_p),
-                                        _dp(mfcc_offsets.contiguous()), _dp(mfcc), _dp(n_frames)))
+    n_frames = torch.zeros(offsets.numel() - 1, dtype=torch.int32, device=dev)
+    _mfcc_device(_bind(dev), samples.contiguous(), offsets.contiguous(), None, start.contiguous(), end.contiguous(), p, fb,
+                 dct, mfcc_offsets.contiguous(), mfcc, n_frames)
     return mfcc[:total_frames], n_frames
 
 
@@ -216,22 +185,11 @@ def _(samples, offsets, start, end, mfcc_offsets, total_frames, frame_length, fr
             samples.new_empty(offsets.shape[0] - 1, dtype=torch.int32))
 
 
-_dtw_cache = OrderedDict()
-
-
 def _dtw_handle(t_feats, t_offsets, t_labels, k):
-    """Fitted handles are kept per (storage, version, k), like _knn_handle: a query batch against the same templates
-    does not copy them again."""
-    from .device import DeviceDTW
     key = (t_feats.data_ptr(), tuple(t_feats.shape), t_feats._version, t_offsets.data_ptr(), t_offsets.numel(),
            t_offsets._version, t_labels.data_ptr(), t_labels._version, int(k), t_feats.device.index)
-    dtw = _dtw_cache.get(key)
-    if dtw is None:
-        dtw = DeviceDTW(k, device=t_feats.device).fit(t_feats.contiguous(), t_offsets.contiguous(), t_labels.contiguous())
-        _dtw_cache[key] = dtw
-        while len(_dtw_cache) > 4:
-            _dtw_cache.popitem(last=False)[1].free()
-    return dtw
+    return _fitted(_dtw_cache, key, lambda: DeviceDTW(k, device=t_feats.device).fit(
+        t_feats.contiguous(), t_offsets.contiguous(), t_labels.contiguous()))
 
 
 @torch.library.custom_op(f"{NS}::dtw_topk", mutates_args=(), device_types="cuda")
