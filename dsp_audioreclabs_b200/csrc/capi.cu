@@ -1056,7 +1056,8 @@ static int knn_stage_tc16(dsp_knn* h, const double* q, int64_t m, const double* 
   s.qnorm_limit = knn_tc16_max_norm();
   Tc16Work work;
   const void* tpacked = h->tc_train_rows.p;
-  const int64_t visits = knn_tc16_padded_rows(m, true) / kTc16UnitQueries * h->prune_tiles;
+  const int unit_q = knn_prune_unit_queries(m, c->sm_count);
+  const int64_t visits = (m + unit_q - 1) / unit_q * h->prune_tiles;
   if (c->knn_prune && visits <= INT32_MAX) {          // (the tile lists take units x tiles ints, indexed in int)
     // tile pruning: queries in curve order, a seed pass bounds every query's k-th distance U (capped by the caller's
     // bound), and the main pass visits per unit only the tiles that can hold a row within U; its candidates are

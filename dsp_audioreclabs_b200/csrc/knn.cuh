@@ -48,7 +48,6 @@ float knn_tc16_max_norm();                                   // largest |x|^2 th
 int64_t knn_tc16_padded_rows(int64_t rows, bool query);
 size_t knn_tc16_packed_bytes(int64_t rows, bool query);
 constexpr int kTc16TileRows = 128;                           // train rows per filter tile
-constexpr int kTc16UnitQueries = 256;                        // queries per filter work unit
 // flags[0] = max |x|^2 (float bits), flags[1] = 1 when a row is outside the range; norms (optional): |x|^2 per row,
 // at the source row; gather (optional): packed row r holds source row gather[r]
 cudaError_t knn_tc16_pack(const double* x, int64_t rows, int d, bool query, void* packed, float* norms, int* flags, cudaStream_t st,
@@ -65,6 +64,7 @@ struct Tc16Work {
   unsigned long long kept_limit = 0;
   const int* qperm = nullptr;        // packed query position -> query index
   const int* tperm = nullptr;        // packed train position -> train row
+  int unit_queries = 256;            // queries per work unit: 256 (two query blocks) or 128 (one)
 };
 // k: neighbours the caller will certify (the filter keeps k + 2 candidates for k <= 3, else 8); needs n >= 64
 // thr0 (optional, [m], by query index): start every query's filter at this score threshold (knn_bound_thresholds)
@@ -73,9 +73,14 @@ cudaError_t knn_tc16_filter(const void* qpacked, const void* tpacked, int64_t m,
 
 // Tile pruning for the filter (knn_tc16.cu).  At fit the train rows are ordered into 128-row tiles by recursive median
 // splits along their principal axes, and every tile keeps its bounding box in those axes.  Per call the queries are
-// sorted along a space-filling curve into 256-query units; a seed pass over each unit's nearest tiles bounds every
-// query's k-th distance U, and a unit visits only the tiles whose box lies within max U of its own box.
+// sorted along a space-filling curve into units of knn_prune_unit_queries() queries; a seed pass over each unit's nearest
+// tiles bounds every query's k-th distance U, and a unit visits only the tiles whose box lies within max U of its own box.
 constexpr int kPruneMaxDim = 15;
+// Queries per unit of a pruned call: 256 when there are at least kPruneUnitsPerSm such units per SM, else 128.  A
+// 128-query unit needs fewer tiles per query and spreads the lists over twice as many units, but each tile visit scores
+// half as many pairs: on one B200 it won at 2.6 units of 256 per SM (100 k queries) and lost at 26 (1 M queries).
+constexpr int kPruneUnitsPerSm = 8;
+int knn_prune_unit_queries(int64_t m, int sm_count);
 constexpr int kPruneSeedTiles = 4;                           // tiles per unit in the seed pass
 struct KnnPruneGeom {
   int d;

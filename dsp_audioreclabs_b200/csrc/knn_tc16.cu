@@ -14,19 +14,22 @@
 //
 // One persistent CTA per SM, 576 threads:
 //   warp 0      TMA producer (cp.async.bulk, no tensor map: the pack kernels write tiles in the tensor core's canonical
-//               K-major no-swizzle layout, so a tile is ONE contiguous 8 KB copy): the CTA's 256 queries
-//               ({hi, lo} x 2 blocks of 128, double-buffered across work units) and a ring of 128-row train tiles
-//   warp 1      one thread issues tcgen05.mma.cta_group::1.kind::f16, M 128 x N 128 x K 16, six per train tile
-//               (2 query blocks x 3 split passes) into a double-buffered accumulator that fills TMEM
-//               (2 stages x 2 query blocks x 128 columns = 512); tcgen05.commit frees the ring slot and publishes the stage
-//   warps 2-17  epilogue, one query per thread (TMEM lane = query row), two warps per (lane group, query block) on 64
-//               columns of every tile each: tcgen05.ld 32 columns at a time; a 3-input min tree gives the minimum of
-//               each 8 scores and of the 32; only when that beats some lane's 8th-best score does the warp reload the
-//               offending 8 columns and look at them one by one.
+//               K-major no-swizzle layout, so a tile is ONE contiguous 8 KB copy): the work unit's QB query blocks of
+//               128 ({hi, lo} x QB, double-buffered across work units) and a ring of 128-row train tiles
+//   warp 1      one thread issues tcgen05.mma.cta_group::1.kind::f16, M 128 x N 128 x K 16, 3 QB per train tile
+//               (QB query blocks x 3 split passes) into an accumulator of 4 / QB stages that fills TMEM
+//               (4 / QB stages x QB query blocks x 128 columns = 512); tcgen05.commit frees the ring slot and publishes
+//               the stage
+//   warps 2-17  epilogue, one query per thread (TMEM lane = query row), 4 / QB warps per (lane group, query block) on
+//               32 QB columns of every tile each: tcgen05.ld 32 columns at a time; a 3-input min tree gives the minimum of
+//               each 8 scores and of the 32; only when that beats some lane's C-th best score does the lane look at the
+//               offending 8 columns one by one.
 //               After the first few thousand train rows that happens for a few columns in a thousand: the epilogue
 //               costs ~0.6 instructions per pair and the kernel is bound by the TMEM -> register path (4 B per pair).
-// A train tile (8 KB) serves 256 queries, which halves the L2 -> SM operand traffic per pair against one M = 128 block
-// per CTA (the scan moves 25 GB from L2 for 10^11 pairs) and keeps it below the tensor pipe's time.
+// QB = 2 (256-query units): a train tile (8 KB) serves 256 queries, which halves the L2 -> SM operand traffic and the
+// per-tile barrier round trips per pair against QB = 1 (the scan moves 25 GB from L2 for 10^11 pairs).  QB = 1
+// (128-query units) is chosen for pruned calls with few units per SM (knn_prune_unit_queries): a unit visits only the
+// tiles near all of its queries, and 128 queries close on the curve need fewer of them (DESIGN.md §7 item 4).
 #include <cuda_fp16.h>
 
 #include <algorithm>
@@ -50,22 +53,22 @@ constexpr int kRows = 128;                       // rows of one operand tile (qu
 constexpr int kK = 16;                           // padded feature dimension = one MMA K step
 constexpr int kPlaneBytes = kRows * kK * 2;      // one fp16 plane of a tile: 4 KB
 constexpr int kTileBytes = 2 * kPlaneBytes;      // {hi, lo}: 8 KB
-constexpr int kUnitQ = 2 * kRows;                // queries per work unit
-constexpr int kQBufBytes = 2 * kTileBytes;       // two query blocks
+constexpr int kMaxUnitQ = 2 * kRows;            // queries per work unit: QB = 1 or 2 query blocks (query padding: 256)
 constexpr int kTStages = 16;                     // 128 KB of train tiles in flight; with the query buffers and the candidate lists the CTA owns its SM (all of TMEM is allocated)
-constexpr int kAccStages = 2;
+constexpr int kMaxAccStages = 4;                 // QB = 1: 4 stages of 128 columns; QB = 2: 2 stages of 2 x 128
 constexpr int kEpiWarps = 16;
 constexpr int kTcThreads = 32 * (2 + kEpiWarps);
 constexpr int kTmemCols = 512;
 constexpr int kEpiThreads = 32 * kEpiWarps;
 constexpr int kListBytes = 2 * kKnnCand * kEpiThreads * 4;     // per-thread candidate lists: scores and indices, [entry][thread]
-constexpr size_t kTcSmem = 2 * kQBufBytes + (size_t)kTStages * kTileBytes + kListBytes + 1024;   // + mbarriers and the TMEM address slot
+// query buffers, train ring, candidate lists + mbarriers and the TMEM address slot
+constexpr size_t tc_smem(int qb) { return 2 * (size_t)qb * kTileBytes + (size_t)kTStages * kTileBytes + kListBytes + 1024; }
 // canonical K-major no-swizzle layout: core matrix = 8 rows x 16 bytes (128 B contiguous); the two core matrices along
 // K of one 8-row group are adjacent (LBO = 128 B); row groups follow every 256 B (SBO)
 constexpr uint32_t kLBO = 128, kSBO = 256;
 // instruction descriptor (kind::f16): D = F32 (bit 4), A = B = F16, both K-major, N >> 3 at bit 17, M >> 4 at bit 24
 constexpr uint32_t kIdesc = (1u << 4) | ((uint32_t)(kRows >> 3) << 17) | ((uint32_t)(kRows >> 4) << 24);
-static_assert(8 * (4 + 2 * kTStages + 2 * kAccStages) + 8 <= 512, "barrier block of the shared-memory plan (unit slots at 512)");
+static_assert(8 * (4 + 2 * kTStages + 2 * kMaxAccStages) + 8 <= 512, "barrier block of the shared-memory plan (unit slots at 512)");
 constexpr float kPadNorm = 30000.f;              // |t|^2 of padding rows: above every real score (knn_tc16_max_norm)
 
 __device__ __forceinline__ float min3f(float a, float b, float c) { return fminf(fminf(a, b), c); }
@@ -172,15 +175,17 @@ __device__ __noinline__ float tc16_slow8(float v0, float v1, float v2, float v3,
 // kC: candidates kept per query (k + 2 for k <= 3, else 8): a shorter list is inserted into less often (C ln(n / C)
 // insertions per query, each executed by the whole warp for the one or two lanes that need it) and costs less per
 // insertion; the float64 certificate decides, per query, whether it was enough.
-template <int kC>
+template <int kC, int kQB>
 __global__ void __launch_bounds__(kTcThreads, 1)
 knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned char* __restrict__ tpacked, int64_t m, int n,
                        int units, int t_tiles, const int* __restrict__ qflags, int* __restrict__ cand_idx,
                        float* __restrict__ cand_worst, const float* __restrict__ thr0, const Tc16Work w) {
+  constexpr int kUnitQ = kQB * kRows, kQBufBytes = kQB * kTileBytes, kAccStages = 4 / kQB;
+  constexpr int kWarpsPerBlock = 4 / kQB, kWarpCols = 32 * kQB;     // epilogue warps per (lane group, query block)
   extern __shared__ __align__(1024) unsigned char smem[];
   // (a query outside the filter's range was packed as the zero vector: it gets candidates like any other and the rerank
   //  kernel sends it to the exhaustive float64 scan -- qflags is informational)
-  unsigned char* s_q = smem;                                // [2][2 blocks][hi | lo]
+  unsigned char* s_q = smem;                                // [2][kQB blocks][hi | lo]
   unsigned char* s_t = smem + 2 * kQBufBytes;               // [kTStages][hi | lo]
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 2 * kQBufBytes + (size_t)kTStages * kTileBytes);
   uint64_t* q_full = bars;
@@ -254,15 +259,15 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
           tc_fence_after();
           const uint32_t t_hi = smem_u32(s_t + (size_t)s * kTileBytes), t_lo = t_hi + kPlaneBytes;
 #pragma unroll
-          for (int h = 0; h < 2; ++h) {
+          for (int h = 0; h < kQB; ++h) {
             const uint32_t q_hi = q0 + (uint32_t)h * kTileBytes, q_lo = q_hi + kPlaneBytes;
-            const uint32_t d_tmem = tmem_base + (uint32_t)((as * 2 + h) * kRows);
+            const uint32_t d_tmem = tmem_base + (uint32_t)((as * kQB + h) * kRows);
             umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_hi), umma_desc<kLBO, kSBO>(t_hi), kIdesc, 0u);
             umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_hi), umma_desc<kLBO, kSBO>(t_lo), kIdesc, 1u);
             umma_f16(d_tmem, umma_desc<kLBO, kSBO>(q_lo), umma_desc<kLBO, kSBO>(t_hi), kIdesc, 1u);
           }
           umma_commit(&t_empty[s]);                         // ring slot free once these MMAs have read it
-          umma_commit(&acc_full[as]);                       // both query blocks of this stage are complete
+          umma_commit(&acc_full[as]);                       // every query block of this stage is complete
           if (++s == kTStages) { s = 0; ph ^= 1u; }
           if (++as == kAccStages) { as = 0; aph ^= 1u; }
         }
@@ -272,10 +277,10 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
     }
     __syncwarp();
   } else {
-    // ===== epilogue: TMEM lane group = warp % 4 (hardware rule); (warp - 2) / 4 picks the query block and, with two
-    // warps per (lane group, query block), the 64-column half of every tile the warp compares =====
+    // ===== epilogue: TMEM lane group = warp % 4 (hardware rule); (warp - 2) / 4 picks the query block and, with
+    // kWarpsPerBlock warps per (lane group, query block), the kWarpCols columns of every tile the warp compares =====
     const int lg = warp & 3, grp = (warp - 2) >> 2;
-    const int h = grp >> 1, half = grp & 1;
+    const int h = grp / kWarpsPerBlock, part = grp % kWarpsPerBlock;
     const int et = tid - 64;                                   // epilogue thread
     float* l_cd = reinterpret_cast<float*>(smem + 2 * kQBufBytes + (size_t)kTStages * kTileBytes + 1024) + et;     // behind the barrier block
     int* l_ci = reinterpret_cast<int*>(l_cd - et + kKnnCand * kEpiThreads) + et;
@@ -317,47 +322,51 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
         }
         __syncwarp();
       };
-      // Two warps per (lane group, query block), each on its own 64 columns of every tile with its own candidate list:
-      // four epilogue warps per scheduler hide one another's TMEM-load and min-tree latencies (with two, issue slots
-      // were 28 % busy and the tensor pipe 20 %), the accumulator stage goes back to the MMA thread as soon as the 64
-      // scores are in registers, and the two lists are merged once per work unit.
+      // kWarpsPerBlock warps per (lane group, query block), each on its own kWarpCols columns of every tile with its own
+      // candidate list: four epilogue warps per scheduler hide one another's TMEM-load and min-tree latencies (with two,
+      // issue slots were 28 % busy and the tensor pipe 20 %), the accumulator stage goes back to the MMA thread as soon
+      // as the warp's scores are in registers, and the lists are merged once per work unit.
       uint32_t va[32], vb[32];
       int row_next = cnt > 0 ? tile_row(0) : 0;
       for (int tb = 0; tb < cnt; ++tb) {
-        const int base = row_next + half * 64;
+        const int base = row_next + part * kWarpCols;
         if (tb + 1 < cnt) row_next = tile_row(tb + 1);
         mbar_wait(&acc_full[as], aph);
         tc_fence_after();
-        const uint32_t col = (uint32_t)((as * 2 + h) * kRows + half * 64);
+        const uint32_t col = (uint32_t)((as * kQB + h) * kRows + part * kWarpCols);
         tmem_ld32(lane_addr + col, va);
-        tmem_ld32(lane_addr + col + 32, vb);
+        if constexpr (kQB == 2) tmem_ld32(lane_addr + col + 32, vb);
         tmem_ld_wait();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_empty[as]);
         if (++as == kAccStages) { as = 0; aph ^= 1u; }
         process(va, base);
-        process(vb, base + 32);
+        if constexpr (kQB == 2) process(vb, base + 32);
       }
-      // merge: the warp of half 0 folds its partner's list (same lane group, same query block: 128 threads up) into its own
+      // merge: the warp of part 0 folds the lists of its (lane group, query block)'s other warps (128, 256, 384 epilogue
+      // threads up) into its own
       const int pair_bar = 1 + lg + 4 * h;
-      bar_sync(pair_bar, 64);
-      if (half == 0) {
+      bar_sync(pair_bar, 32 * kWarpsPerBlock);
+      if (part == 0) {
         float cd[kC]; int ci[kC];
 #pragma unroll
         for (int c = 0; c < kC; ++c) { cd[c] = l_cd[c * kEpiThreads]; ci[c] = l_ci[c * kEpiThreads]; }
 #pragma unroll
-        for (int b = 0; b < kC; ++b) {
-          float d = l_cd[b * kEpiThreads + 128]; int i = l_ci[b * kEpiThreads + 128];
+        for (int p = 1; p < kWarpsPerBlock; ++p) {
 #pragma unroll
-          for (int c = 0; c < kC; ++c) {          // sorted insertion: carry the displaced entry down the list
-            if (d < cd[c]) { const float td = cd[c]; const int ti = ci[c]; cd[c] = d; ci[c] = i; d = td; i = ti; }
+          for (int b = 0; b < kC; ++b) {
+            float d = l_cd[b * kEpiThreads + p * 128]; int i = l_ci[b * kEpiThreads + p * 128];
+#pragma unroll
+            for (int c = 0; c < kC; ++c) {          // sorted insertion: carry the displaced entry down the list
+              if (d < cd[c]) { const float td = cd[c]; const int ti = ci[c]; cd[c] = d; ci[c] = i; d = td; i = ti; }
+            }
           }
         }
 #pragma unroll
         for (int c = 0; c < kC; ++c) { l_cd[c * kEpiThreads] = cd[c]; l_ci[c * kEpiThreads] = ci[c]; }
       }
-      if (half == 0 && q_idx >= 0) {
+      if (part == 0 && q_idx >= 0) {
 #pragma unroll
         for (int c = 0; c < kKnnCand; ++c) {
           const int i = c < kC ? l_ci[c * kEpiThreads] : -1;
@@ -365,8 +374,8 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
         }
         cand_worst[q_idx] = l_cd[(kC - 1) * kEpiThreads];
       }
-      // the partner must not re-initialise its list for the next unit before it has been read
-      bar_sync(pair_bar, 64);
+      // the other warps must not re-initialise their lists for the next unit before they have been read
+      bar_sync(pair_bar, 32 * kWarpsPerBlock);
     }
   }
   tc_fence_before();
@@ -381,7 +390,7 @@ knn_tc16_filter_kernel(const unsigned char* __restrict__ qpacked, const unsigned
 // ---------------------------------------------------------------------------------------
 // tile pruning (knn.cuh): everything here runs once per call before the main filter pass, block = one work unit
 // ---------------------------------------------------------------------------------------
-constexpr int kPruneThreads = kUnitQ;     // one thread per query of a unit
+// Every kernel here is built for both unit sizes: kPruneThreads = queries per unit, one thread per query.
 // Skip test: LB(unit box, tile box) > U (1 + kPruneRel).  The margin covers the eigenvectors' deviation from exact
 // orthonormality (|V^T V - I| ~ 1e-14 after Jacobi) and the float64 rounding of the distances; the rounding of the
 // projections is covered by the per-box slack, which is subtracted from every axis gap.
@@ -424,6 +433,7 @@ __global__ void knn_prune_keys_kernel(const double* __restrict__ q, int64_t m, c
   vals[i] = (int)i;
 }
 
+template <int kPruneThreads>
 __device__ __forceinline__ double block_max(double v, double* sh) {
   v = warp_reduce(v, [](double a, double b) { return fmax(a, b); });
   __syncthreads();
@@ -436,13 +446,14 @@ __device__ __forceinline__ double block_max(double v, double* sh) {
 
 // box of a unit's queries in the principal axes; queries outside the filter's range (rescanned in float64 anyway) and
 // padding positions do not count
+template <int kPruneThreads>
 __global__ void __launch_bounds__(kPruneThreads)
 knn_prune_unit_box_kernel(const double* __restrict__ q, int64_t m, const KnnPruneGeom* __restrict__ g, const int* __restrict__ qperm,
                           const float* __restrict__ qnorm, float qnorm_limit, double* __restrict__ ulo, double* __restrict__ uhi,
                           double* __restrict__ uslack) {
   __shared__ double s_lo[kPruneThreads / 32][kPruneMaxDim], s_hi[kPruneThreads / 32][kPruneMaxDim], s_red[kPruneThreads / 32];
   const int u = blockIdx.x, d = g->d, w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t pos = (int64_t)u * kUnitQ + threadIdx.x;
+  const int64_t pos = (int64_t)u * kPruneThreads + threadIdx.x;
   const int64_t qi = pos < m ? qperm[pos] : -1;
   const bool valid = qi >= 0 && qnorm[qi] <= qnorm_limit;
   double p[kPruneMaxDim], l1 = 0.0;
@@ -454,7 +465,7 @@ knn_prune_unit_box_kernel(const double* __restrict__ q, int64_t m, const KnnPrun
     const double hi = warp_reduce(valid ? p[a] : -INFINITY, [](double x, double y) { return fmax(x, y); });
     if (lane == 0) { s_lo[w][a] = lo; s_hi[w][a] = hi; }
   }
-  const double l1max = block_max(l1, s_red);            // (its barriers also publish s_lo / s_hi)
+  const double l1max = block_max<kPruneThreads>(l1, s_red);            // (its barriers also publish s_lo / s_hi)
   if (threadIdx.x < d) {
     double lo = INFINITY, hi = -INFINITY;
     for (int ww = 0; ww < kPruneThreads / 32; ++ww) { lo = fmin(lo, s_lo[ww][threadIdx.x]); hi = fmax(hi, s_hi[ww][threadIdx.x]); }
@@ -467,6 +478,7 @@ knn_prune_unit_box_kernel(const double* __restrict__ q, int64_t m, const KnnPrun
 __device__ __forceinline__ bool less_dt(double da, int ta, double db, int tb) { return da < db || (da == db && ta < tb); }
 
 // seed lists: the kPruneSeedTiles tiles whose box centre is nearest the unit's box centre
+template <int kPruneThreads>
 __global__ void __launch_bounds__(kPruneThreads)
 knn_prune_seed_kernel(int t_tiles, int d, const double* __restrict__ ulo, const double* __restrict__ uhi, const double* __restrict__ tlo,
                       const double* __restrict__ thi, int S, int* __restrict__ seed, int* __restrict__ seed_cnt) {
@@ -517,13 +529,14 @@ knn_prune_seed_kernel(int t_tiles, int d, const double* __restrict__ ulo, const 
 
 // U per query: the k-th float64 distance among the seed pass's candidates (real rows, so an upper bound on the k-th
 // neighbour's distance), capped by the caller's bound; the unit's radius is the largest U of its queries in range
+template <int kPruneThreads>
 __global__ void __launch_bounds__(kPruneThreads)
 knn_prune_bound_kernel(const double* __restrict__ train, const double* __restrict__ q, int64_t m, int d, int k,
                        const int* __restrict__ qperm, const int* __restrict__ cand_idx, const float* __restrict__ qnorm, float qnorm_limit,
                        const double* __restrict__ caller_bound, double* __restrict__ bound, double* __restrict__ unit_rad) {
   __shared__ double s_red[kPruneThreads / 32];
   const int u = blockIdx.x;
-  const int64_t pos = (int64_t)u * kUnitQ + threadIdx.x;
+  const int64_t pos = (int64_t)u * kPruneThreads + threadIdx.x;
   const int64_t qi = pos < m ? qperm[pos] : -1;
   const bool valid = qi >= 0 && qnorm[qi] <= qnorm_limit;
   double U = INFINITY;
@@ -543,12 +556,13 @@ knn_prune_bound_kernel(const double* __restrict__ train, const double* __restric
     if (caller_bound) U = fmin(U, caller_bound[qi]);
     bound[qi] = U;
   }
-  const double any = block_max(valid ? 1.0 : 0.0, s_red);
-  const double r = block_max(valid ? U : -INFINITY, s_red);
+  const double any = block_max<kPruneThreads>(valid ? 1.0 : 0.0, s_red);
+  const double r = block_max<kPruneThreads>(valid ? U : -INFINITY, s_red);
   if (threadIdx.x == 0) unit_rad[u] = any > 0.0 ? r : INFINITY;      // no query in range: keep every tile
 }
 
 // the main pass's tile list of a unit, in tile order: every tile whose box may hold a row within the unit's radius
+template <int kPruneThreads>
 __global__ void __launch_bounds__(kPruneThreads)
 knn_prune_list_kernel(int t_tiles, int d, const double* __restrict__ ulo, const double* __restrict__ uhi, const double* __restrict__ uslack,
                       const double* __restrict__ unit_rad, const double* __restrict__ tlo, const double* __restrict__ thi,
@@ -590,7 +604,7 @@ knn_prune_list_kernel(int t_tiles, int d, const double* __restrict__ ulo, const 
 }  // namespace
 
 float knn_tc16_max_norm() { return 8192.f; }       // |x|^2 <= 8192: every real score stays below kPadNorm - 2 |q| |t|
-int64_t knn_tc16_padded_rows(int64_t rows, bool query) { const int b = query ? kUnitQ : kRows; return (rows + b - 1) / b * b; }
+int64_t knn_tc16_padded_rows(int64_t rows, bool query) { const int b = query ? kMaxUnitQ : kRows; return (rows + b - 1) / b * b; }
 size_t knn_tc16_packed_bytes(int64_t rows, bool query) { return (size_t)(knn_tc16_padded_rows(rows, query) / kRows) * kTileBytes; }
 
 cudaError_t knn_tc16_pack(const double* x, int64_t rows, int d, bool query, void* packed, float* norms, int* flags, cudaStream_t st,
@@ -606,13 +620,17 @@ cudaError_t knn_tc16_pack(const double* x, int64_t rows, int d, bool query, void
 cudaError_t knn_tc16_filter(const void* qpacked, const void* tpacked, int64_t m, int64_t n, int k, const int* qflags, int* cand_idx,
                             float* cand_worst, int sm_count, cudaStream_t st, const float* thr0, const Tc16Work& work) {
   if (m == 0) return cudaSuccess;
-  const int units = (int)(knn_tc16_padded_rows(m, true) / kUnitQ), t_tiles = (int)(knn_tc16_padded_rows(n, false) / kRows);
-  auto fn = k <= 3 ? knn_tc16_filter_kernel<5> : knn_tc16_filter_kernel<kKnnCand>;
-  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem);
+  const int qb = work.unit_queries / kRows;
+  if (work.unit_queries != qb * kRows || qb < 1 || qb > 2) return cudaErrorInvalidValue;
+  const int units = (int)((m + work.unit_queries - 1) / work.unit_queries), t_tiles = (int)(knn_tc16_padded_rows(n, false) / kRows);
+  auto fn = qb == 1 ? (k <= 3 ? knn_tc16_filter_kernel<5, 1> : knn_tc16_filter_kernel<kKnnCand, 1>)
+                    : (k <= 3 ? knn_tc16_filter_kernel<5, 2> : knn_tc16_filter_kernel<kKnnCand, 2>);
+  const size_t smem = tc_smem(qb);
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   const int grid = units < sm_count ? units : sm_count;
   if (work.counter) cudaMemsetAsync(work.counter, 0, sizeof(int), st);
-  fn<<<grid, kTcThreads, kTcSmem, st>>>(static_cast<const unsigned char*>(qpacked), static_cast<const unsigned char*>(tpacked), m, (int)n,
+  fn<<<grid, kTcThreads, smem, st>>>(static_cast<const unsigned char*>(qpacked), static_cast<const unsigned char*>(tpacked), m, (int)n,
                                         units, t_tiles, qflags, cand_idx, cand_worst, thr0, work);
   return cudaGetLastError();
 }
@@ -661,12 +679,15 @@ struct PruneScratch {
   unsigned long long* kept;
 };
 
+// sized for the smaller unit (the most units), so one layout serves both unit sizes
 size_t prune_layout(int64_t m, int64_t n, unsigned char* base, PruneScratch& s) {
-  const int64_t units = knn_tc16_padded_rows(m, true) / kUnitQ, t_tiles = knn_tc16_padded_rows(n, false) / kRows;
-  size_t b1 = 0, b2 = 0;
+  const int64_t units = (m + kRows - 1) / kRows, t_tiles = knn_tc16_padded_rows(n, false) / kRows;
+  size_t b1 = 0, b2 = 0, b3 = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, b1, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr, (int*)nullptr, (int)m, 0, 30);
   cub::DeviceRadixSort::SortPairsDescending(nullptr, b2, (const int*)nullptr, (int*)nullptr, (const int*)nullptr, (int*)nullptr, (int)units);
-  s.sort_bytes = std::max(b1, b2);
+  cub::DeviceRadixSort::SortPairsDescending(nullptr, b3, (const int*)nullptr, (int*)nullptr, (const int*)nullptr, (int*)nullptr,
+                                            (int)((m + kMaxUnitQ - 1) / kMaxUnitQ));
+  s.sort_bytes = std::max({b1, b2, b3});
   size_t off = 0;
   auto take = [&](size_t bytes) { void* p = base ? base + off : nullptr; off += (bytes + 255) / 256 * 256; return p; };
   for (int i = 0; i < 2; ++i) { s.keys[i] = (unsigned*)take(4 * (size_t)m); s.vals[i] = (int*)take(4 * (size_t)m); }
@@ -768,14 +789,21 @@ size_t knn_prune_scratch_bytes(int64_t m, int64_t n) {
   return prune_layout(m, n, nullptr, s);
 }
 
-cudaError_t knn_prune_prepare(const double* q, int64_t m, int64_t n, int d, int k, const double* train, const KnnPruneGeom* geom,
-                              const int* tperm, const double* tile_lo, const double* tile_hi, const double* tile_slack, const void* tpacked,
-                              void* qpacked, float* qnorm, int* qflags, const double* caller_bound, double* bound, int* cand_idx,
-                              float* cand_worst, void* scratch, bool auto_fallback, int sm_count, cudaStream_t st, Tc16Work& work) {
-  if (m == 0) return cudaSuccess;
+int knn_prune_unit_queries(int64_t m, int sm_count) {
+  return (m + kMaxUnitQ - 1) / kMaxUnitQ >= (int64_t)kPruneUnitsPerSm * sm_count ? kMaxUnitQ : kRows;
+}
+
+namespace {
+
+template <int kUnitQ>
+cudaError_t prune_prepare(const double* q, int64_t m, int64_t n, int d, int k, const double* train, const KnnPruneGeom* geom,
+                          const int* tperm, const double* tile_lo, const double* tile_hi, const double* tile_slack, const void* tpacked,
+                          void* qpacked, float* qnorm, int* qflags, const double* caller_bound, double* bound, int* cand_idx,
+                          float* cand_worst, void* scratch, bool auto_fallback, int sm_count, cudaStream_t st, Tc16Work& work) {
+  constexpr int kPruneThreads = kUnitQ;
   PruneScratch s;
   prune_layout(m, n, static_cast<unsigned char*>(scratch), s);
-  const int units = (int)(knn_tc16_padded_rows(m, true) / kUnitQ), t_tiles = (int)(knn_tc16_padded_rows(n, false) / kRows);
+  const int units = (int)((m + kUnitQ - 1) / kUnitQ), t_tiles = (int)(knn_tc16_padded_rows(n, false) / kRows);
   const float limit = knn_tc16_max_norm();
   // query order along the curve, packed in that order
   knn_prune_keys_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(q, m, geom, s.keys[0], s.vals[0]);
@@ -784,18 +812,18 @@ cudaError_t knn_prune_prepare(const double* q, int64_t m, int64_t n, int d, int 
   if (e != cudaSuccess) return e;
   const int* qperm = s.vals[1];
   if ((e = knn_tc16_pack(q, m, d, true, qpacked, qnorm, qflags, st, qperm)) != cudaSuccess) return e;
-  knn_prune_unit_box_kernel<<<units, kPruneThreads, 0, st>>>(q, m, geom, qperm, qnorm, limit, s.ulo, s.uhi, s.uslack);
+  knn_prune_unit_box_kernel<kPruneThreads><<<units, kPruneThreads, 0, st>>>(q, m, geom, qperm, qnorm, limit, s.ulo, s.uhi, s.uslack);
   // seed pass: each unit against its nearest tiles
   const int S = std::min(kPruneSeedTiles, t_tiles);
-  knn_prune_seed_kernel<<<units, kPruneThreads, 0, st>>>(t_tiles, d, s.ulo, s.uhi, tile_lo, tile_hi, S, s.seed, s.seed_cnt);
+  knn_prune_seed_kernel<kPruneThreads><<<units, kPruneThreads, 0, st>>>(t_tiles, d, s.ulo, s.uhi, tile_lo, tile_hi, S, s.seed, s.seed_cnt);
   Tc16Work seed;
   seed.tiles = s.seed; seed.tile_count = s.seed_cnt; seed.stride = S;
-  seed.qperm = qperm; seed.tperm = tperm;
+  seed.qperm = qperm; seed.tperm = tperm; seed.unit_queries = kUnitQ;
   if ((e = knn_tc16_filter(qpacked, tpacked, m, n, k, qflags, cand_idx, cand_worst, sm_count, st, nullptr, seed)) != cudaSuccess) return e;
-  knn_prune_bound_kernel<<<units, kPruneThreads, 0, st>>>(train, q, m, d, k, qperm, cand_idx, qnorm, limit, caller_bound, bound, s.rad);
+  knn_prune_bound_kernel<kPruneThreads><<<units, kPruneThreads, 0, st>>>(train, q, m, d, k, qperm, cand_idx, qnorm, limit, caller_bound, bound, s.rad);
   // tile lists, units longest first
   cudaMemsetAsync(s.kept, 0, sizeof(unsigned long long), st);
-  knn_prune_list_kernel<<<units, kPruneThreads, 0, st>>>(t_tiles, d, s.ulo, s.uhi, s.uslack, s.rad, tile_lo, tile_hi, tile_slack, s.tiles,
+  knn_prune_list_kernel<kPruneThreads><<<units, kPruneThreads, 0, st>>>(t_tiles, d, s.ulo, s.uhi, s.uslack, s.rad, tile_lo, tile_hi, tile_slack, s.tiles,
                                                          s.count[0], s.ids[0], s.kept);
   bytes = s.sort_bytes;
   e = cub::DeviceRadixSort::SortPairsDescending(s.sort_tmp, bytes, s.count[0], s.count[1], s.ids[0], s.ids[1], units, 0, 32, st);
@@ -805,8 +833,20 @@ cudaError_t knn_prune_prepare(const double* q, int64_t m, int64_t n, int d, int 
   work.unit_order = s.ids[1]; work.counter = s.counter;
   work.kept = s.kept;
   work.kept_limit = auto_fallback ? (unsigned long long)(0.85 * (double)units * (double)t_tiles) : ~0ull;
-  work.qperm = qperm; work.tperm = tperm;
+  work.qperm = qperm; work.tperm = tperm; work.unit_queries = kUnitQ;
   return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t knn_prune_prepare(const double* q, int64_t m, int64_t n, int d, int k, const double* train, const KnnPruneGeom* geom,
+                              const int* tperm, const double* tile_lo, const double* tile_hi, const double* tile_slack, const void* tpacked,
+                              void* qpacked, float* qnorm, int* qflags, const double* caller_bound, double* bound, int* cand_idx,
+                              float* cand_worst, void* scratch, bool auto_fallback, int sm_count, cudaStream_t st, Tc16Work& work) {
+  if (m == 0) return cudaSuccess;
+  auto fn = knn_prune_unit_queries(m, sm_count) == kRows ? prune_prepare<kRows> : prune_prepare<kMaxUnitQ>;
+  return fn(q, m, n, d, k, train, geom, tperm, tile_lo, tile_hi, tile_slack, tpacked, qpacked, qnorm, qflags, caller_bound, bound,
+            cand_idx, cand_worst, scratch, auto_fallback, sm_count, st, work);
 }
 
 }  // namespace dsp
