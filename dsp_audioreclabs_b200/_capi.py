@@ -101,6 +101,7 @@ SIGNATURES = {
     "dsp_mfcc_batch_device": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, C.POINTER(MfccParams), _P, _P, _P, _P, _P]),
     "dsp_dtw_fit_device": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I32, _I32, _I64, C.POINTER(_P)]),
     "dsp_dtw_topk_device": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _P]),
+    "dsp_dtw_topk_bounded_device": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _P, _P]),
     "dsp_dtw_last_stats": (C.c_int, [_P, C.POINTER(_I64), C.POINTER(_I64)]),
     "dsp_dtw_free": (C.c_int, [_P]),
     "dsp_wav_scan": (C.c_int, [_P, _I64, _I32, _P]),

@@ -1348,6 +1348,12 @@ int dsp_dtw_fit_device(dsp_context* c, const float* t_feats, const int64_t* t_of
 
 int dsp_dtw_topk_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offsets, const int32_t* q_lengths, int64_t nq,
                         int32_t max_q_frames, double* nbr_cost, int64_t* nbr_idx, int32_t* nbr_label) {
+  return dsp_dtw_topk_bounded_device(h, q_feats, q_offsets, q_lengths, nq, max_q_frames, nullptr, nbr_cost, nbr_idx, nbr_label);
+}
+
+int dsp_dtw_topk_bounded_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offsets, const int32_t* q_lengths, int64_t nq,
+                                int32_t max_q_frames, const double* bound_cost, double* nbr_cost, int64_t* nbr_idx,
+                                int32_t* nbr_label) {
   if (!h || nq < 0 || (nq && !q_offsets)) return fail(DSP_ERR_INVALID, "bad argument");   // q_feats: NULL when every query is empty
   dsp_context* c = h->ctx;
   CU(cudaSetDevice(c->device));
@@ -1358,7 +1364,7 @@ int dsp_dtw_topk_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offse
     CU(h->cand_i.ensure(sizeof(int64_t) * cand));
   }
   CU(launch_dtw_topk_fused(q_feats, q_offsets, q_lengths, nq, max_q_frames, h->feats.as<float>(), h->offsets.as<int64_t>(),
-                           h->t_len.as<int32_t>(), h->nt, h->max_t, h->dim, h->k, slices, h->warps, h->index_base,
+                           h->t_len.as<int32_t>(), h->nt, h->max_t, h->dim, h->k, bound_cost, slices, h->warps, h->index_base,
                            h->labels.as<int32_t>(), h->cand_d.as<float>(), h->cand_i.as<int64_t>(),
                            h->stats.as<unsigned long long>(), nbr_cost, nbr_idx, nbr_label, c->stream));
   c->launches += nq > 0 ? 3 : 1;

@@ -261,7 +261,8 @@ __device__ __forceinline__ bool dtw_pair(const float* __restrict__ qp, int n, co
             // still has to cross the previous strip's last row at a column >= j: D >= sufmin[j]; or (c) below it (not
             // in the final strip): it crossed this strip's last row at a column <= j: D >= last_row_min.  The least
             // of these bounds D[n-1][m-1]; strictly above the k-th cost the pair cannot enter the top k even through
-            // the index tie-break.
+            // the index tie-break.  Under a caller's cost bound U, kth never exceeds ru(U) >= U (rounded up to fp32),
+            // so a pair abandoned while the slice's list is short costs more than U and is no candidate either.
             last_row_min = fminf(last_row_min, cur_r);
             float bound = fminf(col_min, i0 > 0 ? sufmin[j] : INFINITY);
             if (!final_strip) bound = fminf(bound, last_row_min);
@@ -356,12 +357,15 @@ __global__ void dtw_topk_kernel(const float* __restrict__ cost, int64_t nq, int6
 // c on lane c, so the k-th cost that decides the early exit is one shuffle away.  Output: cand_d / cand_i [unit][k],
 // (inf, INT64_MAX) where the slice has fewer than k, merged per query by dtw_merge_kernel.  stats[0] / [1] count the
 // pairs scored to the last cell / abandoned.
+// bound (nullable, float64 per query): only templates with cost <= bound[qi] (compared in float64) are candidates, and
+// the abandon threshold starts at the bound rounded up to fp32 instead of inf.  A bound that is not >= 0 (negative,
+// NaN) admits nothing: the slice is skipped and its pairs count as abandoned.  +inf (or no array) is no bound.
 template <int R, int DMAX>
 __global__ void __launch_bounds__(kDtwFusedWarps * 32, 1)
 dtw_topk_fused_kernel(const float* __restrict__ qf, const int64_t* __restrict__ qoff, const int32_t* __restrict__ qlen, int64_t nq,
                       const float* __restrict__ tf, const int64_t* __restrict__ toff, const int32_t* __restrict__ tlen,
-                      int64_t nt, int dim, int max_t_frames, int slices, int k, float* __restrict__ cand_d,
-                      int64_t* __restrict__ cand_i, unsigned long long* __restrict__ stats) {
+                      int64_t nt, int dim, int max_t_frames, int slices, int k, const double* __restrict__ bound,
+                      float* __restrict__ cand_d, int64_t* __restrict__ cand_i, unsigned long long* __restrict__ stats) {
   extern __shared__ float smem[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t unit = (int64_t)blockIdx.x * (blockDim.x >> 5) + w;
@@ -373,13 +377,17 @@ dtw_topk_fused_kernel(const float* __restrict__ qf, const int64_t* __restrict__ 
   const int n = qlen ? qlen[qi] : (int)(qoff[qi + 1] - qoff[qi]);
   const float* qp = qf + qoff[qi] * dim;
   const int64_t t_end = nt * (sl + 1) / slices;
-  float my_d = INFINITY, kth = INFINITY;
+  const double ub = bound ? bound[qi] : (double)INFINITY;
+  const float kth0 = __double2float_ru(ub);     // ub <= kth0: a lower bound above kth0 puts the cost above ub
+  float my_d = INFINITY, kth = kth0;
   int64_t my_i = INT64_MAX;
   float q[R][DMAX];
   int q_strip = -1;
   unsigned long long scored = 0, abandoned = 0;
+  int64_t ti = nt * sl / slices;
+  if (!(ub >= 0)) { abandoned = t_end - ti; ti = t_end; }
 #pragma unroll 1
-  for (int64_t ti = nt * sl / slices; ti < t_end; ++ti) {
+  for (; ti < t_end; ++ti) {
     const int m = tlen[ti];
     float cost = INFINITY;
     if (n > 0 && m > 0) {
@@ -389,7 +397,9 @@ dtw_topk_fused_kernel(const float* __restrict__ qf, const int64_t* __restrict__ 
       if (!dtw_pair<R, DMAX, true>(qp, n, st, m, dim, brow, sufmin, kth, q, q_strip, cost)) { ++abandoned; continue; }
     }
     ++scored;
-    if (cost <= kth) {                          // insert into the sorted list held one entry per lane
+    // insert into the sorted list held one entry per lane; the bound is compared in float64, since kth0 may admit
+    // costs in (ub, kth0]
+    if (cost <= kth && (double)cost <= ub) {
       const bool before = dtw_before(cost, ti, my_d, my_i);
       const bool shift = __shfl_up_sync(0xffffffffu, (int)before, 1) && lane > 0;
       const float up_d = __shfl_up_sync(0xffffffffu, my_d, 1);
@@ -398,7 +408,7 @@ dtw_topk_fused_kernel(const float* __restrict__ qf, const int64_t* __restrict__ 
         if (shift) { my_d = up_d; my_i = up_i; }
         else if (before) { my_d = cost; my_i = ti; }
       }
-      kth = __shfl_sync(0xffffffffu, my_d, k - 1);
+      kth = fminf(kth0, __shfl_sync(0xffffffffu, my_d, k - 1));   // a short list must not lift it to inf
     }
   }
   if (lane < k) { cand_d[unit * k + lane] = my_d; cand_i[unit * k + lane] = my_i; }
@@ -494,9 +504,9 @@ int dtw_fused_slices(int64_t nq, int64_t nt, int sm_count) {
 
 cudaError_t launch_dtw_topk_fused(const float* qf, const int64_t* qoff, const int32_t* qlen, int64_t nq, int max_q_frames,
                                   const float* tf, const int64_t* toff, const int32_t* tlen, int64_t nt, int max_t_frames, int dim,
-                                  int k, int slices, int warps, int64_t index_base, const int32_t* labels, float* cand_d,
-                                  int64_t* cand_i, unsigned long long* stats, double* nbr_cost, int64_t* nbr_idx,
-                                  int32_t* nbr_label, cudaStream_t st) {
+                                  int k, const double* bound, int slices, int warps, int64_t index_base, const int32_t* labels,
+                                  float* cand_d, int64_t* cand_i, unsigned long long* stats, double* nbr_cost,
+                                  int64_t* nbr_idx, int32_t* nbr_label, cudaStream_t st) {
   cudaError_t e = cudaMemsetAsync(stats, 0, 2 * sizeof(unsigned long long), st);
   if (e != cudaSuccess || nq == 0) return e;
   if (dim > kDtwMaxDim || k < 1 || k > kKnnMaxK || warps < 1 || warps > kDtwFusedWarps) return cudaErrorInvalidValue;
@@ -508,7 +518,7 @@ cudaError_t launch_dtw_topk_fused(const float* qf, const int64_t* qoff, const in
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<(unsigned)((units + warps - 1) / warps), 32 * warps, smem, st>>>(qf, qoff, qlen, nq, tf, toff, tlen, nt, dim, mt,
-                                                                            slices, k, cand_d, cand_i, stats);
+                                                                            slices, k, bound, cand_d, cand_i, stats);
     return cudaGetLastError();
   });
   if (e != cudaSuccess) return e;

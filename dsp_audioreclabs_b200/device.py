@@ -331,24 +331,35 @@ class DeviceDTW:
         self.dim = feats.shape[1]
         return self
 
-    def topk(self, feats, offsets, lengths=None, max_q_frames=None):
+    def topk(self, feats, offsets, lengths=None, max_q_frames=None, bound=None):
         """(cost float64, template index int64, label int32), each [nq, k], ties to the lower index, (inf, -1, -1)
-        where fewer than k templates have a finite cost.  max_q_frames (optional) only picks the kernel build."""
+        where fewer than k templates have a finite cost.  max_q_frames (optional) only picks the kernel build.
+
+        bound (optional contiguous float64 CUDA tensor [nq], dsp_dtw_topk_bounded_device): a cost bound per query.
+        Only templates whose cost is <= bound[q] (ties included) are returned: every such template is either returned
+        or displaced by k templates ordered before it by (cost, index), and the query's other slots are (inf, -1, -1).
+        A negative or NaN bound returns an empty list, +inf is no bound.  Returned costs are the unbounded call's, bit
+        for bit.  Uses: rejecting queries no template is close enough to, and row shards of a template set given a
+        cost the caller already knows (pairs above it are abandoned from the first template on)."""
         self._check_seqs(feats, offsets, lengths)
         if feats.shape[1] != self.dim:
             raise ValueError(f"queries have {feats.shape[1]} features, the templates {self.dim}")
-        _bind(self.device, self.ctx)
         nq = offsets.numel() - 1
+        if bound is not None and (not bound.is_cuda or bound.dtype != torch.float64 or not bound.is_contiguous()
+                                  or bound.numel() != nq):
+            raise ValueError(f"bound must be a contiguous float64 CUDA tensor of {nq} entries")
+        _bind(self.device, self.ctx)
         cost = torch.empty(nq, self.k, dtype=torch.float64, device=self.device)
         idx = torch.empty(nq, self.k, dtype=torch.int64, device=self.device)
         lab = torch.empty(nq, self.k, dtype=torch.int32, device=self.device)
-        check(self.ctx.lib.dsp_dtw_topk_device(self.handle, _dp(feats), _dp(offsets), _dp(lengths), nq,
-                                               int(max_q_frames or 0), _dp(cost), _dp(idx), _dp(lab)))
+        check(self.ctx.lib.dsp_dtw_topk_bounded_device(self.handle, _dp(feats), _dp(offsets), _dp(lengths), nq,
+                                                       int(max_q_frames or 0), _dp(bound), _dp(cost), _dp(idx), _dp(lab)))
         return cost, idx, lab
 
-    def predict(self, feats, offsets, lengths=None, max_q_frames=None):
-        """Majority label of the k cheapest templates, ties to the smallest label: int32 [nq]."""
-        cost, idx, lab = self.topk(feats, offsets, lengths, max_q_frames)
+    def predict(self, feats, offsets, lengths=None, max_q_frames=None, bound=None):
+        """Majority label of the k cheapest templates, ties to the smallest label: int32 [nq].  With a bound (see
+        topk) the vote is over the templates within it, and a query with none gets -1."""
+        cost, idx, lab = self.topk(feats, offsets, lengths, max_q_frames, bound)
         nq = cost.shape[0]
         out = torch.empty(nq, dtype=torch.int32, device=self.device)
         if nq:
@@ -357,7 +368,8 @@ class DeviceDTW:
         return out
 
     def last_stats(self):
-        """(pairs scored to their last cell, pairs abandoned early) of the last topk / predict call."""
+        """(pairs scored to their last cell, pairs abandoned early) of the last topk / predict call; the pairs of a
+        query whose bound admits nothing count as abandoned."""
         scored, abandoned = C.c_int64(), C.c_int64()
         check(self.ctx.lib.dsp_dtw_last_stats(self.handle, C.byref(scored), C.byref(abandoned)))
         return int(scored.value), int(abandoned.value)

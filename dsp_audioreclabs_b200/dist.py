@@ -10,7 +10,8 @@
   classify locally (`ShardedKNN.predict_replicated`); `ShardedKNN.predict` picks by size.
 
 * DTW template matching (the self-specified MFCC + DTW variant): templates sharded by row, queries replicated,
-  the same single all-gather of top-k candidates (`ShardedDTW`).
+  the same single all-gather of top-k candidates (`ShardedDTW` on lists of NumPy arrays through the host call,
+  `ShardedDeviceDTW` on device tensors through the fused top-k).
 
 torch.distributed is plumbing only; the compute callbacks default to the CUDA library and can
 be replaced (the CPU gloo tests plug in the oracle, since there is no CPU implementation here).
@@ -238,6 +239,21 @@ class ShardedKNN:
         return self._merge(d2[None], idx[None], lab[None])
 
 
+def merge_topk(cost, idx, lab, k):
+    """k-way selection over R candidate lists [R, m, k] (cost f64, global index i64, label i32), by (cost, global
+    index), empty slots (index < 0) last: a stable sort by index followed by a stable sort by cost, with torch sorts on
+    the tensors' device (no host synchronisation).  Returns (cost, index, label) [m, k]."""
+    m = cost.shape[1]
+    cost = cost.permute(1, 0, 2).reshape(m, -1)
+    idx = idx.permute(1, 0, 2).reshape(m, -1)
+    lab = lab.permute(1, 0, 2).reshape(m, -1)
+    key = torch.where(idx < 0, torch.full_like(idx, torch.iinfo(torch.int64).max), idx)
+    o1 = torch.argsort(key, dim=1, stable=True)
+    o2 = torch.argsort(cost.gather(1, o1), dim=1, stable=True)
+    order = o1.gather(1, o2)[:, :k]
+    return tuple(a.gather(1, order) for a in (cost, idx, lab))
+
+
 class ShardedDTW:
     """Row-sharded DTW template matching (BASELINE config 5: templates sharded by row, queries replicated, ONE
     all-gather of the packed per-shard top-k candidates).  Sequences are lists of [frames, dim] float32 arrays.
@@ -283,17 +299,7 @@ class ShardedDTW:
         if self.device is not None:
             c, i, l = c.to(self.device), i.to(self.device), l.to(self.device)
         cc, ci, cl = all_gather_candidates(c, i, l, self.group)            # the single candidate exchange
-        # k-way selection over the R sorted lists by (cost, global index), on whatever device the group runs on:
-        # a stable sort by index followed by a stable sort by cost
-        m = cc.shape[1]
-        cost = cc.permute(1, 0, 2).reshape(m, -1)
-        idx = ci.permute(1, 0, 2).reshape(m, -1)
-        lab = cl.permute(1, 0, 2).reshape(m, -1)
-        key = torch.where(idx < 0, torch.full_like(idx, torch.iinfo(torch.int64).max), idx)
-        o1 = torch.argsort(key, dim=1, stable=True)
-        o2 = torch.argsort(cost.gather(1, o1), dim=1, stable=True)
-        order = o1.gather(1, o2)[:, :self.k]
-        return tuple(a.gather(1, order).cpu().numpy() for a in (cost, idx, lab))
+        return tuple(a.cpu().numpy() for a in merge_topk(cc, ci, cl, self.k))
 
     def predict(self, queries):
         _, _, lab = self.kneighbors(queries)
@@ -302,6 +308,87 @@ class ShardedDTW:
             vals, cnt = np.unique(row[row >= 0], return_counts=True)
             out[q] = vals[np.argmax(cnt)] if len(vals) else -1      # argmax: first maximum = smallest label
         return out
+
+
+class ShardedDeviceDTW:
+    """Row-sharded DTW template matching on device tensors (BASELINE config 5's exchange: templates sharded by row,
+    queries replicated, ONE all-gather of the packed per-shard top-k candidates).  Sequences are packed as
+    device.DeviceDTW takes them: float32 [frames, dim] feats, int64 offsets [n + 1] in frames, optional int32 lengths.
+
+    The queries must be the same on every rank (same sequences, same order): the ranks exchange candidates for query
+    positions, and nothing checks that the positions mean the same sequence everywhere.  Once the shapes are warm a
+    call enqueues its work with no host synchronisation.
+
+    local_topk(t_feats, t_offsets, t_labels, q_feats, q_offsets, k, index_base, bound=None, t_lengths=None,
+    q_lengths=None, max_q_frames=None) -> (cost f64, global index i64, label i32) [nq, k], sorted by (cost, index),
+    (inf, -1, -1) in empty slots, only templates with cost <= bound[q] when a bound is given; defaults to the fused
+    top-k of device.DeviceDTW.  merge_vote(cost [R, nq, k], idx, label) -> int32 [nq] labels; defaults to
+    dsp_knn_merge_vote_device.  Labels are class indices >= 0 (-1 marks an empty slot)."""
+
+    def __init__(self, n_neighbors=1, group=None, local_topk=None, merge_vote=None):
+        self.k = int(n_neighbors)
+        self.group = group
+        self._topk = local_topk or self._cuda_topk
+        self._merge = merge_vote or self._cuda_merge
+        self._dtw = None
+        self._merger = None
+
+    # -- CUDA callbacks ---------------------------------------------------------------------
+    def _cuda_topk(self, t_feats, t_offsets, t_labels, q_feats, q_offsets, k, index_base, bound=None, t_lengths=None,
+                   q_lengths=None, max_q_frames=None):
+        from .device import DeviceDTW
+        if self._dtw is None:
+            self._dtw = DeviceDTW(k, device=q_feats.device, index_base=index_base)
+            if t_offsets.numel() > 1:
+                self._dtw.fit(t_feats, t_offsets, t_labels, t_lengths)
+        if self._dtw.handle is None:            # a shard without templates: every slot empty
+            nq = q_offsets.numel() - 1
+            return (torch.full((nq, k), float("inf"), dtype=torch.float64, device=q_feats.device),
+                    torch.full((nq, k), -1, dtype=torch.int64, device=q_feats.device),
+                    torch.full((nq, k), -1, dtype=torch.int32, device=q_feats.device))
+        return self._dtw.topk(q_feats, q_offsets, q_lengths, max_q_frames, bound)
+
+    def _cuda_merge(self, cost, idx, lab):
+        from .device import DeviceKNN
+        if self._merger is None:
+            self._merger = DeviceKNN(self.k, device=cost.device)
+        return self._merger.merge_vote(cost, idx, lab)[0]
+
+    # -- API -------------------------------------------------------------------------------
+    def fit(self, feats, offsets, labels, lengths=None):
+        """Keep this rank's template shard; the global index of its first template and the size of the whole template
+        set come from one all-gather of the shard sizes.  A second fit() starts from scratch."""
+        world, rank = dist.get_world_size(self.group), dist.get_rank(self.group)
+        if labels.numel() and int(labels.min()) < 0:
+            raise ValueError("labels must be class indices >= 0 (encode them with np.unique(..., return_inverse=True))")
+        if self._dtw is not None:
+            self._dtw.free()
+        self._dtw = None
+        n = torch.tensor([offsets.numel() - 1], dtype=torch.int64, device=offsets.device)
+        sizes = torch.empty(world, dtype=torch.int64, device=offsets.device)
+        dist.all_gather_into_tensor(sizes, n, group=self.group)
+        sizes = [int(v) for v in sizes.tolist()]
+        self.index_base = int(sum(sizes[:rank]))
+        self.n_total = int(sum(sizes))
+        self.feats, self.offsets, self.labels, self.lengths = feats, offsets, labels, lengths
+        return self
+
+    def _gathered(self, q_feats, q_offsets, q_lengths, bound, max_q_frames):
+        c, i, l = self._topk(self.feats, self.offsets, self.labels, q_feats, q_offsets, self.k, self.index_base,
+                             bound=bound, t_lengths=self.lengths, q_lengths=q_lengths, max_q_frames=max_q_frames)
+        return all_gather_candidates(c, i, l, self.group)                 # the single candidate exchange
+
+    def kneighbors(self, q_feats, q_offsets, q_lengths=None, bound=None, max_q_frames=None):
+        """(cost f64, global template index i64, label i32) [nq, k] on the device for the (replicated) queries, ties to
+        the lower index, (inf, -1, -1) in empty slots.  bound (optional float64 [nq]): only templates with cost <=
+        bound[q] (device.DeviceDTW.topk); every shard abandons the pairs above it from its first template on.
+        max_q_frames (optional) only picks the kernel build."""
+        return merge_topk(*self._gathered(q_feats, q_offsets, q_lengths, bound, max_q_frames), self.k)
+
+    def predict(self, q_feats, q_offsets, q_lengths=None, bound=None, max_q_frames=None):
+        """Majority label of the k cheapest templates over all shards, ties to the smallest label, -1 where no template
+        lies within the bound: int32 [nq] on the device."""
+        return self._merge(*self._gathered(q_feats, q_offsets, q_lengths, bound, max_q_frames))
 
 
 def zscore_stats_allreduce(x_local, group=None):

@@ -309,8 +309,22 @@ int dsp_dtw_fit_device(dsp_context* ctx, const float* t_feats, const int64_t* t_
 int dsp_dtw_topk_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offsets,
                         const int32_t* q_lengths, int64_t nq, int32_t max_q_frames, double* nbr_cost,
                         int64_t* nbr_idx, int32_t* nbr_label);
-/* Pairs of the last dsp_dtw_topk_device call scored to their last cell / abandoned early (waits
- * for that call). */
+/* dsp_dtw_topk_device with a cost bound per query (device float64 [nq]; NULL = no bound): only
+ * templates whose cost is <= bound_cost[q] (compared in float64, ties included) are candidates,
+ * and every template within the bound is either returned or displaced by k templates ordered
+ * before it by (cost, index); the query's other slots are (inf, -1, -1).  A bound that is not
+ * >= 0 (negative, NaN) returns an empty list, +inf is no bound.  Returned costs are those of
+ * dsp_dtw_topk_device, bit for bit.  The bound also starts the early exit: pairs whose lower
+ * bound exceeds it are abandoned from the first template on.  Uses: rejection ("no template is
+ * close enough"), and row shards given a cost the caller already knows.  Same launches, no
+ * synchronisation, no allocation beyond the unbounded call's. */
+int dsp_dtw_topk_bounded_device(dsp_dtw* h, const float* q_feats, const int64_t* q_offsets,
+                                const int32_t* q_lengths, int64_t nq, int32_t max_q_frames,
+                                const double* bound_cost, double* nbr_cost, int64_t* nbr_idx,
+                                int32_t* nbr_label);
+/* Pairs of the last dsp_dtw_topk_device / _bounded_device call scored to their last cell /
+ * abandoned early (waits for that call); the pairs of a query whose bound admits nothing count as
+ * abandoned. */
 int dsp_dtw_last_stats(dsp_dtw* h, int64_t* pairs_scored, int64_t* pairs_abandoned);
 int dsp_dtw_free(dsp_dtw* h);
 
